@@ -1,7 +1,7 @@
 #!/usr/bin/env python
-"""Benchmark of the batched LM hot path (contract: see the task prompt / DESIGN.md section 6).
+"""Benchmark of the batched LM hot path (see DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json config 3): 8-exponential correlator, 64 correlated time slices,
 16 diagonal priors, svdcut=1e-12, 10^4 bootstrap copies per GPU per step, p0 = prior mean,
@@ -59,7 +59,32 @@ def parse():
     ap.add_argument("--cpu-sample", type=int, default=2000, help="fits timed on the host for cpu_baseline")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C1/C2/C4/C5 and saturated-batch figures")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step as DIR/<name>.npy (float64; above 60 MB in all, "
+                         "a seeded sample of the fits)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no fit results")
+    return args
+
+
+DUMP_LIMIT = 60 * 1000 * 1000
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as <path>/<name>.npy in float64 (nit and status are small integers, exact in float64).  Above
+    DUMP_LIMIT bytes in all, every array keeps the same fraction of its rows (fits), chosen by a fixed seed from its
+    shape alone: two builds run with the same arguments write the same rows and can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    arrays = dict((k, np.asarray(v, dtype=np.float64)) for k, v in arrays.items())
+    frac = min(1.0, DUMP_LIMIT / float(sum(a.nbytes for a in arrays.values())))
+    for name, a in sorted(arrays.items()):
+        if frac < 1.0:
+            rows = np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * frac), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def load_configs():
@@ -565,6 +590,7 @@ def run_ours(args, rank, local_rank, world):
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     barrier()
+    gathered = None
     for k in range(args.steps):
         flush.zero_()                       # L2 flush between timed iterations (not timed)
         ev[k][0].record()
@@ -573,7 +599,7 @@ def run_ours(args, rank, local_rank, world):
         kev[k][1].record()
         if world > 1:
             packed = lbdist.pack_results(out.x, out.chi2, out.nit, out.status)
-            lbdist.gather_results(packed, comm=nccl_comm)
+            gathered = lbdist.gather_results(packed, comm=nccl_comm)
         ev[k][1].record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
@@ -594,6 +620,9 @@ def run_ours(args, rank, local_rank, world):
     t_ms, tk_ms = float(tt[0]), float(tt[1])
     max_nit = int(ts[3])
     res = out.numpy()
+    if args.dump_outputs and rank == 0:
+        # what the last timed step returned, before the e2e and queued runs below reuse `out`
+        dump_outputs(args.dump_outputs, dict(res, gathered=gathered.cpu().numpy()) if world > 1 else res)
     conv = float((res["status"] > 0).mean())
     warps_per_fit = plan.last_team()
 

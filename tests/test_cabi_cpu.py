@@ -4,6 +4,8 @@ fallback) when no CUDA device is present.  No compute calls are made here."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -45,10 +47,20 @@ def test_functor_registry_matches_host_mirror():
 
 
 def test_no_cpu_fallback():
-    """Without a GPU a plan cannot be created: the product path must fail loudly."""
+    """Without a GPU a plan cannot be created: the product path must fail loudly.  Where a GPU is present, the same
+    checks run in a child process that sees no device (CUDA_VISIBLE_DEVICES empty)."""
     import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+    if not torch.cuda.is_available():
+        _no_device_checks()
+        return
+    code = "import sys; sys.path[:0] = [%r, %r]; import test_cabi_cpu; test_cabi_cpu._no_device_checks()" % (
+        ROOT, os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
+
+
+def _no_device_checks():
     cabi = _lib()
     assert cabi.lib.b200lm_device_count() == 0
     h = cabi.handle_t()
