@@ -86,7 +86,8 @@ int b200lm_nchiv(b200lm_handle h);
  *   d_mean   [B][N] means of y(+)prior per fit (mean_stride = N) or one shared vector
  *            (mean_stride = 0)  -- what bootstrapped_fit_iter / simulated_fit_iter vary
  *            (src/lsqfit/__init__.py:1619-1623, 545-552)
- *   d_p0     [B][np] starting points (p0_stride = np) or one shared start (p0_stride = 0)
+ *   d_p0     [B][np] starting points (p0_stride = np) or one shared start (p0_stride = 0); with bounds
+ *            (b200lm_set_bounds) every start is projected into the box as scipy's make_strictly_feasible does
  *   xtol, gtol, ftol, maxit   as normalised at src/lsqfit/_scipy.py:124-132
  *   scaler   1 = More' column scaling (GSL scaler='more', scipy x_scale='jac'); 0 = none
  *   polish   max number of undamped Gauss-Newton refinement steps taken after the trust-region
@@ -147,6 +148,17 @@ int b200lm_last_order(b200lm_handle h);
  *       12 (info 2: gtol) or 14 (info 27: no progress in the first iteration) -- stopping_criterion = status - 10
  *       (_gsl.pyx:689-701). */
 int b200lm_set_policy(b200lm_handle h, int policy);
+/* bound constraints of the following fit_batch calls on this handle: scipy's ``bounds`` (lsqfit.scipy_least_squares(
+ * bounds=...), src/lsqfit/_scipy.py:77).  h_lb, h_ub: HOST arrays of np entries in device parameter order, -inf / +inf
+ * for "no bound"; one box for every fit of a batch.  NULL, NULL clears the bounds, and so do bounds that are all
+ * infinite (scipy then runs its unbounded trf: the results are those of an unbounded batch, bit for bit).
+ * B200LM_EINVAL for lb >= ub in any entry or a NaN.  A bounded batch runs scipy's trf_bounds decisions (Coleman-Li
+ * scaling, reflective select_step) in the one-warp kernel: team and wave requests are overridden (b200lm_last_team
+ * reports 1), polish is skipped (undamped steps would leave the box), and the GSL policy is refused (EINVAL at
+ * fit_batch).  b200lm_fit_batch projects every start into the box (scipy's make_strictly_feasible with rstep=1e-10);
+ * b200lm_fit_batch_host refuses a host p0 outside the box ("`x0` is infeasible.", as scipy does).  Every returned x
+ * lies in the box. */
+int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub);
 /* number of kernel launches issued through this handle so far */
 long long b200lm_launch_count(b200lm_handle h);
 

@@ -1,5 +1,6 @@
 // C-ABI layer of libb200lm.so: plan objects, functor dispatch, launches.
 // Declarations and the reference interfaces they replace: include/b200lm.h.
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -218,6 +219,7 @@ void b200lm_destroy(b200lm_handle h) {
     cudaFree(h->d_blk); cudaFree(h->d_blk_idx); cudaFree(h->d_blk_wt); cudaFree(h->d_blk_wt2); cudaFree(h->d_wfull);
     cudaFree(h->d_counter); cudaFree(h->d_stats); cudaFree(h->d_stage); cudaFree(h->d_scratch);
     cudaFree(h->d_order_key); cudaFree(h->d_order); cudaFree(h->d_wave_A);
+    cudaFree(h->d_lb); cudaFree(h->d_ub);
     if (h->h_pinned) cudaFreeHost(h->h_pinned);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -339,6 +341,8 @@ int b200lm_fit_batch(b200lm_handle h, int B,
     if (scaler != 0 && scaler != 1 && !(scaler == 2 && h->policy == 1))
         return set_error(h, B200LM_EINVAL, "scaler must be 0 (levenberg), 1 (more) or, with the GSL policy, 2 (marquardt)");
     if (maxit < 1) return set_error(h, B200LM_EINVAL, "maxit must be >= 1");
+    if (h->bounded && h->policy == 1)
+        return set_error(h, B200LM_EINVAL, "bounds need the scipy trf policy (GSL's lm has no bound constraints)");
     if (B == 0) return B200LM_OK;
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
@@ -348,6 +352,7 @@ int b200lm_fit_batch(b200lm_handle h, int B,
     P.xtol = xtol; P.gtol = gtol; P.ftol = ftol; P.maxit = maxit; P.scaler = scaler; P.polish = polish < 0 ? 0 : polish;
     P.x_out = d_x; P.chi2 = d_chi2; P.cov = d_cov; P.logdet = d_logdet; P.nit = d_nit; P.status = d_status;
     P.f_out = d_f; P.J_out = d_J;
+    if (h->bounded) { P.bounded = 1; P.lb = h->d_lb; P.ub = h->d_ub; }
     CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(int), s), "reset work queue");
     CUDA_TRY(h, cudaMemsetAsync(h->d_stats, 0, 16 * sizeof(unsigned long long), s), "reset stats");
     // queue order: chi2 at the start point of every fit (one evaluation each, resjac kernel without f / J outputs),
@@ -376,6 +381,7 @@ int b200lm_fit_batch(b200lm_handle h, int B,
     int team = default_team(h);
     if (const char* env = getenv("B200LM_TEAM")) team = atoi(env);
     if (h->policy == 1) team = 1;            // the GSL decisions are compiled into the one-warp kernel only (fit_kernel<F, 1>)
+    if (h->bounded) team = 1;                // so are the bounded scipy decisions (fit_kernel<F, 3>)
     const int ti = team == 4 ? 1 : (team == 2 ? 0 : -1);
     if (team == 32 && wave_ok(h)) {
         // wave kernel: the trust-region loops of 32 fits per CTA in lock step, then covariance / log det / f / J
@@ -452,6 +458,31 @@ int b200lm_set_order(b200lm_handle h, int mode) {
 }
 
 int b200lm_last_order(b200lm_handle h) { return h ? h->last_order : B200LM_EINVAL; }
+
+int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub) {
+    if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (!h_lb != !h_ub) return set_error(h, B200LM_EINVAL, "give both bounds or neither");
+    bool finite = false;
+    if (h_lb) {
+        for (int j = 0; j < h->np; ++j) {
+            if (h_lb[j] != h_lb[j] || h_ub[j] != h_ub[j]) return set_error(h, B200LM_EINVAL, "bounds must not be NaN");
+            if (!(h_lb[j] < h_ub[j]))
+                return set_error(h, B200LM_EINVAL, "Each lower bound must be strictly less than each upper bound.");
+            finite = finite || h_lb[j] > -INFINITY || h_ub[j] < INFINITY;
+        }
+    }
+    if (!finite) {                               // no bounds, or all infinite: scipy's unbounded trf
+        h->bounded = false;
+        h->h_lb.clear(); h->h_ub.clear();
+        return B200LM_OK;
+    }
+    CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
+    CUDA_TRY(h, upload(&h->d_lb, h_lb, (size_t)h->np), "upload bounds");
+    CUDA_TRY(h, upload(&h->d_ub, h_ub, (size_t)h->np), "upload bounds");
+    h->h_lb.assign(h_lb, h_lb + h->np); h->h_ub.assign(h_ub, h_ub + h->np);
+    h->bounded = true;
+    return B200LM_OK;
+}
 
 int b200lm_set_policy(b200lm_handle h, int policy) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
@@ -553,6 +584,14 @@ int b200lm_fit_batch_host(b200lm_handle h, int B,
     if (B == 0) return B200LM_OK;                 // empty batch
     if (B < 0 || !h_mean || !h_p0 || !h_x || !h_chi2 || !h_nit || !h_status)
         return set_error(h, B200LM_EINVAL, "NULL required argument");
+    if (h->bounded) {                             // scipy refuses a start outside the box (least_squares: "`x0` is infeasible.")
+        const long long nst = p0_stride ? (long long)B : 1;
+        for (long long b = 0; b < nst; ++b)
+            for (int j = 0; j < h->np; ++j) {
+                const double x = h_p0[b * p0_stride + j];
+                if (!(x >= h->h_lb[j] && x <= h->h_ub[j])) return set_error(h, B200LM_EINVAL, "`x0` is infeasible.");
+            }
+    }
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     const size_t np = h->np, N = h->N, nchiv = h->nchiv;
     const size_t n_mean = mean_stride ? (size_t)B * mean_stride : N;

@@ -33,6 +33,10 @@ struct b200lm_handle_s {
     int team_request = 0;       // 0: default policy; 1, 2, 4: warps per fit asked for by b200lm_set_team
     int policy = 0;             // trust-region decisions: 0 scipy TRF, 1 GSL trust/lm (b200lm_set_policy)
     int last_team = 1;          // warps per fit of the last fit_batch launch
+    // bound constraints (b200lm_set_bounds): device copies [np] and the host copies the host-buffer call checks p0 against
+    double* d_lb = nullptr; double* d_ub = nullptr;
+    std::vector<double> h_lb, h_ub;
+    bool bounded = false;
     // queue order (longest-expected fits first): key = chi2 at the start point, one evaluation per fit
     int order_request = -1;     // -1: default policy (by problem shape and batch size); 0: off; 1: on  (b200lm_set_order)
     int last_order = 0;         // 1 if the last fit_batch launch used an ordered queue

@@ -501,11 +501,13 @@ __device__ __forceinline__ double fast_rcp(double x) {
 // HALF: two systems per warp (np <= 16): lanes 0..15 use alpha_lo, lanes 16..31 alpha_hi, each half
 // with its own L^T (LT0 / LT1) -- the same instructions factor both (16-wide shuffles).
 // Per-lane outputs refer to the lane's own system; `ok` false = not numerically positive definite.
-template <int NP, int LDA, bool HALF>
+// EXTRA: the factored matrix is  d_i A_ij d_j + (alpha + ex_i) delta_ij  with a per-lane extra diagonal ex (the
+// Coleman-Li term of the bounded driver); it enters where alpha does, at the pivot.
+template <int NP, int LDA, bool HALF, bool EXTRA = false>
 __device__ __forceinline__ void ldl_solve(const double* A, const double* dsc, double* LT0, double* LT1, double* idg,
                                           double* colb, int lane, double alpha_lo, double alpha_hi, double gh_in,
                                           bool want_ratio, double& p_out, double& pn_out, double& w2_out,
-                                          double& minr_out, bool& ok_out) {
+                                          double& minr_out, bool& ok_out, double ex = 0.0) {
     static_assert(!HALF || NP <= 16, "two systems per warp need np <= 16");
     static_assert(NP <= 32, "one lane per row");
     constexpr int W = HALF ? 16 : 32;
@@ -521,7 +523,8 @@ __device__ __forceinline__ void ldl_solve(const double* A, const double* dsc, do
     const double di = dsc[ii];
 #pragma unroll
     for (int k = 0; k < NP; ++k) r[k] = A[ii * LDA + k] * di * dsc[k];
-    const double mdiag = fma(A[ii * LDA + ii] * di, di, alpha);               // diagonal entry of this lane's row
+    double mdiag = fma(A[ii * LDA + ii] * di, di, alpha);                     // diagonal entry of this lane's row
+    if constexpr (EXTRA) mdiag += ex;
     double myrcp = 1.0, mypiv = 1.0;
     bool ok = true;
     double b = act ? -gh : 0.0;
@@ -535,6 +538,10 @@ __device__ __forceinline__ void ldl_solve(const double* A, const double* dsc, do
         if (B200LM_LDL_VARIANT & 4) {
             __syncwarp();
             piv = cb[j] + alpha;
+            if constexpr (EXTRA) piv += __shfl_sync(B200LM_FULL, ex, j, W);
+        } else if constexpr (EXTRA) {
+            piv = __shfl_sync(B200LM_FULL, ((B200LM_LDL_VARIANT & 1) ? pivsrc : cj) + ex, j, W) + alpha;
+            __syncwarp();
         } else {
             piv = __shfl_sync(B200LM_FULL, (B200LM_LDL_VARIANT & 1) ? pivsrc : cj, j, W) + alpha;
             __syncwarp();
@@ -626,6 +633,23 @@ __device__ __noinline__ bool factor_solve(const double* A, const double* dsc, do
     return ok;
 }
 
+// the same with the per-lane extra diagonal ex (bounded driver)
+template <int NP, int LDA>
+__device__ __noinline__ bool factor_solve_ex(const double* A, const double* dsc, double* LT, double* idg, double* colb,
+                                             int lane, double alpha, double gh, double ex, double* p_out, double* res) {
+    __builtin_assume(__isShared(A));
+    __builtin_assume(__isShared(dsc));
+    __builtin_assume(__isShared(LT));
+    __builtin_assume(__isShared(idg));
+    __builtin_assume(__isShared(colb));
+    double p, pn, w2, minr;
+    bool ok;
+    ldl_solve<NP, LDA, false, true>(A, dsc, LT, LT, idg, colb, lane, alpha, alpha, gh, false, p, pn, w2, minr, ok, ex);
+    *p_out = ok ? p : 0.0;
+    res[0] = ok ? pn : 0.0; res[1] = ok ? w2 : 0.0; res[2] = 0.0;
+    return ok;
+}
+
 // Gauss-Newton step of the current outer iteration (alpha = 0), cached across rejected trials
 struct GNCache {
     bool valid, full_rank;
@@ -636,12 +660,18 @@ struct GNCache {
 // gh: lane-distributed scaled gradient.  Returns lane-distributed step; updates alpha.
 // (cf. scipy/optimize/_lsq/common.py: solve_lsq_trust_region, with the secular equation
 // evaluated through Cholesky factors instead of singular values.)
-template <class F>
-__device__ double solve_tr(WarpCtx<F>& c, double gh, double Delta, double& alpha, int& nfac, GNCache& gn, long long& fclk) {
+// EXTRA: Ah = d A d + diag(ex) (bounded driver: scipy's Coleman-Li augmented normal matrix).
+template <class F, bool EXTRA>
+__device__ __forceinline__ double solve_tr_impl(WarpCtx<F>& c, double gh, double Delta, double& alpha, int& nfac,
+                                                GNCache& gn, long long& fclk, double ex) {
     typedef FitLayout<F> Lay;
     constexpr int NP = Lay::NP, LDA = Lay::LDA;
     const int lane = c.lane;
     const bool act = lane < NP;
+    auto factor = [&](double a, double* p_out, double* r) -> bool {
+        if constexpr (EXTRA) return factor_solve_ex<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, a, gh, ex, p_out, r);
+        else return factor_solve<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, a, gh, false, p_out, r);
+    };
     double res[3];
     double p = 0.0, pn = 0.0;
     bool have_p = false;
@@ -653,7 +683,7 @@ __device__ double solve_tr(WarpCtx<F>& c, double gh, double Delta, double& alpha
         ++nfac;
         tried_warm = true;
         const long long tq = B200LM_CLOCK();
-        warm_ok = factor_solve<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, alpha, gh, false, &warm_p, res);
+        warm_ok = factor(alpha, &warm_p, res);
         fclk += B200LM_CLOCK() - tq;
         if (warm_ok) { warm_pn = res[0]; warm_w2 = res[1]; warm_phi = warm_pn - Delta; }
     }
@@ -661,7 +691,7 @@ __device__ double solve_tr(WarpCtx<F>& c, double gh, double Delta, double& alpha
     if (!gn.valid && need_gn) {
         ++nfac;
         const long long tq = B200LM_CLOCK();
-        gn.full_rank = factor_solve<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, 0.0, gh, false, &p, res);
+        gn.full_rank = factor(0.0, &p, res);
         fclk += B200LM_CLOCK() - tq;
         gn.p = p; gn.pn = res[0]; gn.w2 = res[1];
         gn.valid = true;
@@ -692,7 +722,7 @@ __device__ double solve_tr(WarpCtx<F>& c, double gh, double Delta, double& alpha
                 alpha = fmax(0.001 * alpha_upper, sqrt(alpha_lower * alpha_upper));
             ++nfac;
             const long long tq = B200LM_CLOCK();
-            ok = factor_solve<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, alpha, gh, false, &pt, res);
+            ok = factor(alpha, &pt, res);
             fclk += B200LM_CLOCK() - tq;
         }
         if (!ok) {
@@ -716,6 +746,11 @@ __device__ double solve_tr(WarpCtx<F>& c, double gh, double Delta, double& alpha
     pn = sqrt(warp_sum(act ? p * p : 0.0));
     if (pn > 0.0) p *= Delta / pn;
     return p;
+}
+
+template <class F>
+__device__ double solve_tr(WarpCtx<F>& c, double gh, double Delta, double& alpha, int& nfac, GNCache& gn, long long& fclk) {
+    return solve_tr_impl<F, false>(c, gh, Delta, alpha, nfac, gn, fclk, 0.0);
 }
 
 // ---------------------------------------------------------------------------
@@ -957,6 +992,147 @@ __device__ double covariance_from_qr(WarpCtx<F>& c, double* cov_out) {
 }
 
 // ---------------------------------------------------------------------------
+// bound constraints: scipy's trf_bounds restated on the warp (numpy model: tests/lm_model_bounded.py).
+// scipy/optimize/_lsq/trf.py: trf_bounds, select_step; common.py: CL_scaling_vector, step_size_to_bound,
+// intersect_trust_region, minimize_quadratic_1d, make_strictly_feasible.  One lane per parameter; idle lanes carry
+// x = s = 0 and an unbounded box.
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ double warp_min(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(B200LM_FULL, v, o));
+    return v;
+}
+
+// CL_scaling_vector: v = distance to the bound the anti-gradient points at (1 if none), dv = its derivative
+__device__ __forceinline__ void cl_scaling(double x, double g, double lb, double ub, double& v, double& dv) {
+    v = 1.0; dv = 0.0;
+    if (g < 0.0 && isfinite(ub)) { v = ub - x; dv = -1.0; }
+    if (g > 0.0 && isfinite(lb)) { v = x - lb; dv = 1.0; }
+}
+
+// make_strictly_feasible(x, lb, ub, rstep=1e-10): the start point of a bounded fit
+__device__ __forceinline__ double feasible_start(double x, double lb, double ub) {
+    const double lt = 1e-10 * fmax(1.0, fabs(lb)), ut = 1e-10 * fmax(1.0, fabs(ub));
+    const double ld = x - lb, ud = ub - x;
+    double xn = x;
+    if (isfinite(lb) && ld <= fmin(ud, lt)) xn = lb + lt;
+    if (isfinite(ub) && ud <= fmin(ld, ut)) xn = ub - ut;
+    if (xn < lb || xn > ub) xn = 0.5 * (lb + ub);
+    return xn;
+}
+
+// make_strictly_feasible(x, lb, ub, rstep=0): every trial point
+__device__ __forceinline__ double feasible_trial(double x, double lb, double ub) {
+    double xn = x;
+    if (x <= lb) xn = nextafter(lb, ub);
+    if (x >= ub) xn = nextafter(ub, lb);
+    if (xn < lb || xn > ub) xn = 0.5 * (lb + ub);
+    return xn;
+}
+
+// step_size_to_bound: the largest t with x + t s in the box (min over s_i != 0); hit = this lane reaches it
+__device__ __forceinline__ double step_to_bound(bool act, double x, double s, double lb, double ub, bool& hit) {
+    const bool nz = act && s != 0.0;
+    const double st = nz ? fmax((lb - x) / s, (ub - x) / s) : INFINITY;
+    const double m = warp_min(st);
+    hit = nz && st == m;
+    return m;
+}
+
+// minimize_quadratic_1d: argmin of a t^2 + b t + c over [lo, hi] -> (t, value)
+__device__ __forceinline__ double min_quad_1d(double a, double b, double lo, double hi, double c, double& val) {
+    double t = lo, y = lo * (a * lo + b) + c;
+    const double yh = hi * (a * hi + b) + c;
+    if (yh < y) { t = hi; y = yh; }
+    if (a != 0.0) {
+        const double e = -0.5 * b / a;
+        const double ye = e * (a * e + b) + c;
+        if (lo < e && e < hi && ye < y) { t = e; y = ye; }
+    }
+    val = y;
+    return t;
+}
+
+// select_step: the trust-region step p_h (scaled space, x = d x_h) if x + d p_h stays in the box; otherwise the best of
+// that step cut back to the box (times theta), its reflection off the box minimised along the reflected direction,
+// and the cut-back anti-gradient step, on q(s) = 1/2 s^T Ah s + gh^T s with Ah = d A d + diag(ex).  Returns the step
+// in x space; s_h becomes the step in scaled space, `predicted` = -q(s_h).  Scratch: c.idg.
+template <class F>
+__device__ double select_step(WarpCtx<F>& c, double x, double gh, double& s_h, double d, double ex, double Delta,
+                              double theta, double lb, double ub, double& predicted) {
+    typedef FitLayout<F> Lay;
+    constexpr int NP = Lay::NP, LDA = Lay::LDA;
+    const int lane = c.lane;
+    const bool act = lane < NP;
+    auto Ah = [&](double s) -> double {            // (Ah s)_lane
+        if (act) c.idg[lane] = d * s;
+        __syncwarp();
+        double t = 0.0;
+        if (act) {
+            const double* Ar = c.A + lane * LDA;
+#pragma unroll
+            for (int j = 0; j < NP; ++j) t = fma(Ar[j], c.idg[j], t);
+        }
+        __syncwarp();
+        return act ? fma(d, t, ex * s) : 0.0;
+    };
+    double p_h = act ? s_h : 0.0;
+    double p = d * p_h;
+    double qa = p_h * Ah(p_h), qb = gh * p_h;
+    double xo = (act && !(x + p >= lb && x + p <= ub)) ? 1.0 : 0.0;       // lanes whose step leaves the box
+    warp_sum3(qa, qb, xo);
+    if (xo == 0.0) { predicted = -(0.5 * qa + qb); return p; }
+    bool hit;
+    const double p_stride = step_to_bound(act, x, p, lb, ub, hit);
+    double r_h = hit ? -p_h : p_h;
+    const double r = d * r_h;
+    p *= p_stride; p_h *= p_stride;
+    qa *= p_stride * p_stride; qb *= p_stride;            // p_h^T Ah p_h and gh^T p_h of the cut-back step
+    double r_value = INFINITY, r_step = 0.0, r_hs = 0.0;
+    {
+        double ra = r_h * r_h, rb = p_h * r_h, pp = p_h * p_h;       // intersect_trust_region(p_h, r_h, Delta)
+        warp_sum3(ra, rb, pp);
+        const double cc = pp - Delta * Delta;
+        const double disc = sqrt(fmax(rb * rb - ra * cc, 0.0));
+        const double q = -(rb + copysign(disc, rb));
+        const double to_tr = fmax(q / ra, cc / q);
+        bool h2;
+        const double to_bound = step_to_bound(act, x + p, r, lb, ub, h2);
+        const double r_stride = fmin(to_bound, to_tr);
+        double lo = 0.0, hi = -1.0;
+        if (r_stride > 0.0) {
+            lo = (1.0 - theta) * p_stride / r_stride;
+            hi = r_stride == to_bound ? theta * to_bound : to_tr;
+        }
+        if (lo <= hi) {
+            const double Ar = Ah(r_h);
+            double a = r_h * Ar, b = gh * r_h + p_h * Ar, z = 0.0;
+            warp_sum3(a, b, z);
+            const double t = min_quad_1d(0.5 * a, b, lo, hi, 0.5 * qa + qb, r_value);
+            r_hs = fma(r_h, t, p_h);
+            r_step = d * r_hs;
+        }
+    }
+    const double p_value = 0.5 * theta * theta * qa + theta * qb;
+    double ag_h = act ? -gh : 0.0;
+    double ag_value, ag_stride;
+    {
+        const double Aag = Ah(ag_h);
+        double a = ag_h * Aag, b = gh * ag_h, gg = ag_h * ag_h;
+        warp_sum3(a, b, gg);
+        const double to_tr = Delta / sqrt(gg);
+        bool h3;
+        const double to_bound = step_to_bound(act, x, d * ag_h, lb, ub, h3);
+        const double hi = to_bound < to_tr ? theta * to_bound : to_tr;
+        ag_stride = min_quad_1d(0.5 * a, b, 0.0, hi, 0.0, ag_value);
+    }
+    if (p_value < r_value && p_value < ag_value) { s_h = theta * p_h; predicted = -p_value; return theta * p; }
+    if (r_value < p_value && r_value < ag_value) { s_h = r_hs; predicted = -r_value; return r_step; }
+    s_h = ag_h * ag_stride; predicted = -ag_value;
+    return d * ag_h * ag_stride;
+}
+
+// ---------------------------------------------------------------------------
 // the fit kernel
 // ---------------------------------------------------------------------------
 template <class F>
@@ -1015,7 +1191,8 @@ struct PhaseClock {
 
 // MODE selects what is COMPILED into a kernel (the trust-region loop is the hot code: every policy it does not run
 // would only cost registers and instruction cache):  0 = scipy TRF decisions (the default kernels),  1 = GSL trust/lm
-// decisions (b200lm_set_policy),  2 = no loop at all: finalisation of fits the wave kernel has already converged.
+// decisions (b200lm_set_policy),  2 = no loop at all: finalisation of fits the wave kernel has already converged,
+// 3 = scipy TRF with bound constraints (trf_bounds: Coleman-Li scaling, select_step; b200lm_set_bounds).
 template <class F, class EV, int MODE = 0>
 __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& P, int b,
                                         unsigned long long& tot_nfev, unsigned long long& tot_njev,
@@ -1028,6 +1205,13 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
         c.mean = ev.begin(c, P, b);
         const double* p0 = P.p0 + (size_t)b * P.p0_stride;
         if (act) c.p[lane] = p0[lane];
+        double lbi = -INFINITY, ubi = INFINITY;             // this lane's bounds (MODE 3)
+        if constexpr (MODE == 3) {
+            if (act) {
+                lbi = P.lb[lane]; ubi = P.ub[lane];
+                c.p[lane] = feasible_start(c.p[lane], lbi, ubi);
+            }
+        }
         __syncwarp();
 
         int cur = 0;                              // buffer holding J^T J, J^T r of the current point
@@ -1065,6 +1249,13 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
             if (sinv == 0.0) sinv = 1.0;
         }
         double t = act ? c.p[lane] * sinv : 0.0;
+        if constexpr (MODE == 3) {
+            // Delta0 = |x0 scale_inv / sqrt(v)|, v of the Coleman-Li scaling (scaled by scale_inv where it varies)
+            double v, dv;
+            cl_scaling(act ? c.p[lane] : 0.0, act ? c.g[lane] : 0.0, lbi, ubi, v, dv);
+            if (dv != 0.0) v *= sinv;
+            t = act ? t / sqrt(v) : 0.0;
+        }
         double Delta = sqrt(warp_sum(t * t));
         if (Delta == 0.0) Delta = 1.0;
         double alpha = 0.0;
@@ -1162,10 +1353,16 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
             sinv = diag;
         }
 
-        while (MODE == 0 && status == -2) {
+        // MODE 3 (bounds) is the same loop with scipy's trf_bounds changes: the gtol test on |g v|_inf, the scaling
+        // d = sqrt(v) / scale_inv, the Coleman-Li diagonal in the sub-problem, select_step, strictly feasible trials
+        while ((MODE == 0 || MODE == 3) && status == -2) {
             const double gi = act ? c.g[lane] : 0.0;
+            double v = 1.0, dv = 0.0;                              // Coleman-Li scaling (MODE 3)
+            const double xi = act ? c.p[lane] : 0.0;
+            if constexpr (MODE == 3) cl_scaling(xi, gi, lbi, ubi, v, dv);
             // |g|_inf and |x|^2 of the current point in one reduction (x does not change until a step is accepted)
             double xx = 0.0, g_norm = fabs(gi);
+            if constexpr (MODE == 3) g_norm = fabs(gi * v);
             {
                 const double pi_ = act ? c.p[lane] : 0.0;
                 xx = pi_ * pi_;
@@ -1174,7 +1371,14 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
             if (g_norm < P.gtol) { status = 1; break; }
             if (nfev >= P.maxit) { status = 0; break; }
             const double xthr = P.xtol * (P.xtol + sqrt(xx));      // xtol test: |step| < xtol (xtol + |x|)
-            const double d = 1.0 / sinv;
+            double d = 1.0 / sinv;
+            double ex = 0.0, theta = 0.0;                          // Coleman-Li diagonal, select_step's theta (MODE 3)
+            if constexpr (MODE == 3) {
+                if (dv != 0.0) v *= sinv;
+                ex = act ? gi * dv * d : 0.0;
+                d = act ? sqrt(v) * d : 0.0;
+                theta = fmax(0.995, 1.0 - g_norm);
+            }
             if (act) c.dsc[lane] = d;
             __syncwarp();
             const double gh = d * gi;
@@ -1188,13 +1392,24 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
                 // two shifts per round pay off where the factorisation dominates a trial (np = 12..16: +8 % on
                 // C3); for small np the extra control flow and code size cost more than they save (C4, np = 6:
                 // -10 %), so those kernels do not even contain the dual path
-                if constexpr (NP >= 12 && NP <= 16) {
+                if constexpr (MODE == 3) {
+                    sh = solve_tr_impl<F, true>(c, gh, Delta, alpha, nfac, gn, pk.fact, ex);
+                } else if constexpr (NP >= 12 && NP <= 16) {
                     sh = (P.dual_from >= 0 && nfev >= P.dual_from) ? solve_tr_dual<F>(c, gh, Delta, alpha, nfac, gn, lm, pk.fact)
                                                                    : solve_tr<F>(c, gh, Delta, alpha, nfac, gn, pk.fact);
                 } else {
                     sh = solve_tr<F>(c, gh, Delta, alpha, nfac, gn, pk.fact);
                 }
                 pk.solve += B200LM_CLOCK() - t_s0;
+                double predicted, step2, sh2;
+                if constexpr (MODE == 3) {
+                    const double step = select_step<F>(c, xi, gh, sh, d, ex, Delta, theta, lbi, ubi, predicted);
+                    if (act) c.pn[lane] = feasible_trial(xi + step, lbi, ubi);
+                    step2 = step * step;
+                    sh2 = act ? sh * sh : 0.0;
+                    double z = 0.0;
+                    warp_sum3(step2, sh2, z);
+                } else {
                 const double step = act ? d * sh : 0.0;
                 if (act) { c.pn[lane] = c.p[lane] + step; c.idg[lane] = step; }
                 __syncwarp();
@@ -1216,10 +1431,11 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
                     As = (a0 + a1) + (a2 + a3);
                 }
                 // predicted reduction, |step|^2 and |sh|^2 in ONE reduction
-                double predicted = act ? -step * (0.5 * As + gi) : 0.0;
-                double step2 = step * step;
-                double sh2 = act ? sh * sh : 0.0;
+                predicted = act ? -step * (0.5 * As + gi) : 0.0;
+                step2 = step * step;
+                sh2 = act ? sh * sh : 0.0;
                 warp_sum3(predicted, step2, sh2);
+                }
                 __syncwarp();
                 // Speculative evaluation: residual AND Jacobian / normal equations at the trial
                 // point, into the other buffer.  ~87 % of the trials are accepted, and then no
@@ -1269,7 +1485,13 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
             }
             if (term != -2) {
                 // the solver behind the reference re-tests gtol before leaving (trf.py loop head)
-                const double gf = warp_max(act ? fabs(c.g[lane]) : 0.0);
+                double gl = act ? fabs(c.g[lane]) : 0.0;
+                if constexpr (MODE == 3) {
+                    double v2, dv2;
+                    cl_scaling(act ? c.p[lane] : 0.0, act ? c.g[lane] : 0.0, lbi, ubi, v2, dv2);
+                    gl *= v2;
+                }
+                const double gf = warp_max(gl);
                 status = gf < P.gtol ? 1 : term;
             }
         }
@@ -1280,7 +1502,8 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
         // from the stationary point (so does the reference's solver).  Undamped Gauss-Newton
         // steps, accepted on the decrease of the Newton decrement instead of the cost, take the
         // solution on to the gradient's rounding level.
-        if (status >= 1 && P.polish > 0) {
+        // (not with bounds: undamped steps would leave the box)
+        if (MODE != 3 && status >= 1 && P.polish > 0) {
             // Newton decrement dec = g^T (J^T J)^-1 g = predicted decrease of chi2; sqrt(dec) is
             // the distance to the stationary point in standard deviations.
             const double d = 1.0 / sinv;
@@ -1473,6 +1696,7 @@ cudaError_t launch_fit(FitParams P, int sm_count, size_t smem_budget, cudaStream
     cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li);
     if (e != cudaSuccess) return e;
     if (P.finalize_only) return launch_fit_mode<F, 2>(P, li, stream);
+    if (P.bounded) return launch_fit_mode<F, 3>(P, li, stream);
     if (P.policy == 1) return launch_fit_mode<F, 1>(P, li, stream);
     return launch_fit_mode<F, 0>(P, li, stream);
 }

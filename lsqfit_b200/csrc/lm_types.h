@@ -74,6 +74,10 @@ struct FitParams {
                                 // finalisation pass (which then needs no evaluation of its own)
     const int* order;           // optional: the queue hands out fit order[i] instead of fit i (longest-expected first)
     unsigned long long* stats;  // [0] total nfev, [1] total jacobian evals, [2] total factorisations
+    // ---- bound constraints (last: the offsets of every field above are those of the kernels without bounds) ----
+    const double* lb;           // [np] lower bounds (-inf: none), device parameter order
+    const double* ub;           // [np] upper bounds (+inf: none)
+    int bounded;                // 1: scipy's trf_bounds decisions (fit_kernel<F, 3>); lb / ub are set
 };
 
 }  // namespace b200lm

@@ -125,16 +125,43 @@ class Plan(object):
         _cabi.check(_cabi.lib.b200lm_set_policy(self._h, POLICY[policy]), self._h)
         return SCALER[scaler]
 
+    def _bounds(self, bounds):
+        """(lb, ub) -> two contiguous float64 host arrays of np entries (scalars broadcast)."""
+        lb, ub = (np.array(np.broadcast_to(np.asarray(b, dtype=np.float64), (self.np,))) for b in bounds)
+        if np.isnan(lb).any() or np.isnan(ub).any():
+            raise ValueError("bounds must not be NaN")
+        if not np.all(lb < ub):
+            raise ValueError("Each lower bound must be strictly less than each upper bound.")     # scipy least_squares
+        return lb, ub
+
+    def _launch_bounded(self, bounds, launch):
+        """Run ``launch()`` with the box set on the handle (b200lm_set_bounds); the plan is cached and shared (the
+        parent fit, other drivers), so the bounds are cleared again afterwards."""
+        if bounds is None:
+            return launch()
+        lb, ub = bounds
+        _cabi.check(_cabi.lib.b200lm_set_bounds(self._h, lb.ctypes.data, ub.ctypes.data), self._h)
+        try:
+            return launch()
+        finally:
+            _cabi.lib.b200lm_set_bounds(self._h, None, None)
+
     def fit_batch(self, mean, p0, tol=1e-8, maxit=1000, scaler="more", B=None,
-                  want_cov=True, want_fJ=False, out=None, polish=0, policy="trf"):
+                  want_cov=True, want_fJ=False, out=None, polish=0, policy="trf", bounds=None):
         """Fit B problems on the device; inputs may be numpy arrays or device tensors.
 
         mean: [B, N] or [N] (shared);  p0: [B, np] or [np] (shared).
+        bounds: None or (lb, ub) in device parameter order, scipy's ``bounds`` (±inf: none); p0 must lie in the box.
         Returns a BatchResult of device tensors (no host synchronisation)."""
         xtol, gtol, ftol = normalize_tol(tol)
         sc = self._set_policy(policy, scaler)
         tm, sm = self._dev(mean, self.N)
         tp, sp = self._dev(p0, self.np)
+        if bounds is not None:
+            bounds = self._bounds(bounds)
+            tl, tu = (torch.as_tensor(b).to(self.tdev) for b in bounds)
+            if not bool(torch.all((tp >= tl) & (tp <= tu))):           # one reduction (scipy: "`x0` is infeasible.")
+                raise ValueError("`x0` is infeasible.")
         if B is None:
             B = tm.shape[0] if sm else (tp.shape[0] if sp else 1)
         if (sm and tm.shape[0] != B) or (sp and tp.shape[0] != B):
@@ -150,17 +177,18 @@ class Plan(object):
                 torch.empty((B, self.nchiv), **kw) if want_fJ else None,
                 torch.empty((B, self.nchiv, self.np), **kw) if want_fJ else None)
         ptr = lambda t: t.data_ptr() if t is not None else None
-        _cabi.check(_cabi.lib.b200lm_fit_batch(
+        self._launch_bounded(bounds, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch(
             self._h, B, tm.data_ptr(), sm, tp.data_ptr(), sp, xtol, gtol, ftol, int(maxit), sc, int(polish),
             out.x.data_ptr(), out.chi2.data_ptr(), ptr(out.cov), out.logdet.data_ptr(),
-            out.nit.data_ptr(), out.status.data_ptr(), ptr(out.f), ptr(out.J), self._stream()), self._h)
+            out.nit.data_ptr(), out.status.data_ptr(), ptr(out.f), ptr(out.J), self._stream()), self._h))
         out._keep = (tm, tp)        # keep inputs alive until the stream has consumed them
         return out
 
     def fit_batch_host(self, mean, p0, tol=1e-8, maxit=1000, scaler="more", want_cov=True,
-                       want_fJ=False, out=None, polish=0, policy="trf"):
+                       want_fJ=False, out=None, polish=0, policy="trf", bounds=None):
         """Same fit through the host-buffer C entry point: numpy in, numpy out.
-        ``out`` may hold preallocated arrays (dict with keys x, chi2, cov, logdet, nit, status)."""
+        ``out`` may hold preallocated arrays (dict with keys x, chi2, cov, logdet, nit, status).
+        ``bounds`` as for fit_batch."""
         xtol, gtol, ftol = normalize_tol(tol)
         sc = self._set_policy(policy, scaler)
         # the C entry point reads raw host pointers: dtype, contiguity and shapes are checked HERE
@@ -198,11 +226,15 @@ class Plan(object):
                         and a.flags["WRITEABLE"] and tuple(a.shape) == shp):
                     raise ValueError("out[%r] must be a writable C-contiguous %s array of shape %s"
                                      % (k, np.dtype(dt).name, shp))
+        if bounds is not None:
+            bounds = self._bounds(bounds)
+            if not np.all((p0 >= bounds[0]) & (p0 <= bounds[1])):
+                raise ValueError("`x0` is infeasible.")
         ptr = lambda a: a.ctypes.data if a is not None else None
-        _cabi.check(_cabi.lib.b200lm_fit_batch_host(
+        self._launch_bounded(bounds, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch_host(
             self._h, B, mean.ctypes.data, sm, p0.ctypes.data, sp, xtol, gtol, ftol, int(maxit), sc, int(polish),
             ptr(out["x"]), ptr(out["chi2"]), ptr(out.get("cov")), ptr(out["logdet"]),
-            ptr(out["nit"]), ptr(out["status"]), ptr(out.get("f")), ptr(out.get("J"))), self._h)
+            ptr(out["nit"]), ptr(out["status"]), ptr(out.get("f")), ptr(out.get("J"))), self._h))
         return out
 
     def last_stats(self):

@@ -230,13 +230,24 @@ class nonlinear_fit(object):
         # fastest on saturated batches (10^5 ... 10^6 copies of a small model); see b200lm_set_team
         kernel = args.pop("kernel", None)
         kernel = 32 if kernel == "wave" else kernel
+        if args.get("loss", "linear") != "linear":
+            raise ValueError("batched fits with a robust loss (loss=%r) are not built: fit the copies one at a time "
+                             "(fitter='b200_dense')" % (args["loss"],))
+        # scipy's bounds=(lower, upper) in this fit's parameter order -> device order (as the single-fit path does)
+        bounds = args.pop("bounds", None)
+        if bounds is not None:
+            from .engine import POLICY
+            if POLICY.get(args.get("policy", "trf")) == 1:
+                raise ValueError("b200_lm: policy='gsl' has no bound constraints")
+            bounds = tuple(self._spec.to_device(np.broadcast_to(np.asarray(b, dtype=float), (self._spec.np,)))
+                           for b in bounds)
         if kernel is not None:
             plan.set_team(int(kernel))
         try:
             out = plan.fit_batch(means, p0, tol=self.tol if tol is None else tol,
                                  maxit=self.maxit if maxit is None else maxit, want_cov=want_cov,
                                  scaler=args.pop("scaler", "more"), polish=args.pop("polish", 0),
-                                 policy=args.pop("policy", "trf"))
+                                 policy=args.pop("policy", "trf"), bounds=bounds)
         finally:
             if kernel is not None:
                 plan.set_team(0)                 # (the plan is cached and shared: back to the default policy)

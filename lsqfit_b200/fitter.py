@@ -156,7 +156,8 @@ class b200_lm(object):
                   dogleg / lmaccel methods only) are accepted.
       ``scaler``  'more' (default) | 'levenberg' | 'marquardt' (gsl policy only)   (_gsl.pyx:621-653)
       ``bounds``  (lower, upper): scipy's bound constraints (``lsqfit.scipy_least_squares(bounds=...)``); such fits run on
-                  the single-fit path (lsqfit_b200/dense.py) with scipy trf's reflective step selection.
+                  the single-fit path (lsqfit_b200/dense.py) with scipy trf's reflective step selection; the batch
+                  drivers of the fit (bootstrapped_fits, simulated_fits) fit their copies with the same box on the device.
       ``loss``, ``f_scale``  scipy's robust loss functions ('linear' | 'huber' | 'soft_l1' | 'cauchy' | 'arctan';
                   ``lsqfit.scipy_least_squares(loss=...)``, src/lsqfit/_scipy.py:77): also on the single-fit path.
       ``method``  None | 'trf' (scipy's other methods are different solvers and are refused).
