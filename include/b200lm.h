@@ -49,10 +49,28 @@ int b200lm_device_count(void);
 /* ---- device functor registry ---------------------------------------------------------
  * The reference receives the fit function as an opaque Python callable
  * (src/lsqfit/__init__.py:566, 1997-2042: flatfcn).  Here the model is one of a registry
- * of CUDA device functors, selected by family name + number of parameters. */
+ * of CUDA device functors, selected by family name + number of parameters.
+ * The registry lists the built-in functors first (families 0 ... 30, always at the same
+ * indices), then the entries of run-time plug-ins in load order.  The registry only grows;
+ * reading and appending are thread-safe. */
 int b200lm_functor_count(void);
 int b200lm_functor_info(int i, int* family, int* np, int* nx, const char** name);
 int b200lm_functor_family(const char* name);            /* family id, or B200LM_ENOFUNCTOR */
+
+/* Add the functors of a plug-in to the registry: a shared object compiled from the library's
+ * own headers with its flags (lsqfit_b200.cuda_functor generates and builds one from a model
+ * body) that exports b200lm_plugin_entries (csrc/registry.h).  The plug-in is dlopen'ed and
+ * its ABI record checked against the library (version, sizeof(FitParams),
+ * sizeof(FunctorEntry), digest of the headers and flags): a mismatch is B200LM_EINVAL with
+ * the field named.  All entries of one plug-in share one model name, np in 1..25, nx in 1..8;
+ * they get the family *family_out, numbered from B200LM_USER_FAMILY0 upward in load order.
+ * A name that a built-in functor or another plug-in already uses is B200LM_EINVAL; loading
+ * the same name from the same model source again returns its family.  Plug-ins are never
+ * unloaded (plans hold their launchers).  Needs no GPU. */
+#define B200LM_USER_FAMILY0 1000
+#define B200LM_USER_MAX_NP 25
+#define B200LM_USER_MAX_NX 8
+int b200lm_load_functors(const char* path, int* family_out);
 
 /* ---- plan ---------------------------------------------------------------------------
  * One handle per (functor, ny, np, device).  noprior != 0 means fits without a prior

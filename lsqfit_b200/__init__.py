@@ -10,6 +10,7 @@ creating a plan without a CUDA device raises.
 from . import _cabi                                    # noqa: F401  (fails loudly if the .so is missing)
 from ._cabi import B200LMError
 from .functors import Functor, FAMILY, NIST_FORM
+from .user_functor import cuda_functor, UserFunctor
 from .engine import Plan, BatchResult, STOPPING_CRITERION, normalize_tol
 from .whiten import PDF, cov_blocks
 from .fitter import b200_lm, ChivSpec, DeviceChiv

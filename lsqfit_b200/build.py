@@ -36,8 +36,15 @@ def _headers_digest():
             if f.endswith((".h", ".cuh")):
                 with open(os.path.join(d, f), "rb") as fh:
                     h.update(fh.read())
-    h.update(" ".join(ARCH + CFLAGS).encode())
+    # the include path in its in-tree form: a tree built in one place and run from another keeps its digest
+    h.update(" ".join(ARCH + CFLAGS).replace(INCLUDE, "include").encode())
     return h.hexdigest()
+
+
+def digest_define(hdig):
+    """the -D flag that compiles the headers digest into the library (capi.cu checks plug-ins against it) and into
+    every functor plug-in (lsqfit_b200/user_functor.py)"""
+    return '-DB200LM_HEADERS_DIGEST="%s"' % hdig
 
 
 def _compile(src, hdig, force):
@@ -47,7 +54,7 @@ def _compile(src, hdig, force):
         dig = hashlib.sha256(fh.read() + hdig.encode()).hexdigest()
     if not force and os.path.exists(obj) and os.path.exists(stamp) and open(stamp).read() == dig:
         return obj, False
-    cmd = [NVCC] + ARCH + CFLAGS + ["-c", os.path.join(CSRC, src), "-o", obj]
+    cmd = [NVCC] + ARCH + CFLAGS + [digest_define(hdig), "-c", os.path.join(CSRC, src), "-o", obj]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (src, r.stdout, r.stderr))

@@ -5,8 +5,12 @@
 #include <cstring>
 #include <string>
 #include <vector>
+#include <deque>
+#include <map>
+#include <mutex>
 #include <algorithm>
 #include <cuda_runtime.h>
+#include <dlfcn.h>
 #include <stdlib.h>
 #include "../../include/b200lm.h"
 #include "handle.h"
@@ -46,19 +50,23 @@ void fill_params(b200lm_handle_s* h, FitParams& P) {
 }  // namespace b200lm
 
 
-static std::vector<FunctorEntry>& registry() {
-    static std::vector<FunctorEntry> r;
-    if (r.empty()) {
-        int n = 0;
-        const FunctorEntry* e;
-        e = registry_multiexp(&n); r.insert(r.end(), e, e + n);
-        e = registry_multiexp_b(&n); r.insert(r.end(), e, e + n);
-        e = registry_nist_a(&n);   r.insert(r.end(), e, e + n);
-        e = registry_nist_b(&n);   r.insert(r.end(), e, e + n);
-        e = registry_misc(&n);     r.insert(r.end(), e, e + n);
-        e = registry_misc_b(&n);   r.insert(r.end(), e, e + n);
-        e = registry_poly_b(&n);   r.insert(r.end(), e, e + n);
-    }
+// The registry: the built-in tables in a fixed order, then the entries of run-time plug-ins (b200lm_load_functors) in
+// load order.  A deque: handles keep pointers to their entry, and appending must not move the others.  Every read
+// and every append holds g_registry_mu.
+static std::mutex g_registry_mu;
+
+static std::deque<FunctorEntry>& registry() {
+    static std::deque<FunctorEntry> r = [] {
+        std::deque<FunctorEntry> d;
+        const FunctorEntry* (*tables[])(int*) = {registry_multiexp, registry_multiexp_b, registry_nist_a,
+                                                  registry_nist_b, registry_misc, registry_misc_b, registry_poly_b};
+        for (auto t : tables) {
+            int n = 0;
+            const FunctorEntry* e = t(&n);
+            d.insert(d.end(), e, e + n);
+        }
+        return d;
+    }();
     return r;
 }
 
@@ -157,9 +165,13 @@ int b200lm_device_count(void) {
     return n;
 }
 
-int b200lm_functor_count(void) { return (int)registry().size(); }
+int b200lm_functor_count(void) {
+    std::lock_guard<std::mutex> lock(g_registry_mu);
+    return (int)registry().size();
+}
 
 int b200lm_functor_info(int i, int* family, int* np, int* nx, const char** name) {
+    std::lock_guard<std::mutex> lock(g_registry_mu);
     auto& r = registry();
     if (i < 0 || i >= (int)r.size()) return set_error(nullptr, B200LM_EINVAL, "functor index out of range");
     if (family) *family = r[i].family;
@@ -171,8 +183,84 @@ int b200lm_functor_info(int i, int* family, int* np, int* nx, const char** name)
 
 int b200lm_functor_family(const char* name) {
     if (!name) return B200LM_EINVAL;
+    std::lock_guard<std::mutex> lock(g_registry_mu);
     for (auto& e : registry()) if (strcmp(e.name, name) == 0) return e.family;
     return set_error(nullptr, B200LM_ENOFUNCTOR, std::string("unknown functor family: ") + name);
+}
+
+#ifndef B200LM_HEADERS_DIGEST
+#error "B200LM_HEADERS_DIGEST must be defined (lsqfit_b200/build.py passes the digest of the headers and flags)"
+#endif
+
+int b200lm_load_functors(const char* path, int* family_out) {
+    if (!path || !family_out) return set_error(nullptr, B200LM_EINVAL, "NULL argument");
+    const std::string where = std::string("functor plug-in ") + path + ": ";
+    // never dlclose'd: plans created on its entries hold its launchers
+    void* so = dlopen(path, RTLD_NOW | RTLD_LOCAL);
+    if (!so) {
+        const char* m = dlerror();
+        return set_error(nullptr, B200LM_EINVAL, where + (m ? m : "dlopen failed"));
+    }
+    auto entries_fn = (b200lm_plugin_entries_fn)dlsym(so, "b200lm_plugin_entries");
+    if (!entries_fn) return set_error(nullptr, B200LM_EINVAL, where + "no symbol b200lm_plugin_entries");
+    b200lm_plugin_abi abi;
+    memset(&abi, 0, sizeof abi);
+    const FunctorEntry* e = nullptr;
+    int n = 0;
+    if (entries_fn(&e, &n, &abi) != 0 || !e || n < 1) return set_error(nullptr, B200LM_EINVAL, where + "no entries");
+    abi.headers[sizeof abi.headers - 1] = 0;
+    abi.model[sizeof abi.model - 1] = 0;
+    auto mismatch = [&](const char* field, const std::string& got, const std::string& want) {
+        return set_error(nullptr, B200LM_EINVAL, where + "ABI mismatch in " + field + ": plug-in " + got +
+                                                 ", library " + want + " (rebuild the plug-in)");
+    };
+    if (abi.version != B200LM_VERSION)
+        return mismatch("version", std::to_string(abi.version), std::to_string(B200LM_VERSION));
+    if (abi.fitparams_size != (int)sizeof(FitParams))
+        return mismatch("fitparams_size", std::to_string(abi.fitparams_size), std::to_string(sizeof(FitParams)));
+    if (abi.entry_size != (int)sizeof(FunctorEntry))
+        return mismatch("entry_size", std::to_string(abi.entry_size), std::to_string(sizeof(FunctorEntry)));
+    if (strcmp(abi.headers, B200LM_HEADERS_DIGEST) != 0) return mismatch("headers", abi.headers, B200LM_HEADERS_DIGEST);
+    if (!e[0].name || !e[0].name[0] || strlen(e[0].name) > 64)
+        return set_error(nullptr, B200LM_EINVAL, where + "bad model name");
+    const std::string name = e[0].name;
+    for (int i = 0; i < n; ++i) {
+        const FunctorEntry& f = e[i];
+        char buf[160];
+        snprintf(buf, sizeof buf, "entry %d (np=%d, nx=%d): ", i, f.np, f.nx);
+        if (!f.name || name != f.name) return set_error(nullptr, B200LM_EINVAL, where + buf + "one model name per plug-in");
+        if (f.np < 1 || f.np > B200LM_USER_MAX_NP || f.nx < 1 || f.nx > B200LM_USER_MAX_NX)
+            return set_error(nullptr, B200LM_EINVAL, where + buf + "np must be in 1..25 and nx in 1..8");
+        if (!f.fit || !f.resjac || !f.per_warp_bytes || !f.model_rows)
+            return set_error(nullptr, B200LM_EINVAL, where + buf + "missing launcher");
+        for (int j = 0; j < i; ++j)
+            if (e[j].np == f.np) return set_error(nullptr, B200LM_EINVAL, where + buf + "np listed twice");
+    }
+    // name -> (family, model digest) of every plug-in loaded so far; names of plug-in entries are owned here
+    static std::map<std::string, std::pair<int, std::string>> loaded;
+    static std::deque<std::string> names;
+    std::lock_guard<std::mutex> lock(g_registry_mu);
+    auto& r = registry();
+    auto it = loaded.find(name);
+    if (it != loaded.end()) {
+        if (it->second.second != abi.model)
+            return set_error(nullptr, B200LM_EINVAL, where + "the name '" + name + "' is used by a different plug-in");
+        *family_out = it->second.first;
+        return B200LM_OK;
+    }
+    for (const auto& f : r)
+        if (name == f.name) return set_error(nullptr, B200LM_EINVAL, where + "the name '" + name + "' is a built-in functor");
+    const int family = B200LM_USER_FAMILY0 + (int)loaded.size();
+    names.push_back(name);
+    for (int i = 0; i < n; ++i) {
+        FunctorEntry f = e[i];
+        f.family = family;
+        f.name = names.back().c_str();
+        r.push_back(f);
+    }
+    loaded[name] = std::make_pair(family, std::string(abi.model));
+    *family_out = family;
+    return B200LM_OK;
 }
 
 int b200lm_create(int family, int ny, int np, int nx, int noprior, int device, b200lm_handle* out) {
@@ -180,7 +268,10 @@ int b200lm_create(int family, int ny, int np, int nx, int noprior, int device, b
     *out = nullptr;
     if (ny <= 0 || np <= 0) return set_error(nullptr, B200LM_EINVAL, "ny and np must be positive");
     const FunctorEntry* fe = nullptr;
-    for (auto& e : registry()) if (e.family == family && e.np == np) { fe = &e; break; }
+    {
+        std::lock_guard<std::mutex> lock(g_registry_mu);
+        for (auto& e : registry()) if (e.family == family && e.np == np) { fe = &e; break; }
+    }
     if (!fe) {
         char buf[128];
         snprintf(buf, sizeof buf, "no device functor for family %d with np=%d", family, np);

@@ -37,6 +37,20 @@ const FunctorEntry* registry_poly_b(int* n);
 
 }  // namespace b200lm
 
+// Run-time plug-ins (b200lm_load_functors, lsqfit_b200/user_functor.py): a shared object built from the same headers
+// and flags as the library exports
+//     extern "C" int b200lm_plugin_entries(const b200lm::FunctorEntry** out, int* n, b200lm_plugin_abi* abi);
+// which fills the record below and returns 0.  The library copies the entries only when every field of the record
+// matches its own: the entries hold launchers that take FitParams by value.
+struct b200lm_plugin_abi {
+    int version;               // B200LM_VERSION
+    int fitparams_size;        // sizeof(b200lm::FitParams)
+    int entry_size;            // sizeof(b200lm::FunctorEntry)
+    char headers[72];          // B200LM_HEADERS_DIGEST: sha256 of the headers and compiler flags (build.py)
+    char model[72];            // digest of the plug-in's model source: the same name from the same source is one family
+};
+typedef int (*b200lm_plugin_entries_fn)(const b200lm::FunctorEntry** out, int* n, b200lm_plugin_abi* abi);
+
 #ifdef B200LM_DEFINE_ENTRIES
 #include "lm_kernel.cuh"
 #include "lm_team.cuh"

@@ -163,17 +163,25 @@ _HOST = dict(
 )
 
 
+# name -> UserFunctor of every model loaded at run time (lsqfit_b200/user_functor.py: cuda_functor)
+USER = {}
+
+
 class Functor(object):
     """A registered device model; also callable on the host as ``fcn(x, p)``.
 
     ``Functor('multiexp')`` works for any parameter count the device registry was
     compiled for (``lsqfit_b200.available()``); the count is taken from ``p0`` / the
-    prior when a fit is set up.
+    prior when a fit is set up.  The name of a model loaded with ``cuda_functor`` resolves too.
     """
 
     def __init__(self, name):
+        if name in USER:
+            u = USER[name]
+            self.name, self.family, self.nx, self._host = u.name, u.family, u.nx, u._host
+            return
         if name not in FAMILY:
-            raise ValueError("unknown functor family: %s (known: %s)" % (name, ", ".join(sorted(FAMILY))))
+            raise ValueError("unknown functor family: %s (known: %s)" % (name, ", ".join(sorted(FAMILY) + sorted(USER))))
         self.name = name
         self.family = FAMILY[name]
         self.nx = NX.get(name, 1)
