@@ -96,6 +96,27 @@ int b200lm_set_weights(b200lm_handle h, int ndiag, const int* h_diag_idx, const 
                        const int* h_blk_idx, const double* h_blk_w);
 int b200lm_nchiv(b200lm_handle h);
 
+/* ---- fit windows ---------------------------------------------------------------------------
+ * nwin problems that share the plan's functor, np, x grid [ny][nx] and y(+)prior layout, each with its own data rows
+ * and whitening (a fit-window scan: one model fitted to many ranges of the same data).  The arrays hold the windows one
+ * after the other, each with the meaning of b200lm_set_weights: h_ndiag[w] and h_nblk[w] entries of window w, then
+ * the next window's; indices address the FULL y(+)prior vector.  A window lists every prior entry and its own data
+ * rows exactly once and no other data row (at least one); every window is validated as b200lm_set_weights validates a
+ * description, and errors name the window.  Host pointers; copied once.
+ * Replaces the plan's weights; b200lm_set_weights switches the plan back.  With windows set:
+ *   - b200lm_fit_batch / _host fit B = nwin x copies (B % nwin != 0: EINVAL).  Fit b belongs to window b / copies; its
+ *     means are row b % copies of d_mean (mean_stride; 0 = shared), its start row b / copies of d_p0 (p0_stride;
+ *     0 = shared).  One warp per fit: the queue order (set_order, B200LM_ORDER) and the team / wave choice
+ *     (set_team, B200LM_TEAM) are ignored and b200lm_last_team reports 1.
+ *   - b200lm_nchiv returns the largest window nchiv: the row stride of d_f and d_J.  A fit's rows are in its window's
+ *     chiv order and zero beyond that window's own nchiv (b200lm_window_nchiv).
+ *   - the GSL policy, bounds, b200lm_residual_jacobian and b200lm_propagate return EINVAL. */
+int b200lm_set_windows(b200lm_handle h, int nwin, const int* h_ndiag, const int* h_diag_idx, const double* h_diag_w,
+                       const int* h_nblk, const int* h_blk_nin, const int* h_blk_nout,
+                       const int* h_blk_idx, const double* h_blk_w);
+/* residuals of every window: h_nchiv [nwin] (EINVAL if no windows are set) */
+int b200lm_window_nchiv(b200lm_handle h, int* h_nchiv);
+
 /* ---- the fit --------------------------------------------------------------------------
  * Replaces   fit = FITTERS[fitter](p0, nf, chiv, tol=tol, maxit=maxit, **fitterargs)
  * (src/lsqfit/__init__.py:662-664) and the plugin behind it (src/lsqfit/_scipy.py:115-181,

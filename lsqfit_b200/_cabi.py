@@ -44,6 +44,9 @@ SIGNATURES = {
     "b200lm_set_weights": (C.c_int, [handle_t, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200lm_nchiv": (C.c_int, [handle_t]),
+    "b200lm_set_windows": (C.c_int, [handle_t, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200lm_window_nchiv": (C.c_int, [handle_t, C.c_void_p]),
     "b200lm_fit_batch": (C.c_int, [handle_t, C.c_int, C.c_void_p, C.c_longlong, C.c_void_p, C.c_longlong,
                                    C.c_double, C.c_double, C.c_double, C.c_int, C.c_int, C.c_int,
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

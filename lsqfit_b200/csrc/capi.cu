@@ -153,6 +153,84 @@ static cudaError_t upload(T** dst, const T* src, size_t n) {
     return cudaMemcpy(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice);
 }
 
+// One whitening description (the arguments of b200lm_set_weights), checked and laid out for the kernels.
+// allowed[i]: 0 = entry i of y(+)prior must not appear, 1 = may appear, 2 = must appear; each appears at most once.
+// Returns "" or the error ("size": a block too large for the shared-memory plan).
+struct WeightTables {
+    std::vector<int> fn_idx, pr_idx, blk_idx;
+    std::vector<double> fn_w, pr_w, wt, wt2;
+    std::vector<BlockDesc> blk;
+    int nchiv = 0, ndata = 0;
+    long long nw = 0;              // doubles of blk_w read
+};
+
+static std::string parse_weights(b200lm_handle_s* h, const std::vector<char>& allowed, int ndiag, const int* diag_idx,
+                                 const double* diag_w, int nblk, const int* blk_nin, const int* blk_nout,
+                                 const int* blk_idx, const double* blk_w, WeightTables& t) {
+    if (ndiag < 0 || nblk < 0 || (ndiag > 0 && (!diag_idx || !diag_w)) ||
+        (nblk > 0 && (!blk_nin || !blk_nout || !blk_idx || !blk_w)))
+        return "bad weight description";
+    const int N = h->N;
+    std::vector<char> seen(N, 0);
+    auto take = [&](int idx) {
+        if (idx < 0 || idx >= N || seen[idx] || !allowed[idx]) return false;
+        seen[idx] = 1;
+        if (idx < h->ny) ++t.ndata;
+        return true;
+    };
+    // 1x1 blocks: data rows first (in the given order), then prior rows -- this is the
+    // reference's chiv order because gvar lists 1x1 indices in ascending order.
+    bool prior_seen = false;
+    for (int i = 0; i < ndiag; ++i) {
+        const int idx = diag_idx[i];
+        if (!take(idx)) return "diag index out of range or repeated";
+        if (idx < h->ny) {
+            if (prior_seen) return "diag indices must list data rows before prior rows";
+            t.fn_idx.push_back(idx); t.fn_w.push_back(diag_w[i]);
+        } else { prior_seen = true; t.pr_idx.push_back(idx); t.pr_w.push_back(diag_w[i]); }
+    }
+    t.blk.resize(nblk);
+    int idx_off = 0, chiv_off = ndiag;
+    for (int k = 0; k < nblk; ++k) {
+        const int nin = blk_nin[k], nout = blk_nout[k];
+        if (nin <= 0 || nout < 0 || nout > nin) return "bad block shape";
+        for (int j = 0; j < nin; ++j)
+            if (!take(blk_idx[idx_off + j])) return "block index out of range or repeated";
+        BlockDesc& b = t.blk[k];
+        b.n_in = nin; b.n_out = nout;
+        // row-major [n_out padded to 8][ldw], zero padded; ldw == 4 (mod 16) >= n_in rounded to 4
+        // keeps the DMMA A-fragment loads at the minimum of two shared-memory wavefronts
+        int ldw = (nin + 3) & ~3;
+        while ((ldw & 15) != 4) ldw += 4;
+        b.ldw = ldw;
+        const int nout8 = ((nout + 7) & ~7) > 0 ? ((nout + 7) & ~7) : 8;
+        b.idx_off = idx_off; b.wt_off = (int)t.wt.size(); b.chiv_off = chiv_off;
+        t.wt.resize(t.wt.size() + (size_t)nout8 * ldw, 0.0);
+        for (int r = 0; r < nout; ++r)
+            for (int j = 0; j < nin; ++j)
+                t.wt[b.wt_off + (size_t)r * ldw + j] = blk_w[t.nw + (size_t)r * nin + j];
+        // team-kernel copy: 16-byte fragment loads want a row stride == 8 (mod 16) >= n_in rounded to 8
+        int ldw2 = (nin + 7) & ~7;
+        while ((ldw2 & 15) != 8) ldw2 += 8;
+        b.ldw2 = ldw2; b.wt2_off = (int)t.wt2.size();
+        const int nout64 = ((nout + 63) & ~63) > 0 ? ((nout + 63) & ~63) : 64;     // whole 64-row groups: no row guards
+        t.wt2.resize(t.wt2.size() + (size_t)nout64 * ldw2, 0.0);
+        for (int r = 0; r < nout; ++r)
+            for (int j = 0; j < nin; ++j)
+                t.wt2[b.wt2_off + (size_t)r * ldw2 + j] = blk_w[t.nw + (size_t)r * nin + j];
+        idx_off += nin; t.nw += (long long)nin * nout; chiv_off += nout;
+    }
+    t.blk_idx.assign(blk_idx, blk_idx + idx_off);
+    for (int i = 0; i < N; ++i)
+        if (allowed[i] == 2 && !seen[i])
+            return i >= h->ny ? "every prior entry must appear in exactly one block"
+                              : "every y(+)prior entry must appear in exactly one block";
+    // does at least one warp fit?
+    if (h->fe->per_warp_bytes(32) + (size_t)(chiv_off - ndiag + 2) * sizeof(double) > h->smem_budget) return "size";
+    t.nchiv = chiv_off;
+    return "";
+}
+
 extern "C" {
 
 int b200lm_version(void) { return B200LM_VERSION; }
@@ -311,6 +389,8 @@ void b200lm_destroy(b200lm_handle h) {
     cudaFree(h->d_counter); cudaFree(h->d_stats); cudaFree(h->d_stage); cudaFree(h->d_scratch);
     cudaFree(h->d_order_key); cudaFree(h->d_order); cudaFree(h->d_wave_A);
     cudaFree(h->d_lb); cudaFree(h->d_ub);
+    cudaFree(h->d_win); cudaFree(h->d_win_dfn_idx); cudaFree(h->d_win_dfn_w); cudaFree(h->d_win_dpr_idx);
+    cudaFree(h->d_win_dpr_w); cudaFree(h->d_win_blk); cudaFree(h->d_win_blk_idx); cudaFree(h->d_win_blk_wt);
     if (h->h_pinned) cudaFreeHost(h->h_pinned);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -329,89 +409,113 @@ int b200lm_set_weights(b200lm_handle h, int ndiag, const int* diag_idx, const do
                        int nblk, const int* blk_nin, const int* blk_nout,
                        const int* blk_idx, const double* blk_w) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
-    if (ndiag < 0 || nblk < 0 || (ndiag > 0 && (!diag_idx || !diag_w)) ||
-        (nblk > 0 && (!blk_nin || !blk_nout || !blk_idx || !blk_w)))
-        return set_error(h, B200LM_EINVAL, "bad weight description");
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
-    const int N = h->N;
-    std::vector<char> seen(N, 0);
-    // 1x1 blocks: data rows first (in the given order), then prior rows -- this is the
-    // reference's chiv order because gvar lists 1x1 indices in ascending order.
-    std::vector<int> fn_idx, pr_idx; std::vector<double> fn_w, pr_w;
-    bool prior_seen = false;
-    for (int i = 0; i < ndiag; ++i) {
-        const int idx = diag_idx[i];
-        if (idx < 0 || idx >= N || seen[idx]) return set_error(h, B200LM_EINVAL, "diag index out of range or repeated");
-        seen[idx] = 1;
-        if (idx < h->ny) {
-            if (prior_seen) return set_error(h, B200LM_EINVAL, "diag indices must list data rows before prior rows");
-            fn_idx.push_back(idx); fn_w.push_back(diag_w[i]);
-        } else { prior_seen = true; pr_idx.push_back(idx); pr_w.push_back(diag_w[i]); }
-    }
-    std::vector<BlockDesc> blk(nblk);
-    std::vector<double> wt, wt2;
-    int idx_off = 0, chiv_off = ndiag, w_off = 0;
-    const int rb = 32;
-    for (int k = 0; k < nblk; ++k) {
-        const int nin = blk_nin[k], nout = blk_nout[k];
-        if (nin <= 0 || nout < 0 || nout > nin) return set_error(h, B200LM_EINVAL, "bad block shape");
-        for (int j = 0; j < nin; ++j) {
-            const int idx = blk_idx[idx_off + j];
-            if (idx < 0 || idx >= N || seen[idx]) return set_error(h, B200LM_EINVAL, "block index out of range or repeated");
-            seen[idx] = 1;
-        }
-        BlockDesc& b = blk[k];
-        b.n_in = nin; b.n_out = nout;
-        // row-major [n_out padded to 8][ldw], zero padded; ldw == 4 (mod 16) >= n_in rounded to 4
-        // keeps the DMMA A-fragment loads at the minimum of two shared-memory wavefronts
-        int ldw = (nin + 3) & ~3;
-        while ((ldw & 15) != 4) ldw += 4;
-        b.ldw = ldw;
-        const int nout8 = ((nout + 7) & ~7) > 0 ? ((nout + 7) & ~7) : 8;
-        b.idx_off = idx_off; b.wt_off = (int)wt.size(); b.chiv_off = chiv_off;
-        wt.resize(wt.size() + (size_t)nout8 * ldw, 0.0);
-        for (int r = 0; r < nout; ++r)
-            for (int j = 0; j < nin; ++j)
-                wt[b.wt_off + (size_t)r * ldw + j] = blk_w[w_off + (size_t)r * nin + j];
-        // team-kernel copy: 16-byte fragment loads want a row stride == 8 (mod 16) >= n_in rounded to 8
-        int ldw2 = (nin + 7) & ~7;
-        while ((ldw2 & 15) != 8) ldw2 += 8;
-        b.ldw2 = ldw2; b.wt2_off = (int)wt2.size();
-        const int nout64 = ((nout + 63) & ~63) > 0 ? ((nout + 63) & ~63) : 64;     // whole 64-row groups: no row guards
-        wt2.resize(wt2.size() + (size_t)nout64 * ldw2, 0.0);
-        for (int r = 0; r < nout; ++r)
-            for (int j = 0; j < nin; ++j)
-                wt2[b.wt2_off + (size_t)r * ldw2 + j] = blk_w[w_off + (size_t)r * nin + j];
-        idx_off += nin; w_off += nin * nout; chiv_off += nout;
-    }
-    for (int i = 0; i < N; ++i)
-        if (!seen[i]) return set_error(h, B200LM_EINVAL, "every y(+)prior entry must appear in exactly one block");
-    // does at least one warp fit?
-    if (h->fe->per_warp_bytes(rb) + (size_t)(chiv_off - ndiag + 2) * sizeof(double) > h->smem_budget)
-        return set_error(h, B200LM_ESIZE, "correlated block too large for the per-warp shared-memory plan");
-    h->nd_fn = (int)fn_idx.size(); h->nd_pr = (int)pr_idx.size();
-    CUDA_TRY(h, upload(&h->d_dfn_idx, fn_idx.data(), fn_idx.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_dfn_w, fn_w.data(), fn_w.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_dpr_idx, pr_idx.data(), pr_idx.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_dpr_w, pr_w.data(), pr_w.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk, blk.data(), blk.size()), "upload weights");
+    WeightTables t;
+    const std::string err = parse_weights(h, std::vector<char>(h->N, 2), ndiag, diag_idx, diag_w, nblk, blk_nin,
+                                          blk_nout, blk_idx, blk_w, t);
+    if (!err.empty()) return set_error(h, err == "size" ? B200LM_ESIZE : B200LM_EINVAL,
+                                       err == "size" ? "correlated block too large for the per-warp shared-memory plan"
+                                                     : err);
+    const int idx_off = (int)t.blk_idx.size();
+    h->nd_fn = (int)t.fn_idx.size(); h->nd_pr = (int)t.pr_idx.size();
+    CUDA_TRY(h, upload(&h->d_dfn_idx, t.fn_idx.data(), t.fn_idx.size()), "upload weights");
+    CUDA_TRY(h, upload(&h->d_dfn_w, t.fn_w.data(), t.fn_w.size()), "upload weights");
+    CUDA_TRY(h, upload(&h->d_dpr_idx, t.pr_idx.data(), t.pr_idx.size()), "upload weights");
+    CUDA_TRY(h, upload(&h->d_dpr_w, t.pr_w.data(), t.pr_w.size()), "upload weights");
+    CUDA_TRY(h, upload(&h->d_blk, t.blk.data(), t.blk.size()), "upload weights");
     CUDA_TRY(h, upload(&h->d_blk_idx, blk_idx, (size_t)idx_off), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk_wt, wt.data(), wt.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk_wt2, wt2.data(), wt2.size()), "upload weights");
-    h->wt2_total = (int)wt2.size();
-    h->nblk = nblk; h->wt_total = (int)wt.size(); h->rb = rb; h->nchiv = chiv_off;
+    CUDA_TRY(h, upload(&h->d_blk_wt, t.wt.data(), t.wt.size()), "upload weights");
+    CUDA_TRY(h, upload(&h->d_blk_wt2, t.wt2.data(), t.wt2.size()), "upload weights");
+    h->wt2_total = (int)t.wt2.size();
+    h->nblk = nblk; h->wt_total = (int)t.wt.size(); h->rb = 32; h->nchiv = t.nchiv;
     h->h_diag_idx.assign(diag_idx, diag_idx + ndiag); h->h_diag_w.assign(diag_w, diag_w + ndiag);
-    h->h_blk = blk; h->h_blk_idx.assign(blk_idx, blk_idx + idx_off);
+    h->h_blk = t.blk; h->h_blk_idx.assign(blk_idx, blk_idx + idx_off);
     if (h->d_wfull) { cudaFree(h->d_wfull); h->d_wfull = nullptr; }
     h->have_weights = true;
+    h->nwin = 0;
+    return B200LM_OK;
+}
+
+int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* diag_idx, const double* diag_w,
+                       const int* nblk, const int* blk_nin, const int* blk_nout, const int* blk_idx,
+                       const double* blk_w) {
+    if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (nwin < 1 || !ndiag || !nblk) return set_error(h, B200LM_EINVAL, "bad window description");
+    CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
+    // a window lists every prior entry and its own data rows exactly once
+    std::vector<char> allowed(h->N, 2);
+    for (int i = 0; i < h->ny; ++i) allowed[i] = 1;
+    WeightTables all;
+    std::vector<WinDesc> win(nwin);
+    std::vector<int> nchiv(nwin);
+    std::vector<int> idx_all;
+    long long o_diag = 0, o_blk = 0, o_idx = 0, o_w = 0;
+    for (int w = 0; w < nwin; ++w) {
+        const std::string where = "window " + std::to_string(w) + ": ";
+        if (ndiag[w] < 0 || nblk[w] < 0) return set_error(h, B200LM_EINVAL, where + "bad weight description");
+        WeightTables t;
+        const std::string err = parse_weights(h, allowed, ndiag[w], diag_idx ? diag_idx + o_diag : nullptr,
+                                              diag_w ? diag_w + o_diag : nullptr, nblk[w],
+                                              blk_nin ? blk_nin + o_blk : nullptr, blk_nout ? blk_nout + o_blk : nullptr,
+                                              blk_idx ? blk_idx + o_idx : nullptr, blk_w ? blk_w + o_w : nullptr, t);
+        if (!err.empty()) return set_error(h, err == "size" ? B200LM_ESIZE : B200LM_EINVAL,
+                                           where + (err == "size" ? "correlated block too large for the per-warp "
+                                                                    "shared-memory plan" : err));
+        if (t.ndata == 0) return set_error(h, B200LM_EINVAL, where + "no data row");
+        WinDesc& d = win[w];
+        d.nd_fn = (int)t.fn_idx.size(); d.nd_pr = (int)t.pr_idx.size(); d.nblk = nblk[w]; d.nchiv = t.nchiv;
+        d.dfn_off = (int)all.fn_idx.size(); d.dpr_off = (int)all.pr_idx.size(); d.blk_off = (int)all.blk.size();
+        for (auto b : t.blk) {               // offsets into the concatenated tables
+            b.idx_off += (int)idx_all.size();
+            b.wt_off += (int)all.wt.size();
+            all.blk.push_back(b);
+        }
+        all.fn_idx.insert(all.fn_idx.end(), t.fn_idx.begin(), t.fn_idx.end());
+        all.fn_w.insert(all.fn_w.end(), t.fn_w.begin(), t.fn_w.end());
+        all.pr_idx.insert(all.pr_idx.end(), t.pr_idx.begin(), t.pr_idx.end());
+        all.pr_w.insert(all.pr_w.end(), t.pr_w.begin(), t.pr_w.end());
+        all.wt.insert(all.wt.end(), t.wt.begin(), t.wt.end());
+        idx_all.insert(idx_all.end(), t.blk_idx.begin(), t.blk_idx.end());
+        nchiv[w] = t.nchiv;
+        o_diag += ndiag[w]; o_blk += nblk[w]; o_idx += (long long)t.blk_idx.size(); o_w += t.nw;
+    }
+    CUDA_TRY(h, upload(&h->d_win, win.data(), win.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_dfn_idx, all.fn_idx.data(), all.fn_idx.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_dfn_w, all.fn_w.data(), all.fn_w.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_dpr_idx, all.pr_idx.data(), all.pr_idx.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_dpr_w, all.pr_w.data(), all.pr_w.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_blk, all.blk.data(), all.blk.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_blk_idx, idx_all.data(), idx_all.size()), "upload windows");
+    CUDA_TRY(h, upload(&h->d_win_blk_wt, all.wt.data(), all.wt.size()), "upload windows");
+    h->nwin = nwin;
+    h->win_nchiv = nchiv;
+    h->nchiv = *std::max_element(nchiv.begin(), nchiv.end());
+    h->rb = 32;
+    return B200LM_OK;
+}
+
+int b200lm_window_nchiv(b200lm_handle h, int* h_nchiv) {
+    if (!h || !h_nchiv) return set_error(h, B200LM_EINVAL, "NULL argument");
+    if (h->nwin == 0) return set_error(h, B200LM_EINVAL, "no windows set (b200lm_set_windows)");
+    for (int w = 0; w < h->nwin; ++w) h_nchiv[w] = h->win_nchiv[w];
     return B200LM_OK;
 }
 
 int b200lm_nchiv(b200lm_handle h) { return h ? h->nchiv : B200LM_EINVAL; }
 
+// what a batch on fit windows does not combine with
+static int window_refusal(b200lm_handle h, int B) {
+    if (h->nwin == 0) return B200LM_OK;
+    if (B % h->nwin != 0)
+        return set_error(h, B200LM_EINVAL, "with windows set, B must be a multiple of the number of windows");
+    if (h->policy == 1) return set_error(h, B200LM_EINVAL, "the GSL policy is not built for window scans");
+    if (h->bounded) return set_error(h, B200LM_EINVAL, "bounds are not built for window scans");
+    return B200LM_OK;
+}
+
 static int check_ready(b200lm_handle h) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
-    if (!h->have_weights) return set_error(h, B200LM_EINVAL, "b200lm_set_weights has not been called");
+    if (!h->have_weights && h->nwin == 0) return set_error(h, B200LM_EINVAL, "b200lm_set_weights has not been called");
     if (!h->have_const) return set_error(h, B200LM_EINVAL, "b200lm_set_const has not been called");
     return B200LM_OK;
 }
@@ -434,6 +538,8 @@ int b200lm_fit_batch(b200lm_handle h, int B,
     if (maxit < 1) return set_error(h, B200LM_EINVAL, "maxit must be >= 1");
     if (h->bounded && h->policy == 1)
         return set_error(h, B200LM_EINVAL, "bounds need the scipy trf policy (GSL's lm has no bound constraints)");
+    rc = window_refusal(h, B);
+    if (rc) return rc;
     if (B == 0) return B200LM_OK;
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
@@ -446,6 +552,22 @@ int b200lm_fit_batch(b200lm_handle h, int B,
     if (h->bounded) { P.bounded = 1; P.lb = h->d_lb; P.ub = h->d_ub; }
     CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(int), s), "reset work queue");
     CUDA_TRY(h, cudaMemsetAsync(h->d_stats, 0, 16 * sizeof(unsigned long long), s), "reset stats");
+    if (h->nwin > 0) {
+        // fit windows: the window kernel (fit_kernel<F, 4>), one warp per fit, queue in input order; the row tables are
+        // those of every window, addressed through P.win
+        P.nwin = h->nwin; P.win_copies = B / h->nwin; P.win = h->d_win;
+        P.nd_fn = 0; P.nd_pr = 0; P.nblk = 0;
+        P.dfn_idx = h->d_win_dfn_idx; P.dfn_w = h->d_win_dfn_w; P.dpr_idx = h->d_win_dpr_idx; P.dpr_w = h->d_win_dpr_w;
+        P.blk = h->d_win_blk; P.blk_idx = h->d_win_blk_idx; P.blk_wt = h->d_win_blk_wt;
+        P.wt_total = 0; P.blk_wt2 = nullptr; P.wt2_total = 0; P.nblk_idx = 0;
+        P.team = 1;
+        CUDA_TRY(h, h->fe->fit(P, h->sm_count, h->smem_budget, s), "window fit kernel launch");
+        h->last_order = 0;
+        h->last_team = 1;
+        h->last_stream = s;
+        h->launches += 1;
+        return B200LM_OK;
+    }
     // queue order: chi2 at the start point of every fit (one evaluation each, resjac kernel without f / J outputs),
     // ranked on the device
     h->last_order = 0;
@@ -635,6 +757,7 @@ int b200lm_residual_jacobian(b200lm_handle h, int B, const double* d_p, long lon
     int rc = check_ready(h);
     if (rc) return rc;
     if (B < 0 || !d_p || !d_mean) return set_error(h, B200LM_EINVAL, "NULL required argument");
+    if (h->nwin > 0) return set_error(h, B200LM_EINVAL, "residual_jacobian is not built for window scans");
     if (B == 0) return B200LM_OK;
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     FitParams P;
@@ -675,6 +798,8 @@ int b200lm_fit_batch_host(b200lm_handle h, int B,
     if (B == 0) return B200LM_OK;                 // empty batch
     if (B < 0 || !h_mean || !h_p0 || !h_x || !h_chi2 || !h_nit || !h_status)
         return set_error(h, B200LM_EINVAL, "NULL required argument");
+    rc = window_refusal(h, B);
+    if (rc) return rc;
     if (h->bounded) {                             // scipy refuses a start outside the box (least_squares: "`x0` is infeasible.")
         const long long nst = p0_stride ? (long long)B : 1;
         for (long long b = 0; b < nst; ++b)
@@ -685,8 +810,9 @@ int b200lm_fit_batch_host(b200lm_handle h, int B,
     }
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     const size_t np = h->np, N = h->N, nchiv = h->nchiv;
-    const size_t n_mean = mean_stride ? (size_t)B * mean_stride : N;
-    const size_t n_p0 = p0_stride ? (size_t)B * p0_stride : np;
+    // with windows: a row of means per copy, a start per window
+    const size_t n_mean = mean_stride ? (size_t)(h->nwin ? B / h->nwin : B) * mean_stride : N;
+    const size_t n_p0 = p0_stride ? (size_t)(h->nwin ? h->nwin : B) * p0_stride : np;
     // device layout (doubles): mean | p0 | x | chi2 | logdet | cov | f | J | nit,status (ints)
     size_t off = 0;
     auto take = [&](size_t n) { size_t o = off; off += (n + 1) & ~(size_t)1; return o; };

@@ -37,6 +37,14 @@ struct b200lm_handle_s {
     double* d_lb = nullptr; double* d_ub = nullptr;
     std::vector<double> h_lb, h_ub;
     bool bounded = false;
+    // fit windows (b200lm_set_windows): concatenated row tables of every window, used instead of the plan's weights
+    // while nwin > 0; b200lm_set_weights sets nwin back to 0 (and nchiv back to the plan's)
+    int nwin = 0;
+    std::vector<int> win_nchiv;
+    b200lm::WinDesc* d_win = nullptr;
+    int* d_win_dfn_idx = nullptr; double* d_win_dfn_w = nullptr;
+    int* d_win_dpr_idx = nullptr; double* d_win_dpr_w = nullptr;
+    b200lm::BlockDesc* d_win_blk = nullptr; int* d_win_blk_idx = nullptr; double* d_win_blk_wt = nullptr;
     // queue order (longest-expected fits first): key = chi2 at the start point, one evaluation per fit
     int order_request = -1;     // -1: default policy (by problem shape and batch size); 0: off; 1: on  (b200lm_set_order)
     int last_order = 0;         // 1 if the last fit_batch launch used an ordered queue

@@ -296,20 +296,14 @@ __device__ __forceinline__ void consume_rows(WarpCtx<F>& c, int nrows, int slot0
 // returns cost.  Optionally writes the residual vector and J to global memory.
 // MODE 0: normal equations (A = J^T J, g = J^T r).  MODE 1: QR factor of J.diag(dsc) in c.A.
 // ---------------------------------------------------------------------------
-template <class F, int MODE, bool WSMEM>
-__device__ __noinline__ double eval_full_impl(const WarpCtx<F>& c_in, const double* pv, double* fout, double* Jout) {
-    WarpCtx<F> c = c_in;                // local copy: the address-space assumptions below attach to SSA values
+// T: the row tables (nd_fn, dfn_idx, dfn_w, nd_pr, dpr_idx, dpr_w, nblk, blk) -- the FitParams themselves, or those of
+// one window (WinRows)
+template <class F, int MODE, bool WSMEM, class RS>
+__device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const double* pv, double* fout, double* Jout) {
     typedef FitLayout<F> Lay;
     constexpr int NP = Lay::NP, NT = Lay::NT, LDR = Lay::LDR, LDA = Lay::LDA, NCOL = Lay::NCOL;
     const FitParams& P = c.P;
     const int lane = c.lane;
-    // per-warp state lives in shared memory: say so, or the out-of-line code uses generic LD/ST
-    __builtin_assume(__isShared(c.R));
-    __builtin_assume(__isShared(c.dvec));
-    __builtin_assume(__isShared(c.A));
-    __builtin_assume(__isShared(c.g));
-    __builtin_assume(__isShared(c.dsc));
-    __builtin_assume(__isShared(pv));
     for (int e = lane; e < NP * LDA; e += 32) c.A[e] = 0.0;
     if (MODE == 0 && lane < NP) c.g[lane] = 0.0;
     __syncwarp();
@@ -317,10 +311,10 @@ __device__ __noinline__ double eval_full_impl(const WarpCtx<F>& c_in, const doub
     NormalAcc<F> na;
     na.clear();
     // 1x1 prior rows: J row = w e_j, analytic contribution
-    for (int i = lane; i < P.nd_pr; i += 32) {
-        const int idx = P.dpr_idx[i];
+    for (int i = lane; i < T.nd_pr; i += 32) {
+        const int idx = T.dpr_idx[i];
         const int j = idx - P.ny;
-        const double w = P.dpr_w[i];
+        const double w = T.dpr_w[i];
         const double r = w * (pv[j] - c.mean[idx]);
         if (MODE == 0) {
             c.A[j * LDA + j] += w * w;
@@ -329,19 +323,19 @@ __device__ __noinline__ double eval_full_impl(const WarpCtx<F>& c_in, const doub
             c.A[j * LDA + j] = w * c.dsc[j];                 // a diagonal matrix is triangular
         }
         acc = fma(r, r, acc);
-        if (fout) fout[P.nd_fn + i] = r;
+        if (fout) fout[T.nd_fn + i] = r;
         if (Jout) {
-            for (int q = 0; q < NP; ++q) Jout[(size_t)(P.nd_fn + i) * NP + q] = (q == j) ? w : 0.0;
+            for (int q = 0; q < NP; ++q) Jout[(size_t)(T.nd_fn + i) * NP + q] = (q == j) ? w : 0.0;
         }
     }
     __syncwarp();
     // 1x1 data rows, staged through the row buffer 32 at a time (one row per lane)
-    for (int c0 = 0; c0 < P.nd_fn; c0 += 32) {
-        const int nrows = min(32, P.nd_fn - c0);
+    for (int c0 = 0; c0 < T.nd_fn; c0 += 32) {
+        const int nrows = min(32, T.nd_fn - c0);
         double* row_ = c.R + lane * LDR;
         if (lane < nrows) {
-            const int row = P.dfn_idx[c0 + lane];
-            const double w = P.dfn_w[c0 + lane];
+            const int row = T.dfn_idx[c0 + lane];
+            const double w = T.dfn_w[c0 + lane];
             const double f = F::value_grad(P.x + (size_t)row * P.nx, row, pv, w, row_);
             row_[NP] = w * (f - c.mean[row]);
 #pragma unroll
@@ -356,8 +350,8 @@ __device__ __noinline__ double eval_full_impl(const WarpCtx<F>& c_in, const doub
     // correlated blocks: J_blk = W.[G | delta] on the FP64 tensor path.  The C fragments of a
     // 64-row output group stay in registers while the input rows stream through the row buffer
     // 32 at a time; the finished rows then pass through the same buffer into J^T J.
-    for (int b = 0; b < P.nblk; ++b) {
-        const BlockDesc bd = P.blk[b];
+    for (int b = 0; b < T.nblk; ++b) {
+        const BlockDesc bd = T.blk[b];
         const double* W = c.wt + bd.wt_off;
         if constexpr (WSMEM) __builtin_assume(__isShared(W));
         for (int g0 = 0; g0 < bd.n_out; g0 += 64) {
@@ -460,11 +454,62 @@ __device__ __noinline__ double eval_full_impl(const WarpCtx<F>& c_in, const doub
     return 0.5 * warp_sum(acc);
 }
 
+template <class F, int MODE, bool WSMEM>
+__device__ __noinline__ double eval_full_impl(const WarpCtx<F>& c_in, const double* pv, double* fout, double* Jout) {
+    WarpCtx<F> c = c_in;                // local copy: the address-space assumptions below attach to SSA values
+    // per-warp state lives in shared memory: say so, or the out-of-line code uses generic LD/ST
+    __builtin_assume(__isShared(c.R));
+    __builtin_assume(__isShared(c.dvec));
+    __builtin_assume(__isShared(c.A));
+    __builtin_assume(__isShared(c.g));
+    __builtin_assume(__isShared(c.dsc));
+    __builtin_assume(__isShared(pv));
+    return eval_rows<F, MODE, WSMEM>(c, c.P, pv, fout, Jout);
+}
+
 // the block weights are staged in shared memory whenever they fit (P.wt_in_smem, uniform)
 template <class F, int MODE = 0>
 __device__ __forceinline__ double eval_full(WarpCtx<F>& c, const double* pv, double* fout, double* Jout) {
     return c.P.wt_in_smem ? eval_full_impl<F, MODE, true>(c, pv, fout, Jout)
                           : eval_full_impl<F, MODE, false>(c, pv, fout, Jout);
+}
+
+// the row tables of one window (P.win[w]), in the names eval_rows reads
+struct WinRows {
+    int nd_fn, nd_pr, nblk;
+    const int* dfn_idx;
+    const double* dfn_w;
+    const int* dpr_idx;
+    const double* dpr_w;
+    const BlockDesc* blk;
+};
+
+// window evaluation: the weights stay in global memory (a scan's windows together are too large to stage, and the
+// fits of one window are contiguous in the batch, so the warps in flight share a few windows' weights in L2)
+template <class F, int MODE>
+__device__ __noinline__ double eval_win_impl(const WarpCtx<F>& c_in, int w, const double* pv, double* fout, double* Jout) {
+    WarpCtx<F> c = c_in;
+    __builtin_assume(__isShared(c.R));
+    __builtin_assume(__isShared(c.dvec));
+    __builtin_assume(__isShared(c.A));
+    __builtin_assume(__isShared(c.g));
+    __builtin_assume(__isShared(c.dsc));
+    __builtin_assume(__isShared(pv));
+    const FitParams& P = c.P;
+    const WinDesc wd = P.win[w];
+    WinRows T;
+    T.nd_fn = wd.nd_fn; T.nd_pr = wd.nd_pr; T.nblk = wd.nblk;
+    T.dfn_idx = P.dfn_idx + wd.dfn_off; T.dfn_w = P.dfn_w + wd.dfn_off;
+    T.dpr_idx = P.dpr_idx + wd.dpr_off; T.dpr_w = P.dpr_w + wd.dpr_off;
+    T.blk = P.blk + wd.blk_off;
+    const double cost = eval_rows<F, MODE, false>(c, T, pv, fout, Jout);
+    // f / J rows have the stride of the largest window: zero beyond this window's own residuals
+    for (int i = wd.nchiv + c.lane; i < P.nchiv; i += 32) {
+        if (fout) fout[i] = 0.0;
+        if (Jout)
+            for (int q = 0; q < F::NP; ++q) Jout[(size_t)i * F::NP + q] = 0.0;
+    }
+    return cost;
 }
 
 // ---------------------------------------------------------------------------
@@ -1178,6 +1223,23 @@ struct WarpEval {
     }
 };
 
+// Evaluator of the window kernel (fit_kernel<F, 4>): one warp per fit, fit b is copy b % win_copies of window
+// b / win_copies, with that window's rows and weights
+template <class F>
+struct WinEval {
+    int w;
+    __device__ __forceinline__ const double* begin(WarpCtx<F>&, const FitParams& P, int b) {
+        w = b / P.win_copies;
+        return P.mean + (size_t)(b % P.win_copies) * P.mean_stride;
+    }
+    __device__ __forceinline__ double run(WarpCtx<F>& c, const double* pv, double* fout, double* Jout, int mode) {
+        return mode == 0 ? eval_win_impl<F, 0>(c, w, pv, fout, Jout) : eval_win_impl<F, 1>(c, w, pv, fout, Jout);
+    }
+};
+
+template <class F, int MODE> struct EvalOf { typedef WarpEval<F> type; };
+template <class F> struct EvalOf<F, 4> { typedef WinEval<F> type; };
+
 // One complete fit (number b of the batch) driven by the warp that owns `c`: trust-region loop, optional
 // polish, covariance, results.  EV::run evaluates residual + Jacobian + normal equations at a point -- by
 // this warp alone (WarpEval) or by the warps of a team (lm_team.cuh: TeamEval); everything else is the
@@ -1192,7 +1254,8 @@ struct PhaseClock {
 // MODE selects what is COMPILED into a kernel (the trust-region loop is the hot code: every policy it does not run
 // would only cost registers and instruction cache):  0 = scipy TRF decisions (the default kernels),  1 = GSL trust/lm
 // decisions (b200lm_set_policy),  2 = no loop at all: finalisation of fits the wave kernel has already converged,
-// 3 = scipy TRF with bound constraints (trf_bounds: Coleman-Li scaling, select_step; b200lm_set_bounds).
+// 3 = scipy TRF with bound constraints (trf_bounds: Coleman-Li scaling, select_step; b200lm_set_bounds),
+// 4 = scipy TRF on fit windows (the loop of MODE 0; EV = WinEval: rows, weights and means per window, b200lm_set_windows).
 template <class F, class EV, int MODE = 0>
 __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& P, int b,
                                         unsigned long long& tot_nfev, unsigned long long& tot_njev,
@@ -1203,7 +1266,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
     const bool act = lane < NP;
     {
         c.mean = ev.begin(c, P, b);
-        const double* p0 = P.p0 + (size_t)b * P.p0_stride;
+        const double* p0 = P.p0 + (size_t)(MODE == 4 ? b / P.win_copies : b) * P.p0_stride;     // MODE 4: per window
         if (act) c.p[lane] = p0[lane];
         double lbi = -INFINITY, ubi = INFINITY;             // this lane's bounds (MODE 3)
         if constexpr (MODE == 3) {
@@ -1355,7 +1418,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
 
         // MODE 3 (bounds) is the same loop with scipy's trf_bounds changes: the gtol test on |g v|_inf, the scaling
         // d = sqrt(v) / scale_inv, the Coleman-Li diagonal in the sub-problem, select_step, strictly feasible trials
-        while ((MODE == 0 || MODE == 3) && status == -2) {
+        while ((MODE == 0 || MODE == 3 || MODE == 4) && status == -2) {
             const double gi = act ? c.g[lane] : 0.0;
             double v = 1.0, dv = 0.0;                              // Coleman-Li scaling (MODE 3)
             const double xi = act ? c.p[lane] : 0.0;
@@ -1600,7 +1663,7 @@ __global__ void __launch_bounds__(FitLayout<F>::MAX_WARPS * 32, 1) fit_kernel(co
     setup_ctx<F>(c, smem, P);
     const int lane = c.lane;
     unsigned long long tot_nfev = 0, tot_njev = 0, tot_nfac = 0;
-    WarpEval<F> ev;
+    typename EvalOf<F, MODE>::type ev;
     PhaseClock pk;
     pk.clear();
 
@@ -1612,7 +1675,7 @@ __global__ void __launch_bounds__(FitLayout<F>::MAX_WARPS * 32, 1) fit_kernel(co
         }
         b = __shfl_sync(B200LM_FULL, b, 0);
         if (b >= P.B) break;
-        fit_one<F, WarpEval<F>, MODE>(c, ev, P, b, tot_nfev, tot_njev, tot_nfac, pk);
+        fit_one<F, typename EvalOf<F, MODE>::type, MODE>(c, ev, P, b, tot_nfev, tot_njev, tot_nfac, pk);
     }
     if (lane == 0 && P.stats) {
         atomicAdd(&P.stats[0], tot_nfev);
@@ -1662,7 +1725,7 @@ inline cudaError_t plan_launch(FitParams& P, int sm_count, size_t smem_budget, L
     typedef FitLayout<F> Lay;
     const size_t wt_bytes = ((size_t)(P.wt_total + 1) & ~(size_t)1) * sizeof(double);
     const size_t per_warp = (size_t)Lay::per_warp_doubles(P.rb) * sizeof(double);
-    P.wt_in_smem = (P.wt_total > 0 && wt_bytes + 4 * per_warp <= smem_budget) ? 1 : 0;
+    P.wt_in_smem = (P.nwin == 0 && P.wt_total > 0 && wt_bytes + 4 * per_warp <= smem_budget) ? 1 : 0;
     const size_t avail = smem_budget - (P.wt_in_smem ? wt_bytes : 0);
     int warps = (int)(avail / per_warp);
     if (warps < 1) return cudaErrorInvalidConfiguration;
@@ -1695,6 +1758,7 @@ cudaError_t launch_fit(FitParams P, int sm_count, size_t smem_budget, cudaStream
     LaunchInfo li;
     cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li);
     if (e != cudaSuccess) return e;
+    if (P.nwin > 0) return launch_fit_mode<F, 4>(P, li, stream);
     if (P.finalize_only) return launch_fit_mode<F, 2>(P, li, stream);
     if (P.bounded) return launch_fit_mode<F, 3>(P, li, stream);
     if (P.policy == 1) return launch_fit_mode<F, 1>(P, li, stream);

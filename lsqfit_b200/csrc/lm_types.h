@@ -17,6 +17,13 @@ struct BlockDesc {
     int wt2_off;     // offset into blk_wt2[]
 };
 
+// One window of a window scan (b200lm_set_windows): its part of the concatenated row tables of FitParams.
+// BlockDesc::idx_off and wt_off address the concatenated blk_idx / blk_wt, chiv_off the window's own residual vector.
+struct WinDesc {
+    int nd_fn, nd_pr, nblk, nchiv;
+    int dfn_off, dpr_off, blk_off;
+};
+
 // normal_diag_kernel (lm_rows.cuh): rows of the per-CTA partial buffer that b200lm_normal_diag allocates per SM
 constexpr int ND_MAX_PARTS_PER_SM = 8;
 
@@ -78,6 +85,11 @@ struct FitParams {
     const double* lb;           // [np] lower bounds (-inf: none), device parameter order
     const double* ub;           // [np] upper bounds (+inf: none)
     int bounded;                // 1: scipy's trf_bounds decisions (fit_kernel<F, 3>); lb / ub are set
+    // ---- fit windows (last, for the same reason; b200lm_set_windows) ----
+    int nwin;                   // > 0: fit b is copy b % win_copies of window b / win_copies (fit_kernel<F, 4>); the
+                                // tables above (dfn_*, dpr_*, blk, blk_idx, blk_wt) hold every window, one after the other
+    int win_copies;
+    const WinDesc* win;         // [nwin]
 };
 
 }  // namespace b200lm

@@ -20,6 +20,7 @@ extern "C" int b200lm_propagate(b200lm_handle h, int B, const double* d_x, const
                                 const double* d_C, double* d_D, double* d_covp, void* stream) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
     if (!h->have_weights || !h->have_const) return set_error(h, B200LM_EINVAL, "plan is not complete");
+    if (h->nwin > 0) return set_error(h, B200LM_EINVAL, "propagate is not built for window scans");
     if (B < 0 || !d_x || !d_cov || !d_D) return set_error(h, B200LM_EINVAL, "NULL required argument");
     if (d_covp && !d_C) return set_error(h, B200LM_EINVAL, "d_C is required for cov(p)");
     if (B == 0) return B200LM_OK;

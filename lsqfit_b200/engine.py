@@ -85,6 +85,25 @@ class Plan(object):
             self._h, len(idx0), idx0.ctypes.data, w0.ctypes.data, len(nin),
             nin.ctypes.data, nout.ctypes.data, bidx.ctypes.data, bw.ctypes.data), self._h)
         self.nchiv = _cabi.lib.b200lm_nchiv(self._h)
+        self.nwin = 0
+
+    def set_windows(self, desc):
+        """Fit windows instead of the weights (b200lm_set_windows): ``desc`` as made by
+        ``lsqfit_b200.windows.window_weights``.  fit_batch then fits B = nwin x copies: means [copies, N] (or [N]),
+        p0 [nwin, np] (or [np]); fit b is copy b % copies of window b // copies.  ``set_weights`` switches back."""
+        d = dict((k, np.ascontiguousarray(desc[k], dtype=np.float64 if k in ("diag_w", "blk_w") else np.int32))
+                 for k in ("ndiag", "diag_idx", "diag_w", "nblk", "blk_nin", "blk_nout", "blk_idx", "blk_w"))
+        nwin = len(d["ndiag"])
+        _cabi.check(_cabi.lib.b200lm_set_windows(
+            self._h, nwin, *[d[k].ctypes.data for k in ("ndiag", "diag_idx", "diag_w", "nblk", "blk_nin", "blk_nout",
+                                                       "blk_idx", "blk_w")]), self._h)
+        self.nchiv = _cabi.lib.b200lm_nchiv(self._h)
+        self.nwin = nwin
+
+    def window_nchiv(self):
+        out = np.zeros(self.nwin, dtype=np.int32)
+        _cabi.check(_cabi.lib.b200lm_window_nchiv(self._h, out.ctypes.data), self._h)
+        return out
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -163,8 +182,11 @@ class Plan(object):
             if not bool(torch.all((tp >= tl) & (tp <= tu))):           # one reduction (scipy: "`x0` is infeasible.")
                 raise ValueError("`x0` is infeasible.")
         if B is None:
-            B = tm.shape[0] if sm else (tp.shape[0] if sp else 1)
-        if (sm and tm.shape[0] != B) or (sp and tp.shape[0] != B):
+            B = ((tm.shape[0] if sm else 1) * self.nwin if self.nwin else
+                 (tm.shape[0] if sm else (tp.shape[0] if sp else 1)))
+        # with windows: a row of means per copy, a start per window
+        rows_m, rows_p = (B // self.nwin, self.nwin) if self.nwin else (B, B)
+        if (sm and tm.shape[0] != rows_m) or (sp and tp.shape[0] != rows_p):
             raise ValueError("mean and p0 disagree on the batch size")
         if out is None:
             kw = dict(device=self.tdev, dtype=torch.float64)

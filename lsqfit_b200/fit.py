@@ -24,7 +24,7 @@ import time
 import numpy as np
 import torch
 
-from .engine import STOPPING_CRITERION, normalize_tol
+from .engine import STOPPING_CRITERION, BatchResult, normalize_tol
 from .fitter import ChivSpec, DeviceChiv, b200_lm
 from .functors import Functor
 from .whiten import PDF
@@ -322,6 +322,17 @@ class nonlinear_fit(object):
         for f in self.simulated_fits(n, pexact, add_priornoise, seed, **kargs):
             yield f
 
+    def window_fits(self, masks, p0=None, **kargs):
+        """Fit-window scan: the fits of the data windows ``masks`` (bool [nwin, ny]) in ONE launch.
+
+        Window ``w`` is the fit ``nonlinear_fit(data=(x[m], y[m], ycov[m][:, m]), prior=self.prior, fcn=self.fcn,
+        svdcut=self.svdcut, eps=self.eps, p0=p0)`` with ``m = masks[w]``: its y (+) prior covariance is this fit's input
+        covariance restricted to its rows and the prior, whitened on its own.  ``p0``: [np] or [nwin, np], default this
+        fit's ``pmean``.  Fitter arguments are this fit's unless given here (``tol``, ``maxit``, ``scaler``,
+        ``polish``); ``kernel=`` is accepted and ignored (window batches run one warp per fit).  Returns a
+        ``WindowScan``; its ``bootstrapped_fits`` fits every window's bootstrap copies in one more launch."""
+        return WindowScan(self, masks, p0, **kargs)
+
 
 class FitView(object):
     """One fit of a batch, with the attribute names of nonlinear_fit."""
@@ -374,6 +385,128 @@ class BatchFits(object):
         m = x.mean(dim=0)
         d = x - m
         return m.cpu().numpy(), (d.T @ d / max(1, x.shape[0] - 1)).cpu().numpy()
+
+
+class _Window(object):
+    """What FitView and BatchFits read from the fit a result belongs to, for one window of a scan."""
+
+    def __init__(self, parent, pdf, nchiv, np_):
+        self.prior, self.tol = parent.prior, parent.tol
+        self.yp_pdf, self.svdn = pdf, pdf.nmod
+        self.dof = int(nchiv) - int(np_)
+
+
+class WindowScan(object):
+    """The central fits of a fit-window scan (``nonlinear_fit.window_fits``).
+
+    Arrays over windows: ``pmean psdev`` [nwin, np], ``cov`` [nwin, np, np], ``chi2 dof Q logGBF svdn nit
+    stopping_criterion error`` [nwin].  ``scan[w]`` has the attribute names of ``nonlinear_fit``; ``pdfs[w]`` is the
+    window's whitening.  The scan owns its plan: the parent's (cached, shared) plan is left as it was."""
+
+    def __init__(self, parent, masks, p0=None, **kargs):
+        from .engine import POLICY, Plan
+        from .whiten import cov_blocks, whiten_blocks
+        from .windows import check_masks, window_cov, window_weights
+        args = dict(parent.fitterargs)
+        args.update(kargs)
+        args.pop("device", None)
+        args.pop("kernel", None)                     # window batches always run one warp per fit
+        refuse = lambda what: ValueError("b200_lm: %s not built for window scans" % what)
+        if args.pop("bounds", None) is not None:
+            raise refuse("bounds are")
+        if args.pop("loss", "linear") != "linear":
+            raise refuse("a robust loss is")
+        if POLICY.get(args.get("policy", "trf")) == 1:
+            raise refuse("policy='gsl' is")
+        if any(parent.noise):
+            raise refuse("fits made with noise are")
+        spec = parent._spec
+        self.parent, self.device = parent, parent.device
+        self.np, self.ny = spec.np, spec.ny
+        self.masks = check_masks(masks, self.ny)
+        self.nwin = self.masks.shape[0]
+        self.tol = parent.tol if args.get("tol") is None else normalize_tol(args["tol"])
+        self.maxit = parent.maxit if args.get("maxit") is None else int(args["maxit"])
+        self.scaler, self.polish = args.get("scaler", "more"), int(args.get("polish", 0))
+        pdf = parent.yp_pdf
+        cov = pdf.cov_in if pdf.cov_in is not None else pdf.sdev_in
+        wins = [window_cov(cov, self.ny, m) for m in self.masks]
+        # the correlated blocks of every window, whitened in ONE call (b200lm_whiten: one CTA per block, and a block's
+        # result depends on that block alone -- each window's whitening is bit for bit that of a PDF of its own)
+        blocks = [cov_blocks(c)[1] if c.ndim == 2 else [] for _, c in wins]
+        ns = [b.size for bl in blocks for b in bl]
+        if ns:
+            flat = np.concatenate([c[np.ix_(b, b)].reshape(-1) for (_, c), bl in zip(wins, blocks) for b in bl])
+            W, Cc, nout, nmod, ld = whiten_blocks(np.array(ns), flat, pdf.svdcut, pdf.eps, self.device)
+        self.pdfs = []
+        o = k = 0
+        for (sel, c), bl in zip(wins, blocks):
+            nb, nel = len(bl), sum(b.size ** 2 for b in bl)
+            part = (W[o:o + nel], Cc[o:o + nel], nout[k:k + nb], nmod[k:k + nb], ld[k:k + nb]) if nb else None
+            self.pdfs.append(PDF(pdf.mean[sel], c, svdcut=pdf.svdcut, eps=pdf.eps, device=self.device,
+                                 _whitened=part))
+            o, k = o + nel, k + nb
+        self.sels = [sel for sel, _ in wins]
+        desc = window_weights(self.sels, [p.i_invwgts for p in self.pdfs])
+        self.nchiv = desc["nchiv"]
+        self.plan = Plan(spec.functor, spec.np, spec.ny, spec.x, spec.i_invwgts, noprior=spec.noprior,
+                         device=self.device)
+        self.plan.set_windows(desc)
+        self.windows = [_Window(parent, p, n, self.np) for p, n in zip(self.pdfs, self.nchiv)]
+        self.dof = np.array([w.dof for w in self.windows])
+        self.svdn = np.array([w.svdn for w in self.windows])
+        p0 = parent.pmean if p0 is None else np.asarray(p0, dtype=float)
+        self.p0 = np.array(np.broadcast_to(p0, (self.nwin, self.np)))
+        out = self._fit(spec.mean, self.p0, self.nwin)
+        a = out.numpy()
+        self.out, self._arrays = out, a
+        self.pmean, self.cov, self.chi2, self.nit = a["x"], a["cov"], a["chi2"], a["nit"]
+        self.psdev = np.sqrt(np.diagonal(self.cov, axis1=1, axis2=2))
+        self.Q = gammaQ(self.dof / 2., self.chi2 / 2.)
+        self.logGBF = (None if parent.prior is None else
+                       np.array([_logGBF(a["logdet"][w], p.logdet, a["chi2"][w], d)
+                                 for w, (p, d) in enumerate(zip(self.pdfs, self.dof))]))
+        self.stopping_criterion = np.array([STOPPING_CRITERION[int(s)] for s in a["status"]])
+        self.error = np.array([None if s > 0 else "b200_lm: no convergence" for s in a["status"]], dtype=object)
+
+    def _fit(self, means, p0, B):
+        return self.plan.fit_batch(means, p0, tol=self.tol, maxit=self.maxit, scaler=self.scaler, polish=self.polish, B=B)
+
+    def __len__(self):
+        return self.nwin
+
+    def __getitem__(self, w):
+        return FitView(self.windows[w], self._arrays, w)
+
+    def bootstrapped_fits(self, n=None, seed=None, means=None):
+        """n bootstrap copies of every window in ONE launch (nwin * n fits).  The copies are the parent's
+        ``bootstrap_means(n, seed)`` (or ``means`` [n, N]); every window of copy j reads its rows from the same row j,
+        and the copies of window w start from the window's central ``pmean``."""
+        if means is None:
+            means = self.parent.bootstrap_means(n, seed)
+        n = int(means.shape[0])
+        return WindowBootstrap(self, self._fit(means, self.pmean, self.nwin * n), n)
+
+
+class WindowBootstrap(object):
+    """The bootstrap copies of a window scan: fit b is copy b % n of window b // n."""
+
+    def __init__(self, scan, out, n):
+        self.scan, self.out, self.n = scan, out, n
+
+    def __len__(self):
+        return self.out.x.shape[0]
+
+    def arrays(self):
+        return self.out.numpy()
+
+    def window(self, w):
+        """BatchFits of window w's copies (arrays(), iteration, pmean_stats())."""
+        s = slice(w * self.n, (w + 1) * self.n)
+        o = self.out
+        part = BatchResult(*[None if t is None else t[s] for t in (o.x, o.chi2, o.cov, o.logdet, o.nit, o.status,
+                                                                    o.f, o.J)])
+        return BatchFits(self.scan.windows[w], part)
 
 
 class WAvg(object):

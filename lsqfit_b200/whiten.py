@@ -51,7 +51,10 @@ class PDF(object):
     """Whitened Gaussian distribution of y (+) prior (attribute-compatible with gvar.PDF
     as far as lsqfit reads it)."""
 
-    def __init__(self, mean, cov, svdcut=1e-12, eps=None, device=0, noise=False, noise_seed=None):
+    def __init__(self, mean, cov, svdcut=1e-12, eps=None, device=0, noise=False, noise_seed=None, _whitened=None):
+        """``_whitened``: the output of ``whiten_blocks`` for this covariance's correlated blocks, computed elsewhere
+        (a window scan whitens the blocks of all its windows in one call; each block's result depends on that block
+        alone)."""
         mean = np.array(mean, dtype=float).reshape(-1)
         cov = np.asarray(cov, dtype=float)
         if cov.ndim == 1:
@@ -72,11 +75,13 @@ class PDF(object):
             idx0, blocks = np.arange(N, dtype=np.intp), []
             sd0 = np.asarray(sd, dtype=float)
             self._cov_diag_only = sd0 ** 2
+            self.sdev_in = sd0
         else:
             assert cov.shape == (N, N)
             idx0, blocks = cov_blocks(cov)
             sd0 = np.sqrt(cov[idx0, idx0])
             self._cov_diag_only = None
+            self.sdev_in = None
         self.cov_in = cov
         self.i_invwgts = [(idx0, 1.0 / sd0)]
         if idx0.size:
@@ -87,7 +92,8 @@ class PDF(object):
         if blocks:
             ns = np.array([b.size for b in blocks], dtype=np.int32)
             flat = np.concatenate([cov[np.ix_(b, b)].reshape(-1) for b in blocks])
-            W, Cc, nout, nmod, logdet = whiten_blocks(ns, flat, svdcut, eps, device)
+            W, Cc, nout, nmod, logdet = (whiten_blocks(ns, flat, svdcut, eps, device) if _whitened is None
+                                         else _whitened)
             o = 0
             for k, b in enumerate(blocks):
                 n = b.size
