@@ -32,12 +32,13 @@ void fill_params(b200lm_handle_s* h, FitParams& P) {
     memset(&P, 0, sizeof(P));
     P.ny = h->ny; P.np = h->np; P.N = h->N; P.nchiv = h->nchiv; P.nx = h->nx; P.noprior = h->noprior;
     P.x = h->d_x;
-    P.nd_fn = h->nd_fn; P.dfn_idx = h->d_dfn_idx; P.dfn_w = h->d_dfn_w;
-    P.nd_pr = h->nd_pr; P.dpr_idx = h->d_dpr_idx; P.dpr_w = h->d_dpr_w;
-    P.nblk = h->nblk; P.blk = h->d_blk; P.blk_idx = h->d_blk_idx; P.blk_wt = h->d_blk_wt;
-    P.wt_total = h->wt_total;
-    P.blk_wt2 = h->d_blk_wt2; P.wt2_total = h->wt2_total;
-    P.nblk_idx = (int)h->h_blk_idx.size();
+    if (h->nwin > 0) {
+        // the window kernel (fit_kernel<F, 4>) reads each window's counts and offsets from P.win
+        h->win_rows.fill(P);
+        P.nwin = h->nwin; P.win = h->d_win;
+    } else {
+        h->rows.fill(P);
+    }
     P.rb = h->rb;
     {
         const char* e = getenv("B200LM_DUAL_FROM");
@@ -46,6 +47,55 @@ void fill_params(b200lm_handle_s* h, FitParams& P) {
     P.counter = h->d_counter;
     P.stats = h->d_stats;
     P.policy = h->policy;
+}
+}  // namespace b200lm
+
+template <class T>
+static cudaError_t upload(T** dst, const T* src, size_t n) {
+    if (*dst) { cudaFree(*dst); *dst = nullptr; }
+    if (n == 0) return cudaSuccess;
+    cudaError_t e = cudaMalloc((void**)dst, n * sizeof(T));
+    if (e != cudaSuccess) return e;
+    return cudaMemcpy(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice);
+}
+
+namespace b200lm {
+void WeightTables::append(const WeightTables& t) {
+    for (BlockDesc b : t.blk) {
+        b.idx_off += (int)blk_idx.size();
+        b.wt_off += (int)wt.size();
+        blk.push_back(b);
+    }
+    fn_idx.insert(fn_idx.end(), t.fn_idx.begin(), t.fn_idx.end());
+    fn_w.insert(fn_w.end(), t.fn_w.begin(), t.fn_w.end());
+    pr_idx.insert(pr_idx.end(), t.pr_idx.begin(), t.pr_idx.end());
+    pr_w.insert(pr_w.end(), t.pr_w.begin(), t.pr_w.end());
+    blk_idx.insert(blk_idx.end(), t.blk_idx.begin(), t.blk_idx.end());
+    wt.insert(wt.end(), t.wt.begin(), t.wt.end());
+}
+
+cudaError_t RowTables::upload() {
+    cudaError_t e = cudaSuccess;
+    auto put = [&e](auto** dst, const auto& v) { if (e == cudaSuccess) e = ::upload(dst, v.data(), v.size()); };
+    put(&d_fn_idx, host.fn_idx); put(&d_fn_w, host.fn_w);
+    put(&d_pr_idx, host.pr_idx); put(&d_pr_w, host.pr_w);
+    put(&d_blk, host.blk); put(&d_blk_idx, host.blk_idx);
+    put(&d_wt, host.wt); put(&d_wt2, host.wt2);
+    return e;
+}
+
+void RowTables::free() {
+    cudaFree(d_fn_idx); cudaFree(d_fn_w); cudaFree(d_pr_idx); cudaFree(d_pr_w);
+    cudaFree(d_blk); cudaFree(d_blk_idx); cudaFree(d_wt); cudaFree(d_wt2);
+}
+
+void RowTables::fill(FitParams& P) const {
+    P.nd_fn = (int)host.fn_idx.size(); P.dfn_idx = d_fn_idx; P.dfn_w = d_fn_w;
+    P.nd_pr = (int)host.pr_idx.size(); P.dpr_idx = d_pr_idx; P.dpr_w = d_pr_w;
+    P.nblk = (int)host.blk.size(); P.blk = d_blk;
+    P.blk_idx = d_blk_idx; P.nblk_idx = (int)host.blk_idx.size();
+    P.blk_wt = d_wt; P.wt_total = (int)host.wt.size();
+    P.blk_wt2 = d_wt2; P.wt2_total = (int)host.wt2.size();
 }
 }  // namespace b200lm
 
@@ -85,7 +135,7 @@ static std::deque<FunctorEntry>& registry() {
 static int default_team(b200lm_handle_s* h) {
     if (h->team_request > 0) return h->team_request;
     int big = 0;
-    for (const auto& b : h->h_blk) big = b.n_in > big ? b.n_in : big;
+    for (const auto& b : h->rows.host.blk) big = b.n_in > big ? b.n_in : big;
     if (big >= 32 && h->np >= 12) return h->fe->fit_team[0] ? 2 : 4;
     return 1;
 }
@@ -128,7 +178,7 @@ __global__ void __launch_bounds__(256) queue_order_kernel(int B, const double* _
 // predictor (rank correlation 0.18 with the evaluation count) to pay for its own pass on average.  On request:
 // b200lm_set_order(h, 1) or B200LM_ORDER=1.
 static bool order_wanted(b200lm_handle_s* h, int B) {
-    if (B > ORDER_MAX_B || B < 2) return false;
+    if (h->nwin > 0 || B > ORDER_MAX_B || B < 2) return false;
     if (const char* env = getenv("B200LM_ORDER")) return atoi(env) != 0;
     return h->order_request == 1;
 }
@@ -136,33 +186,31 @@ static bool order_wanted(b200lm_handle_s* h, int B) {
 // shapes the wave kernel takes (lm_wave.cuh): one correlated block of <= 64 points, every other entry a 1x1 prior
 // row, np <= 16, the scipy policy
 static bool wave_ok(b200lm_handle_s* h) {
-    if (!h->fe->fit_wave || h->policy != 0 || h->np > 16 || h->nblk != 1 || h->nd_fn != 0) return false;
-    const auto& b = h->h_blk[0];
+    const WeightTables& t = h->rows.host;
+    if (!h->fe->fit_wave || h->policy != 0 || h->np > 16 || t.blk.size() != 1 || !t.fn_idx.empty()) return false;
+    const auto& b = t.blk[0];
     if (b.n_in > 64 || b.n_out > 64 || b.n_out < 1) return false;
-    return h->fe->wave_bytes(h->wt_total) <= h->smem_budget;
+    return h->fe->wave_bytes((int)t.wt.size()) <= h->smem_budget;
+}
+
+// The warps per fit of a batch: 1 (fit_kernel), 2 or 4 (fit_team_kernel) or 32 (the wave kernel).  Windows run in
+// the one-warp kernel (fit_kernel<F, 4>), and so do the GSL decisions and the bounded scipy decisions (fit_kernel<F, 1>
+// and <F, 3>).  Otherwise B200LM_TEAM = 0/1, 2, 4, 32 overrides default_team, and a team that the functor or the
+// shapes do not allow falls back to one warp.
+static int kernel_team(b200lm_handle_s* h) {
+    if (h->nwin > 0 || h->policy == 1 || h->bounded) return 1;
+    int team = default_team(h);
+    if (const char* env = getenv("B200LM_TEAM")) team = atoi(env);
+    if (team == 32) return wave_ok(h) ? 32 : 1;
+    const int ti = team == 4 ? 1 : (team == 2 ? 0 : -1);
+    return ti >= 0 && h->fe->fit_team[ti] && h->fe->team_bytes[ti](h->N) <= h->smem_budget ? team : 1;
 }
 
 #define CUDA_TRY(h, call, what) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return cuda_fail(h, e_, what); } while (0)
 
-template <class T>
-static cudaError_t upload(T** dst, const T* src, size_t n) {
-    if (*dst) { cudaFree(*dst); *dst = nullptr; }
-    if (n == 0) return cudaSuccess;
-    cudaError_t e = cudaMalloc((void**)dst, n * sizeof(T));
-    if (e != cudaSuccess) return e;
-    return cudaMemcpy(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice);
-}
-
 // One whitening description (the arguments of b200lm_set_weights), checked and laid out for the kernels.
 // allowed[i]: 0 = entry i of y(+)prior must not appear, 1 = may appear, 2 = must appear; each appears at most once.
 // Returns "" or the error ("size": a block too large for the shared-memory plan).
-struct WeightTables {
-    std::vector<int> fn_idx, pr_idx, blk_idx;
-    std::vector<double> fn_w, pr_w, wt, wt2;
-    std::vector<BlockDesc> blk;
-    int nchiv = 0, ndata = 0;
-    long long nw = 0;              // doubles of blk_w read
-};
 
 static std::string parse_weights(b200lm_handle_s* h, const std::vector<char>& allowed, int ndiag, const int* diag_idx,
                                  const double* diag_w, int nblk, const int* blk_nin, const int* blk_nout,
@@ -384,13 +432,10 @@ void b200lm_destroy(b200lm_handle h) {
     if (!h) return;
     cudaSetDevice(h->device);
     cudaFree(h->d_x);
-    cudaFree(h->d_dfn_idx); cudaFree(h->d_dfn_w); cudaFree(h->d_dpr_idx); cudaFree(h->d_dpr_w);
-    cudaFree(h->d_blk); cudaFree(h->d_blk_idx); cudaFree(h->d_blk_wt); cudaFree(h->d_blk_wt2); cudaFree(h->d_wfull);
+    h->rows.free(); h->win_rows.free(); cudaFree(h->d_win); cudaFree(h->d_wfull);
     cudaFree(h->d_counter); cudaFree(h->d_stats); cudaFree(h->d_stage); cudaFree(h->d_scratch);
     cudaFree(h->d_order_key); cudaFree(h->d_order); cudaFree(h->d_wave_A);
     cudaFree(h->d_lb); cudaFree(h->d_ub);
-    cudaFree(h->d_win); cudaFree(h->d_win_dfn_idx); cudaFree(h->d_win_dfn_w); cudaFree(h->d_win_dpr_idx);
-    cudaFree(h->d_win_dpr_w); cudaFree(h->d_win_blk); cudaFree(h->d_win_blk_idx); cudaFree(h->d_win_blk_wt);
     if (h->h_pinned) cudaFreeHost(h->h_pinned);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -416,20 +461,9 @@ int b200lm_set_weights(b200lm_handle h, int ndiag, const int* diag_idx, const do
     if (!err.empty()) return set_error(h, err == "size" ? B200LM_ESIZE : B200LM_EINVAL,
                                        err == "size" ? "correlated block too large for the per-warp shared-memory plan"
                                                      : err);
-    const int idx_off = (int)t.blk_idx.size();
-    h->nd_fn = (int)t.fn_idx.size(); h->nd_pr = (int)t.pr_idx.size();
-    CUDA_TRY(h, upload(&h->d_dfn_idx, t.fn_idx.data(), t.fn_idx.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_dfn_w, t.fn_w.data(), t.fn_w.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_dpr_idx, t.pr_idx.data(), t.pr_idx.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_dpr_w, t.pr_w.data(), t.pr_w.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk, t.blk.data(), t.blk.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk_idx, blk_idx, (size_t)idx_off), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk_wt, t.wt.data(), t.wt.size()), "upload weights");
-    CUDA_TRY(h, upload(&h->d_blk_wt2, t.wt2.data(), t.wt2.size()), "upload weights");
-    h->wt2_total = (int)t.wt2.size();
-    h->nblk = nblk; h->wt_total = (int)t.wt.size(); h->rb = 32; h->nchiv = t.nchiv;
-    h->h_diag_idx.assign(diag_idx, diag_idx + ndiag); h->h_diag_w.assign(diag_w, diag_w + ndiag);
-    h->h_blk = t.blk; h->h_blk_idx.assign(blk_idx, blk_idx + idx_off);
+    h->rows.host = std::move(t);
+    CUDA_TRY(h, h->rows.upload(), "upload weights");
+    h->rb = 32; h->nchiv = h->rows.host.nchiv;
     if (h->d_wfull) { cudaFree(h->d_wfull); h->d_wfull = nullptr; }
     h->have_weights = true;
     h->nwin = 0;
@@ -448,11 +482,9 @@ int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* d
     WeightTables all;
     std::vector<WinDesc> win(nwin);
     std::vector<int> nchiv(nwin);
-    std::vector<int> idx_all;
     long long o_diag = 0, o_blk = 0, o_idx = 0, o_w = 0;
     for (int w = 0; w < nwin; ++w) {
         const std::string where = "window " + std::to_string(w) + ": ";
-        if (ndiag[w] < 0 || nblk[w] < 0) return set_error(h, B200LM_EINVAL, where + "bad weight description");
         WeightTables t;
         const std::string err = parse_weights(h, allowed, ndiag[w], diag_idx ? diag_idx + o_diag : nullptr,
                                               diag_w ? diag_w + o_diag : nullptr, nblk[w],
@@ -465,28 +497,13 @@ int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* d
         WinDesc& d = win[w];
         d.nd_fn = (int)t.fn_idx.size(); d.nd_pr = (int)t.pr_idx.size(); d.nblk = nblk[w]; d.nchiv = t.nchiv;
         d.dfn_off = (int)all.fn_idx.size(); d.dpr_off = (int)all.pr_idx.size(); d.blk_off = (int)all.blk.size();
-        for (auto b : t.blk) {               // offsets into the concatenated tables
-            b.idx_off += (int)idx_all.size();
-            b.wt_off += (int)all.wt.size();
-            all.blk.push_back(b);
-        }
-        all.fn_idx.insert(all.fn_idx.end(), t.fn_idx.begin(), t.fn_idx.end());
-        all.fn_w.insert(all.fn_w.end(), t.fn_w.begin(), t.fn_w.end());
-        all.pr_idx.insert(all.pr_idx.end(), t.pr_idx.begin(), t.pr_idx.end());
-        all.pr_w.insert(all.pr_w.end(), t.pr_w.begin(), t.pr_w.end());
-        all.wt.insert(all.wt.end(), t.wt.begin(), t.wt.end());
-        idx_all.insert(idx_all.end(), t.blk_idx.begin(), t.blk_idx.end());
+        all.append(t);
         nchiv[w] = t.nchiv;
         o_diag += ndiag[w]; o_blk += nblk[w]; o_idx += (long long)t.blk_idx.size(); o_w += t.nw;
     }
     CUDA_TRY(h, upload(&h->d_win, win.data(), win.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_dfn_idx, all.fn_idx.data(), all.fn_idx.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_dfn_w, all.fn_w.data(), all.fn_w.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_dpr_idx, all.pr_idx.data(), all.pr_idx.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_dpr_w, all.pr_w.data(), all.pr_w.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_blk, all.blk.data(), all.blk.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_blk_idx, idx_all.data(), idx_all.size()), "upload windows");
-    CUDA_TRY(h, upload(&h->d_win_blk_wt, all.wt.data(), all.wt.size()), "upload windows");
+    h->win_rows.host = std::move(all);
+    CUDA_TRY(h, h->win_rows.upload(), "upload windows");
     h->nwin = nwin;
     h->win_nchiv = nchiv;
     h->nchiv = *std::max_element(nchiv.begin(), nchiv.end());
@@ -540,7 +557,6 @@ int b200lm_fit_batch(b200lm_handle h, int B,
         return set_error(h, B200LM_EINVAL, "bounds need the scipy trf policy (GSL's lm has no bound constraints)");
     rc = window_refusal(h, B);
     if (rc) return rc;
-    if (B == 0) return B200LM_OK;
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
     FitParams P;
@@ -550,24 +566,9 @@ int b200lm_fit_batch(b200lm_handle h, int B,
     P.x_out = d_x; P.chi2 = d_chi2; P.cov = d_cov; P.logdet = d_logdet; P.nit = d_nit; P.status = d_status;
     P.f_out = d_f; P.J_out = d_J;
     if (h->bounded) { P.bounded = 1; P.lb = h->d_lb; P.ub = h->d_ub; }
+    if (h->nwin > 0) P.win_copies = B / h->nwin;
     CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(int), s), "reset work queue");
     CUDA_TRY(h, cudaMemsetAsync(h->d_stats, 0, 16 * sizeof(unsigned long long), s), "reset stats");
-    if (h->nwin > 0) {
-        // fit windows: the window kernel (fit_kernel<F, 4>), one warp per fit, queue in input order; the row tables are
-        // those of every window, addressed through P.win
-        P.nwin = h->nwin; P.win_copies = B / h->nwin; P.win = h->d_win;
-        P.nd_fn = 0; P.nd_pr = 0; P.nblk = 0;
-        P.dfn_idx = h->d_win_dfn_idx; P.dfn_w = h->d_win_dfn_w; P.dpr_idx = h->d_win_dpr_idx; P.dpr_w = h->d_win_dpr_w;
-        P.blk = h->d_win_blk; P.blk_idx = h->d_win_blk_idx; P.blk_wt = h->d_win_blk_wt;
-        P.wt_total = 0; P.blk_wt2 = nullptr; P.wt2_total = 0; P.nblk_idx = 0;
-        P.team = 1;
-        CUDA_TRY(h, h->fe->fit(P, h->sm_count, h->smem_budget, s), "window fit kernel launch");
-        h->last_order = 0;
-        h->last_team = 1;
-        h->last_stream = s;
-        h->launches += 1;
-        return B200LM_OK;
-    }
     // queue order: chi2 at the start point of every fit (one evaluation each, resjac kernel without f / J outputs),
     // ranked on the device
     h->last_order = 0;
@@ -589,30 +590,21 @@ int b200lm_fit_batch(b200lm_handle h, int B,
         h->last_order = 1;
         h->launches += 2;
     }
-    // kernel choice: one warp per fit, or a team of 2 / 4 warps per fit where the functor has one
-    // (B200LM_TEAM = 0/1, 2, 4 overrides the default policy)
-    int team = default_team(h);
-    if (const char* env = getenv("B200LM_TEAM")) team = atoi(env);
-    if (h->policy == 1) team = 1;            // the GSL decisions are compiled into the one-warp kernel only (fit_kernel<F, 1>)
-    if (h->bounded) team = 1;                // so are the bounded scipy decisions (fit_kernel<F, 3>)
-    const int ti = team == 4 ? 1 : (team == 2 ? 0 : -1);
-    if (team == 32 && wave_ok(h)) {
+    P.team = kernel_team(h);
+    if (P.team == 32) {
         // wave kernel: the trust-region loops of 32 fits per CTA in lock step, then covariance / log det / f / J
-        // (and polish) of every fit by the one-warp kernel in finalize_only mode
-        P.team = 32;
-        {
-            // hand J^T J at every solution to the finalisation pass (np(np+1)/2 doubles per fit; skipped above 2 GB,
-            // the pass then evaluates the model once more as it did before)
-            const size_t need = (size_t)B * (size_t)(h->np * (h->np + 1) / 2);
-            if (need * sizeof(double) <= ((size_t)2 << 30) && !getenv("B200LM_WAVE_REEVAL")) {
-                if (need > h->wave_A_cap) {
-                    if (h->d_wave_A) cudaFree(h->d_wave_A);
-                    h->d_wave_A = nullptr; h->wave_A_cap = 0;
-                    if (cudaMalloc((void**)&h->d_wave_A, need * sizeof(double)) == cudaSuccess) h->wave_A_cap = need;
-                    else cudaGetLastError();
-                }
-                P.wave_A = h->wave_A_cap >= need ? h->d_wave_A : nullptr;
+        // (and polish) of every fit by the one-warp kernel in finalize_only mode.
+        // J^T J at every solution goes to the finalisation pass (np(np+1)/2 doubles per fit; skipped above 2 GB,
+        // the pass then evaluates the model once more as it did before)
+        const size_t need = (size_t)B * (size_t)(h->np * (h->np + 1) / 2);
+        if (need * sizeof(double) <= ((size_t)2 << 30) && !getenv("B200LM_WAVE_REEVAL")) {
+            if (need > h->wave_A_cap) {
+                if (h->d_wave_A) cudaFree(h->d_wave_A);
+                h->d_wave_A = nullptr; h->wave_A_cap = 0;
+                if (cudaMalloc((void**)&h->d_wave_A, need * sizeof(double)) == cudaSuccess) h->wave_A_cap = need;
+                else cudaGetLastError();
             }
+            P.wave_A = h->wave_A_cap >= need ? h->d_wave_A : nullptr;
         }
         CUDA_TRY(h, h->fe->fit_wave(P, h->sm_count, h->smem_budget, s), "wave kernel launch");
         CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(int), s), "reset work queue");
@@ -620,13 +612,10 @@ int b200lm_fit_batch(b200lm_handle h, int B,
         Q.finalize_only = 1; Q.p0 = d_x; Q.p0_stride = h->np; Q.team = 1; Q.order = nullptr;
         CUDA_TRY(h, h->fe->fit(Q, h->sm_count, h->smem_budget, s), "finalize kernel launch");
         h->launches += 1;
-    } else if (ti >= 0 && h->fe->fit_team[ti] &&
-        h->fe->team_bytes[ti](h->N) <= h->smem_budget) {
-        P.team = team;
-        CUDA_TRY(h, h->fe->fit_team[ti](P, h->sm_count, h->smem_budget, s), "fit kernel launch");
+    } else if (P.team > 1) {
+        CUDA_TRY(h, h->fe->fit_team[P.team == 4 ? 1 : 0](P, h->sm_count, h->smem_budget, s), "fit kernel launch");
     } else {
-        P.team = 1;
-        CUDA_TRY(h, h->fe->fit(P, h->sm_count, h->smem_budget, s), "fit kernel launch");
+        CUDA_TRY(h, h->fe->fit(P, h->sm_count, h->smem_budget, s), h->nwin ? "window fit kernel launch" : "fit kernel launch");
     }
     h->last_team = P.team;
     h->last_stream = s;

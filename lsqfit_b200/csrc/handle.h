@@ -5,6 +5,33 @@
 #include <cuda_runtime.h>
 #include "registry.h"
 
+namespace b200lm {
+
+// One whitening laid out for the kernels (parse_weights in capi.cu).
+struct WeightTables {
+    std::vector<int> fn_idx, pr_idx, blk_idx;
+    std::vector<double> fn_w, pr_w, wt, wt2;
+    std::vector<BlockDesc> blk;
+    int nchiv = 0, ndata = 0;
+    long long nw = 0;              // doubles of blk_w read
+    // t's rows after these (a window scan's windows, one after the other); not wt2: windows run in the one-warp kernel
+    void append(const WeightTables& t);
+};
+
+// Row tables on the host and their device copies.
+struct RowTables {
+    WeightTables host;
+    int* d_fn_idx = nullptr; double* d_fn_w = nullptr;
+    int* d_pr_idx = nullptr; double* d_pr_w = nullptr;
+    BlockDesc* d_blk = nullptr; int* d_blk_idx = nullptr;
+    double* d_wt = nullptr; double* d_wt2 = nullptr;
+    cudaError_t upload();                   // host -> device (wt2 where the host tables have it)
+    void free();
+    void fill(FitParams& P) const;          // the row-table fields of P
+};
+
+}  // namespace b200lm
+
 struct b200lm_handle_s {
     int device = 0;
     int sm_count = 0;
@@ -13,16 +40,9 @@ struct b200lm_handle_s {
     int ny = 0, np = 0, nx = 0, noprior = 0, N = 0, nchiv = 0;
     // device-resident problem description
     double* d_x = nullptr;
-    int* d_dfn_idx = nullptr; double* d_dfn_w = nullptr; int nd_fn = 0;
-    int* d_dpr_idx = nullptr; double* d_dpr_w = nullptr; int nd_pr = 0;
-    b200lm::BlockDesc* d_blk = nullptr; int nblk = 0;
-    int* d_blk_idx = nullptr; double* d_blk_wt = nullptr; int wt_total = 0;
-    double* d_blk_wt2 = nullptr; int wt2_total = 0;      // team-kernel layout of the same weights
+    b200lm::RowTables rows;     // the plan's whitening (b200lm_set_weights)
     int rb = 64;
     bool have_weights = false, have_const = false;
-    // host copies (used by propagate)
-    std::vector<int> h_diag_idx; std::vector<double> h_diag_w;
-    std::vector<b200lm::BlockDesc> h_blk; std::vector<int> h_blk_idx;
     // whole whitening operator, dense [nchiv][N] (built lazily for propagate)
     double* d_wfull = nullptr;
     // work queue + statistics
@@ -42,9 +62,7 @@ struct b200lm_handle_s {
     int nwin = 0;
     std::vector<int> win_nchiv;
     b200lm::WinDesc* d_win = nullptr;
-    int* d_win_dfn_idx = nullptr; double* d_win_dfn_w = nullptr;
-    int* d_win_dpr_idx = nullptr; double* d_win_dpr_w = nullptr;
-    b200lm::BlockDesc* d_win_blk = nullptr; int* d_win_blk_idx = nullptr; double* d_win_blk_wt = nullptr;
+    b200lm::RowTables win_rows;
     // queue order (longest-expected fits first): key = chi2 at the start point, one evaluation per fit
     int order_request = -1;     // -1: default policy (by problem shape and batch size); 0: off; 1: on  (b200lm_set_order)
     int last_order = 0;         // 1 if the last fit_batch launch used an ordered queue

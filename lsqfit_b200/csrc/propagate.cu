@@ -30,18 +30,15 @@ extern "C" int b200lm_propagate(b200lm_handle h, int B, const double* d_x, const
     const int np = h->np, N = h->N, nchiv = h->nchiv;
     // dense whitening operator W [nchiv][N], built once per weight set
     if (!h->d_wfull) {
+        const WeightTables& t = h->rows.host;
         std::vector<double> W((size_t)nchiv * N, 0.0);
-        const int ndiag = (int)h->h_diag_idx.size();
-        for (int i = 0; i < ndiag; ++i) W[(size_t)i * N + h->h_diag_idx[i]] = h->h_diag_w[i];
-        std::vector<double> wt(h->wt_total);
-        if (h->wt_total) {
-            e = cudaMemcpy(wt.data(), h->d_blk_wt, wt.size() * sizeof(double), cudaMemcpyDeviceToHost);
-            if (e != cudaSuccess) return cuda_fail(h, e, "read weights");
-        }
-        for (auto& b : h->h_blk)
+        const int nfn = (int)t.fn_idx.size();      // 1x1 rows: data rows first, then prior rows
+        for (int i = 0; i < nfn; ++i) W[(size_t)i * N + t.fn_idx[i]] = t.fn_w[i];
+        for (size_t i = 0; i < t.pr_idx.size(); ++i) W[(nfn + i) * N + t.pr_idx[i]] = t.pr_w[i];
+        for (auto& b : t.blk)
             for (int r = 0; r < b.n_out; ++r)
                 for (int j = 0; j < b.n_in; ++j)
-                    W[(size_t)(b.chiv_off + r) * N + h->h_blk_idx[b.idx_off + j]] = wt[b.wt_off + (size_t)r * b.ldw + j];
+                    W[(size_t)(b.chiv_off + r) * N + t.blk_idx[b.idx_off + j]] = t.wt[b.wt_off + (size_t)r * b.ldw + j];
         e = cudaMalloc((void**)&h->d_wfull, W.size() * sizeof(double));
         if (e == cudaSuccess) e = cudaMemcpy(h->d_wfull, W.data(), W.size() * sizeof(double), cudaMemcpyHostToDevice);
         if (e != cudaSuccess) return cuda_fail(h, e, "upload dense whitening operator");

@@ -165,6 +165,30 @@ class Plan(object):
         finally:
             _cabi.lib.b200lm_set_bounds(self._h, None, None)
 
+    def _prepare(self, mean, sm, p0, sp, tol, maxit, scaler, polish, policy, bounds, want_cov, want_fJ, B=None):
+        """What both launch entries check and compute.  mean [rows, N] (sm = N) or [N] (sm = 0), p0 likewise; with
+        windows a row of means per copy and a start per window.  -> (B, solver arguments of the C entry, bounds as
+        two host arrays or None, shape and dtype of every output asked for, None for the others)."""
+        xtol, gtol, ftol = normalize_tol(tol)
+        sc = self._set_policy(policy, scaler)
+        if B is None:
+            B = ((mean.shape[0] if sm else 1) * self.nwin if self.nwin else
+                 (mean.shape[0] if sm else (p0.shape[0] if sp else 1)))
+        rows_m, rows_p = (B // self.nwin, self.nwin) if self.nwin else (B, B)
+        if (sm and mean.shape[0] != rows_m) or (sp and p0.shape[0] != rows_p):
+            raise ValueError("mean and p0 disagree on the batch size")
+        if bounds is not None:
+            bounds = self._bounds(bounds)
+            lo, hi = ((torch.as_tensor(b).to(p0.device) for b in bounds) if isinstance(p0, torch.Tensor) else bounds)
+            if not bool(((p0 >= lo) & (p0 <= hi)).all()):             # one reduction (scipy: "`x0` is infeasible.")
+                raise ValueError("`x0` is infeasible.")
+        # 1-d shapes as B, not (B,): torch parses an int faster, and a launch of one fit is host bound
+        f8, i4 = np.float64, np.int32
+        shapes = dict(x=((B, self.np), f8), chi2=(B, f8), cov=((B, self.np, self.np), f8) if want_cov else None,
+                      logdet=(B, f8), nit=(B, i4), status=(B, i4), f=((B, self.nchiv), f8) if want_fJ else None,
+                      J=((B, self.nchiv, self.np), f8) if want_fJ else None)
+        return B, (xtol, gtol, ftol, int(maxit), sc, int(polish)), bounds, shapes
+
     def fit_batch(self, mean, p0, tol=1e-8, maxit=1000, scaler="more", B=None,
                   want_cov=True, want_fJ=False, out=None, polish=0, policy="trf", bounds=None):
         """Fit B problems on the device; inputs may be numpy arrays or device tensors.
@@ -172,35 +196,17 @@ class Plan(object):
         mean: [B, N] or [N] (shared);  p0: [B, np] or [np] (shared).
         bounds: None or (lb, ub) in device parameter order, scipy's ``bounds`` (±inf: none); p0 must lie in the box.
         Returns a BatchResult of device tensors (no host synchronisation)."""
-        xtol, gtol, ftol = normalize_tol(tol)
-        sc = self._set_policy(policy, scaler)
         tm, sm = self._dev(mean, self.N)
         tp, sp = self._dev(p0, self.np)
-        if bounds is not None:
-            bounds = self._bounds(bounds)
-            tl, tu = (torch.as_tensor(b).to(self.tdev) for b in bounds)
-            if not bool(torch.all((tp >= tl) & (tp <= tu))):           # one reduction (scipy: "`x0` is infeasible.")
-                raise ValueError("`x0` is infeasible.")
-        if B is None:
-            B = ((tm.shape[0] if sm else 1) * self.nwin if self.nwin else
-                 (tm.shape[0] if sm else (tp.shape[0] if sp else 1)))
-        # with windows: a row of means per copy, a start per window
-        rows_m, rows_p = (B // self.nwin, self.nwin) if self.nwin else (B, B)
-        if (sm and tm.shape[0] != rows_m) or (sp and tp.shape[0] != rows_p):
-            raise ValueError("mean and p0 disagree on the batch size")
+        B, solver, bounds, shapes = self._prepare(tm, sm, tp, sp, tol, maxit, scaler, polish, policy, bounds,
+                                                  want_cov, want_fJ, B)
         if out is None:
-            kw = dict(device=self.tdev, dtype=torch.float64)
-            out = BatchResult(
-                torch.empty((B, self.np), **kw), torch.empty(B, **kw),
-                torch.empty((B, self.np, self.np), **kw) if want_cov else None,
-                torch.empty(B, **kw),
-                torch.empty(B, device=self.tdev, dtype=torch.int32),
-                torch.empty(B, device=self.tdev, dtype=torch.int32),
-                torch.empty((B, self.nchiv), **kw) if want_fJ else None,
-                torch.empty((B, self.nchiv, self.np), **kw) if want_fJ else None)
+            out = BatchResult(*[s and torch.empty(s[0], device=self.tdev,
+                                                  dtype=torch.int32 if s[1] is np.int32 else torch.float64)
+                                for s in shapes.values()])
         ptr = lambda t: t.data_ptr() if t is not None else None
         self._launch_bounded(bounds, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch(
-            self._h, B, tm.data_ptr(), sm, tp.data_ptr(), sp, xtol, gtol, ftol, int(maxit), sc, int(polish),
+            self._h, B, tm.data_ptr(), sm, tp.data_ptr(), sp, *solver,
             out.x.data_ptr(), out.chi2.data_ptr(), ptr(out.cov), out.logdet.data_ptr(),
             out.nit.data_ptr(), out.status.data_ptr(), ptr(out.f), ptr(out.J), self._stream()), self._h))
         out._keep = (tm, tp)        # keep inputs alive until the stream has consumed them
@@ -211,8 +217,6 @@ class Plan(object):
         """Same fit through the host-buffer C entry point: numpy in, numpy out.
         ``out`` may hold preallocated arrays (dict with keys x, chi2, cov, logdet, nit, status).
         ``bounds`` as for fit_batch."""
-        xtol, gtol, ftol = normalize_tol(tol)
-        sc = self._set_policy(policy, scaler)
         # the C entry point reads raw host pointers: dtype, contiguity and shapes are checked HERE
         # (np.ascontiguousarray is a no-op for conforming arrays)
         mean = np.ascontiguousarray(mean, dtype=np.float64)
@@ -223,19 +227,11 @@ class Plan(object):
             raise ValueError("p0 must be [np] or [B, np] with np = %d, got %s" % (self.np, p0.shape))
         sm = 0 if mean.ndim == 1 else self.N
         sp = 0 if p0.ndim == 1 else self.np
-        B = mean.shape[0] if sm else (p0.shape[0] if sp else 1)
-        if (sm and mean.shape[0] != B) or (sp and p0.shape[0] != B):
-            raise ValueError("mean and p0 disagree on the batch size")
-        shapes = dict(x=((B, self.np), np.float64), chi2=((B,), np.float64), cov=((B, self.np, self.np), np.float64),
-                      logdet=((B,), np.float64), nit=((B,), np.int32), status=((B,), np.int32),
-                      f=((B, self.nchiv), np.float64), J=((B, self.nchiv, self.np), np.float64))
+        # every array of a given ``out`` is checked
+        B, solver, bounds, shapes = self._prepare(mean, sm, p0, sp, tol, maxit, scaler, polish, policy, bounds,
+                                                  want_cov or out is not None, want_fJ or out is not None)
         if out is None:
-            out = dict(
-                x=np.empty((B, self.np)), chi2=np.empty(B),
-                cov=np.empty((B, self.np, self.np)) if want_cov else None, logdet=np.empty(B),
-                nit=np.empty(B, dtype=np.int32), status=np.empty(B, dtype=np.int32),
-                f=np.empty((B, self.nchiv)) if want_fJ else None,
-                J=np.empty((B, self.nchiv, self.np)) if want_fJ else None)
+            out = dict((k, s and np.empty(*s)) for k, s in shapes.items())
         else:
             for k in ("x", "chi2", "logdet", "nit", "status"):
                 if out.get(k) is None:
@@ -244,17 +240,14 @@ class Plan(object):
                 a = out.get(k)
                 if a is None:
                     continue
+                shp = shp if isinstance(shp, tuple) else (shp,)
                 if not (isinstance(a, np.ndarray) and a.dtype == dt and a.flags["C_CONTIGUOUS"]
                         and a.flags["WRITEABLE"] and tuple(a.shape) == shp):
                     raise ValueError("out[%r] must be a writable C-contiguous %s array of shape %s"
                                      % (k, np.dtype(dt).name, shp))
-        if bounds is not None:
-            bounds = self._bounds(bounds)
-            if not np.all((p0 >= bounds[0]) & (p0 <= bounds[1])):
-                raise ValueError("`x0` is infeasible.")
         ptr = lambda a: a.ctypes.data if a is not None else None
         self._launch_bounded(bounds, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch_host(
-            self._h, B, mean.ctypes.data, sm, p0.ctypes.data, sp, xtol, gtol, ftol, int(maxit), sc, int(polish),
+            self._h, B, mean.ctypes.data, sm, p0.ctypes.data, sp, *solver,
             ptr(out["x"]), ptr(out["chi2"]), ptr(out.get("cov")), ptr(out["logdet"]),
             ptr(out["nit"]), ptr(out["status"]), ptr(out.get("f")), ptr(out.get("J"))), self._h))
         return out

@@ -24,7 +24,7 @@ import time
 import numpy as np
 import torch
 
-from .engine import STOPPING_CRITERION, BatchResult, normalize_tol
+from .engine import STOPPING_CRITERION, BatchResult
 from .fitter import ChivSpec, DeviceChiv, b200_lm
 from .functors import Functor
 from .whiten import PDF
@@ -221,33 +221,37 @@ class nonlinear_fit(object):
             warnings.warn("Possible roundoff errors in fit.p; try svd cut.")
 
     # ---- batched drivers ---------------------------------------------------------------
-    def _batch(self, means, p0, tol=None, maxit=None, want_cov=True, **kargs):
-        plan = self._spec.plan(self.device)
-        args = dict(self.fitterargs)
-        args.update(kargs)
-        args.pop("device", None)
-        # kernel=: None (default, by problem shape), 1 / 2 / 4 warps per fit, or 32 / 'wave' -- the wave kernel, the
-        # fastest on saturated batches (10^5 ... 10^6 copies of a small model); see b200lm_set_team
-        kernel = args.pop("kernel", None)
-        kernel = 32 if kernel == "wave" else kernel
-        if args.get("loss", "linear") != "linear":
-            raise ValueError("batched fits with a robust loss (loss=%r) are not built: fit the copies one at a time "
-                             "(fitter='b200_dense')" % (args["loss"],))
-        # scipy's bounds=(lower, upper) in this fit's parameter order -> device order (as the single-fit path does)
-        bounds = args.pop("bounds", None)
+    def _batch_args(self, kargs):
+        """This fit's fitter arguments with ``kargs`` over them, as the batch drivers read them -> (the arguments of
+        ``Plan.fit_batch``, kernel, loss, gsl).  tol and maxit default to this fit's; scipy's bounds=(lower, upper)
+        in this fit's parameter order go to device order (as the single-fit path does).  kernel=: None (default, by
+        problem shape), 1 / 2 / 4 warps per fit, or 32 / 'wave' -- the wave kernel, the fastest on saturated batches
+        (10^5 ... 10^6 copies of a small model); see b200lm_set_team."""
+        from .engine import POLICY
+        args = dict(self.fitterargs, **kargs)
+        bounds = args.get("bounds")
         if bounds is not None:
-            from .engine import POLICY
-            if POLICY.get(args.get("policy", "trf")) == 1:
-                raise ValueError("b200_lm: policy='gsl' has no bound constraints")
             bounds = tuple(self._spec.to_device(np.broadcast_to(np.asarray(b, dtype=float), (self._spec.np,)))
                            for b in bounds)
+        fit = dict(tol=self.tol if args.get("tol") is None else args["tol"],
+                   maxit=self.maxit if args.get("maxit") is None else args["maxit"],
+                   scaler=args.get("scaler", "more"), polish=args.get("polish", 0), policy=args.get("policy", "trf"),
+                   bounds=bounds)
+        kernel = args.get("kernel")
+        return fit, 32 if kernel == "wave" else kernel, args.get("loss", "linear"), POLICY.get(fit["policy"]) == 1
+
+    def _batch(self, means, p0, tol=None, maxit=None, want_cov=True, **kargs):
+        plan = self._spec.plan(self.device)
+        args, kernel, loss, gsl = self._batch_args(dict(kargs, tol=tol, maxit=maxit))
+        if loss != "linear":
+            raise ValueError("batched fits with a robust loss (loss=%r) are not built: fit the copies one at a time "
+                             "(fitter='b200_dense')" % (loss,))
+        if gsl and args["bounds"] is not None:
+            raise ValueError("b200_lm: policy='gsl' has no bound constraints")
         if kernel is not None:
             plan.set_team(int(kernel))
         try:
-            out = plan.fit_batch(means, p0, tol=self.tol if tol is None else tol,
-                                 maxit=self.maxit if maxit is None else maxit, want_cov=want_cov,
-                                 scaler=args.pop("scaler", "more"), polish=args.pop("polish", 0),
-                                 policy=args.pop("policy", "trf"), bounds=bounds)
+            out = plan.fit_batch(means, p0, want_cov=want_cov, **args)
         finally:
             if kernel is not None:
                 plan.set_team(0)                 # (the plan is cached and shared: back to the default policy)
@@ -404,19 +408,17 @@ class WindowScan(object):
     window's whitening.  The scan owns its plan: the parent's (cached, shared) plan is left as it was."""
 
     def __init__(self, parent, masks, p0=None, **kargs):
-        from .engine import POLICY, Plan
+        from .engine import Plan
         from .whiten import cov_blocks, whiten_blocks
         from .windows import check_masks, window_cov, window_weights
-        args = dict(parent.fitterargs)
-        args.update(kargs)
-        args.pop("device", None)
-        args.pop("kernel", None)                     # window batches always run one warp per fit
+        # kernel= is ignored: window batches always run one warp per fit
+        self.args, _, loss, gsl = parent._batch_args(kargs)
         refuse = lambda what: ValueError("b200_lm: %s not built for window scans" % what)
-        if args.pop("bounds", None) is not None:
+        if self.args["bounds"] is not None:
             raise refuse("bounds are")
-        if args.pop("loss", "linear") != "linear":
+        if loss != "linear":
             raise refuse("a robust loss is")
-        if POLICY.get(args.get("policy", "trf")) == 1:
+        if gsl:
             raise refuse("policy='gsl' is")
         if any(parent.noise):
             raise refuse("fits made with noise are")
@@ -425,9 +427,6 @@ class WindowScan(object):
         self.np, self.ny = spec.np, spec.ny
         self.masks = check_masks(masks, self.ny)
         self.nwin = self.masks.shape[0]
-        self.tol = parent.tol if args.get("tol") is None else normalize_tol(args["tol"])
-        self.maxit = parent.maxit if args.get("maxit") is None else int(args["maxit"])
-        self.scaler, self.polish = args.get("scaler", "more"), int(args.get("polish", 0))
         pdf = parent.yp_pdf
         cov = pdf.cov_in if pdf.cov_in is not None else pdf.sdev_in
         wins = [window_cov(cov, self.ny, m) for m in self.masks]
@@ -470,7 +469,7 @@ class WindowScan(object):
         self.error = np.array([None if s > 0 else "b200_lm: no convergence" for s in a["status"]], dtype=object)
 
     def _fit(self, means, p0, B):
-        return self.plan.fit_batch(means, p0, tol=self.tol, maxit=self.maxit, scaler=self.scaler, polish=self.polish, B=B)
+        return self.plan.fit_batch(means, p0, B=B, **self.args)
 
     def __len__(self):
         return self.nwin

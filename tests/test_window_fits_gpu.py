@@ -269,6 +269,20 @@ def test_refusals_and_kernel_choice():
     _same_bits(a, b, "set_weights after set_windows")
 
 
+def test_host_entry_with_windows():
+    """fit_batch_host with windows set fits nwin x copies (means [copies, N], p0 [nwin, np]), with the bits of
+    fit_batch, whether or not the number of copies equals the number of windows."""
+    _need_gpu()
+    fit, cfg = _fit(4)
+    scan = fit.window_fits(_ranges(cfg["ny"], cfg["np"])[:6])
+    for ncopy in (50, scan.nwin):
+        means = fit.bootstrap_means(ncopy, 17)
+        dev = scan.plan.fit_batch(means, scan.pmean, tol=fit.tol, maxit=fit.maxit).numpy()
+        host = scan.plan.fit_batch_host(means.cpu().numpy(), scan.pmean, tol=fit.tol, maxit=fit.maxit)
+        assert host["x"].shape == (scan.nwin * ncopy, cfg["np"])
+        _same_bits(host, dev, ("host entry", ncopy))
+
+
 def test_parent_plan_untouched():
     _need_gpu()
     fit, cfg = _fit(8)
