@@ -238,6 +238,22 @@ int b200lm_whiten(int device, int nblk, const int* h_n, const double* d_cov,
 int b200lm_propagate(b200lm_handle h, int B, const double* d_x, const double* d_cov,
                      const double* d_C, double* d_D, double* d_covp, void* stream);
 
+/* fit.p of every window of a fit-window scan, jointly (windows set; each window is its own nonlinear_fit of the same
+ * y(+)prior).  d_cov [nwin][np][np] and d_J [nwin][nchiv][np] are the d_cov / d_J outputs of b200lm_fit_batch for the
+ * central batch (B = nwin, one copy per window; nchiv = b200lm_nchiv).  d_C [N][N] is the INPUT covariance of
+ * y(+)prior (no svd correction); d_dC holds each window's svd correction (its corrected minus its input covariance)
+ * per correlated block, n_in x n_in row-major, in b200lm_set_windows block order (NULL: no window is corrected).
+ * Outputs:
+ *   d_D [nwin][np][N] (required): D_w = cov_w . J_w^T . W_w, the derivative of window w's parameters with respect to
+ *       the full y(+)prior; columns of data rows outside the window are 0.
+ *   d_covp [nwin*np][nwin*np] (NULL: D only; needs d_C): the joint covariance of all windows' parameters,
+ *       D_w . C . D_v^T between windows w != v and D_w . C_w . D_w^T (C_w: window w's corrected covariance, the
+ *       covariance of its own fit.p) on the diagonal blocks; exactly symmetric.  (nwin*np)^2 doubles.
+ * The whitening is applied from the window row tables (no dense operator).  Scratch on the handle:
+ * nwin*np*(nchiv + N) doubles. */
+int b200lm_window_propagate(b200lm_handle h, const double* d_cov, const double* d_J, const double* d_C,
+                            const double* d_dC, double* d_D, double* d_covp, void* stream);
+
 /* ---- dense FP64 GEMM on the DMMA path ---------------------------------------------------
  * C[b] (M x N) = alpha * op(A[b]) . op(B[b]) + beta * C[b], all row-major fp64, batch strides in
  * elements (0 = operand shared by the batch).  transA: A is stored [K][M]; transB: B is stored

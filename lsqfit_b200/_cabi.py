@@ -91,6 +91,8 @@ SIGNATURES = {
                                          C.c_int, C.c_ulonglong, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "b200lm_propagate": (C.c_int, [handle_t, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p]),
+    "b200lm_window_propagate": (C.c_int, [handle_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -99,6 +99,7 @@ class Plan(object):
                                                        "blk_idx", "blk_w")]), self._h)
         self.nchiv = _cabi.lib.b200lm_nchiv(self._h)
         self.nwin = nwin
+        self._win_dC = int(np.sum(d["blk_nin"].astype(np.int64) ** 2))      # doubles of window_propagate's dC
 
     def window_nchiv(self):
         out = np.zeros(self.nwin, dtype=np.int32)
@@ -317,4 +318,36 @@ class Plan(object):
         _cabi.check(_cabi.lib.b200lm_propagate(
             self._h, B, tx.data_ptr(), tc.data_ptr(), tC.data_ptr() if tC is not None else None,
             D.data_ptr(), covp.data_ptr() if covp is not None else None, self._stream()), self._h)
+        return D, covp
+
+    def window_propagate(self, cov, J, C_in, dC=None):
+        """fit.p of every window, jointly (windows set; b200lm_window_propagate).  cov [nwin, np, np] and J
+        [nwin, nchiv, np]: the central batch's cov and J (``fit_batch(..., want_fJ=True)``); C_in [N, N]: the INPUT
+        covariance of y (+) prior (None: D only); dC: every window's svd corrections as made by
+        ``lsqfit_b200.windows.window_corrections`` (None: no window corrected).
+        -> D [nwin, np, N] and the joint covariance [nwin, np, nwin, np] (or None): D_w C_in D_v^T between windows,
+        D_w C_w D_w^T (C_w: window w's corrected covariance) within a window."""
+        if not self.nwin:
+            raise ValueError("window_propagate needs windows (set_windows)")
+        nw, npar = self.nwin, self.np
+        dev = lambda a: (a if isinstance(a, torch.Tensor) else torch.as_tensor(np.asarray(a, dtype=np.float64))).to(
+            self.tdev, dtype=torch.float64).contiguous()
+        tc = dev(cov).reshape(nw, npar, npar)
+        tJ = dev(J).reshape(nw, self.nchiv, npar)
+        kw = dict(device=self.tdev, dtype=torch.float64)
+        D = torch.empty((nw, npar, self.N), **kw)
+        tC = tdC = covp = None
+        if C_in is not None:
+            tC = dev(C_in)
+            assert tuple(tC.shape) == (self.N, self.N)
+            covp = torch.empty((nw, npar, nw, npar), **kw)
+        if dC is not None:
+            tdC = dev(dC).reshape(-1)
+            if tdC.numel() != self._win_dC:
+                raise ValueError("dC must hold %d doubles (one n_in x n_in block per correlated block of every window), "
+                                 "got %d" % (self._win_dC, tdC.numel()))
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        _cabi.check(_cabi.lib.b200lm_window_propagate(
+            self._h, tc.data_ptr(), tJ.data_ptr(), ptr(tC), ptr(tdC), D.data_ptr(), ptr(covp), self._stream()),
+            self._h)
         return D, covp

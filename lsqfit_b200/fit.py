@@ -405,7 +405,14 @@ class WindowScan(object):
 
     Arrays over windows: ``pmean psdev`` [nwin, np], ``cov`` [nwin, np, np], ``chi2 dof Q logGBF svdn nit
     stopping_criterion error`` [nwin].  ``scan[w]`` has the attribute names of ``nonlinear_fit``; ``pdfs[w]`` is the
-    window's whitening.  The scan owns its plan: the parent's (cached, shared) plan is left as it was."""
+    window's whitening.  The scan owns its plan: the parent's (cached, shared) plan is left as it was.
+
+    ``p``, ``D`` and ``p_sdev`` (computed on first access, like ``nonlinear_fit.p``): each window is its own fit of
+    the same y (+) prior, so the windows' parameters are correlated.  ``D`` [nwin, np, N] is d pmean[w] / d (y, prior)
+    (zero for data rows outside window w); ``p = (pmean, cov)`` with the joint covariance ``cov`` [nwin, np, nwin, np]:
+    ``D[w] C D[v]^T`` between windows (C: this fit's input covariance of y (+) prior) and ``D[w] C_w D[w]^T`` within
+    window w (C_w: its own svd-corrected covariance, so ``cov[w, :, w, :]`` is the window's own ``fit.p``
+    covariance)."""
 
     def __init__(self, parent, masks, p0=None, **kargs):
         from .engine import Plan
@@ -467,9 +474,36 @@ class WindowScan(object):
                                  for w, (p, d) in enumerate(zip(self.pdfs, self.dof))]))
         self.stopping_criterion = np.array([STOPPING_CRITERION[int(s)] for s in a["status"]])
         self.error = np.array([None if s > 0 else "b200_lm: no convergence" for s in a["status"]], dtype=object)
+        self._p = None
 
-    def _fit(self, means, p0, B):
-        return self.plan.fit_batch(means, p0, B=B, **self.args)
+    def _getp(self):
+        if self._p is None:
+            from .windows import window_corrections
+            # J at the solutions: the central batch once more, with f and J (the same fits, so the same bits)
+            J = self._fit(self.parent._spec.mean, self.p0, self.nwin, want_fJ=True).J
+            pdf = self.parent.yp_pdf
+            C = pdf.cov_in if pdf.cov_in is not None else np.diag(pdf.sdev_in ** 2)
+            D, covp = self.plan.window_propagate(self.out.cov, J, C, window_corrections(self.pdfs))
+            self._D = D.cpu().numpy()
+            self._p = (self.pmean, covp.cpu().numpy())
+        return self._p
+
+    p = property(_getp, doc="(pmean [nwin, np], joint covariance [nwin, np, nwin, np] of every window's fit.p).")
+
+    @property
+    def D(self):
+        """d pmean[w, a] / d buf[i], buf = y (+) prior: [nwin, np, N]."""
+        self._getp()
+        return self._D
+
+    @property
+    def p_sdev(self):
+        """[nwin, np]: standard deviations of ``p``."""
+        c = self._getp()[1].reshape(self.nwin * self.np, -1)
+        return np.sqrt(np.diagonal(c)).reshape(self.nwin, self.np)
+
+    def _fit(self, means, p0, B, want_fJ=False):
+        return self.plan.fit_batch(means, p0, B=B, want_fJ=want_fJ, **self.args)
 
     def __len__(self):
         return self.nwin

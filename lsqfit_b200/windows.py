@@ -69,3 +69,15 @@ def window_weights(sels, invwgts):
                 nblk=np.array(nb, dtype=np.int32), blk_nin=np.array(nin, dtype=np.int32),
                 blk_nout=np.array(nout, dtype=np.int32), blk_idx=cat(bi, np.int32), blk_w=cat(bw, np.float64),
                 nchiv=np.array(nchiv, dtype=np.int64))
+
+
+def window_corrections(pdfs):
+    """Every window's svd correction for ``b200lm_window_propagate``: for each correlated block of each window's
+    whitening ``pdfs[w]`` (a ``PDF``), in the block order of ``window_weights``, the block of its corrected covariance
+    minus its input covariance, row-major n_in x n_in, concatenated.  None when no window has a correlated block or
+    when every correction is exactly zero."""
+    parts = [(cb - p.cov_in[np.ix_(b, b)]).reshape(-1) for p in pdfs for b, cb in p._corrected_blocks]
+    if not parts:
+        return None
+    d = np.ascontiguousarray(np.concatenate(parts), dtype=np.float64)
+    return d if d.any() else None
