@@ -77,6 +77,15 @@ int b200lm_load_functors(const char* path, int* family_out);
  * (src/lsqfit/_utilities.pyx:74-75): the mean vector then has ny entries, otherwise
  * N = ny + np entries (data means followed by prior means, :76-77). */
 int b200lm_create(int family, int ny, int np, int nx, int noprior, int device, b200lm_handle* out);
+/* A fit set: K independent problems of one functor and np stacked in one plan.  y(+)prior is the ny data rows of every
+ * problem, then nslot prior slots of np entries (N = ny + nslot np; N = ny with noprior).  b200lm_create is the
+ * nslot = 1 case.  ny, np > 0 and nslot >= 1, else EINVAL.  With nslot > 1 the plan fits through windows only, one
+ * per problem (b200lm_set_windows): each window lists its own data rows and every entry of exactly one slot, and
+ * a window over two slots, part of a slot or (with a prior) no slot is EINVAL with the window named.
+ * b200lm_set_weights, b200lm_fit_batch / _host before b200lm_set_windows, b200lm_residual_jacobian,
+ * b200lm_propagate and b200lm_window_propagate return EINVAL.
+ * (This declaration and WinDesc::pr_base change the headers digest: functor plug-ins must be rebuilt.) */
+int b200lm_create_set(int family, int ny, int np, int nx, int nslot, int noprior, int device, b200lm_handle* out);
 void b200lm_destroy(b200lm_handle h);
 
 /* model constants: the x array of flatfcn.keywords['x'] (src/lsqfit/__init__.py:1997-2012),

@@ -14,7 +14,7 @@ from .user_functor import cuda_functor, UserFunctor
 from .engine import Plan, BatchResult, STOPPING_CRITERION, normalize_tol
 from .whiten import PDF, cov_blocks
 from .fitter import b200_lm, ChivSpec, DeviceChiv
-from .fit import nonlinear_fit, gammaQ, BatchFits, FitView, wavg, WAvg
+from .fit import nonlinear_fit, gammaQ, BatchFits, FitView, wavg, WAvg, fit_set, FitSet
 from .dense import DenseFit
 from .bootstrap import bootstrap_means, normals
 from .multifit import MultiFitter, FunctorModel, SharedExpModel, ChainedFit

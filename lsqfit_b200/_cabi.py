@@ -39,6 +39,8 @@ SIGNATURES = {
     "b200lm_functor_family": (C.c_int, [C.c_char_p]),
     "b200lm_load_functors": (C.c_int, [C.c_char_p, c_int_p]),
     "b200lm_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(handle_t)]),
+    "b200lm_create_set": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                    C.POINTER(handle_t)]),
     "b200lm_destroy": (None, [handle_t]),
     "b200lm_set_const": (C.c_int, [handle_t, C.c_void_p, C.c_int]),
     "b200lm_set_weights": (C.c_int, [handle_t, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,

@@ -390,9 +390,16 @@ int b200lm_load_functors(const char* path, int* family_out) {
 }
 
 int b200lm_create(int family, int ny, int np, int nx, int noprior, int device, b200lm_handle* out) {
+    return b200lm_create_set(family, ny, np, nx, 1, noprior, device, out);
+}
+
+int b200lm_create_set(int family, int ny, int np, int nx, int nslot, int noprior, int device, b200lm_handle* out) {
     if (!out) return set_error(nullptr, B200LM_EINVAL, "out is NULL");
     *out = nullptr;
     if (ny <= 0 || np <= 0) return set_error(nullptr, B200LM_EINVAL, "ny and np must be positive");
+    if (nslot < 1) return set_error(nullptr, B200LM_EINVAL, "nslot must be positive");
+    if ((long long)ny + (noprior ? 0LL : (long long)nslot * np) > 0x7fffffffLL)
+        return set_error(nullptr, B200LM_EINVAL, "ny + nslot * np does not fit in an int");
     const FunctorEntry* fe = nullptr;
     {
         std::lock_guard<std::mutex> lock(g_registry_mu);
@@ -414,7 +421,8 @@ int b200lm_create(int family, int ny, int np, int nx, int noprior, int device, b
     CUDA_TRY(nullptr, cudaSetDevice(device), "cudaSetDevice");
     b200lm_handle_s* h = new b200lm_handle_s();
     h->device = device; h->fe = fe; h->ny = ny; h->np = np; h->nx = nx; h->noprior = noprior ? 1 : 0;
-    h->N = noprior ? ny : ny + np;
+    h->nslot = nslot;
+    h->N = noprior ? ny : ny + nslot * np;
     cudaDeviceProp prop;
     e = cudaGetDeviceProperties(&prop, device);
     if (e != cudaSuccess) { delete h; return cuda_fail(nullptr, e, "cudaGetDeviceProperties"); }
@@ -454,6 +462,9 @@ int b200lm_set_weights(b200lm_handle h, int ndiag, const int* diag_idx, const do
                        int nblk, const int* blk_nin, const int* blk_nout,
                        const int* blk_idx, const double* blk_w) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (h->nslot > 1)       // one whitening would reach every slot, and the kernel reads the prior as the first slot
+        return set_error(h, B200LM_EINVAL, "b200lm_set_weights is not built for fit sets (nslot > 1): "
+                                           "set one window per problem (b200lm_set_windows)");
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     WeightTables t;
     const std::string err = parse_weights(h, std::vector<char>(h->N, 2), ndiag, diag_idx, diag_w, nblk, blk_nin,
@@ -476,8 +487,9 @@ int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* d
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
     if (nwin < 1 || !ndiag || !nblk) return set_error(h, B200LM_EINVAL, "bad window description");
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
-    // a window lists every prior entry and its own data rows exactly once
-    std::vector<char> allowed(h->N, 2);
+    // a window lists every prior entry and its own data rows exactly once; in a fit set, every entry of one slot
+    // (checked below) and its own data rows
+    std::vector<char> allowed(h->N, h->nslot > 1 ? 1 : 2);
     for (int i = 0; i < h->ny; ++i) allowed[i] = 1;
     WeightTables all;
     std::vector<WinDesc> win(nwin);
@@ -494,7 +506,23 @@ int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* d
                                            where + (err == "size" ? "correlated block too large for the per-warp "
                                                                     "shared-memory plan" : err));
         if (t.ndata == 0) return set_error(h, B200LM_EINVAL, where + "no data row");
+        int pr_base = h->ny;
+        if (h->nslot > 1 && !h->noprior) {
+            int slot = -1, n = 0;
+            for (const std::vector<int>* v : {&t.pr_idx, &t.blk_idx})
+                for (int idx : *v) {
+                    if (idx < h->ny) continue;
+                    const int s = (idx - h->ny) / h->np;
+                    if (slot >= 0 && s != slot)
+                        return set_error(h, B200LM_EINVAL, where + "entries of two prior slots");
+                    slot = s; ++n;
+                }
+            if (slot < 0) return set_error(h, B200LM_EINVAL, where + "no prior slot");
+            if (n != h->np) return set_error(h, B200LM_EINVAL, where + "part of a prior slot");
+            pr_base = h->ny + slot * h->np;
+        }
         WinDesc& d = win[w];
+        d.pr_base = pr_base;
         d.nd_fn = (int)t.fn_idx.size(); d.nd_pr = (int)t.pr_idx.size(); d.nblk = nblk[w]; d.nchiv = t.nchiv;
         d.dfn_off = (int)all.fn_idx.size(); d.dpr_off = (int)all.pr_idx.size(); d.blk_off = (int)all.blk.size();
         all.append(t);
@@ -532,6 +560,9 @@ static int window_refusal(b200lm_handle h, int B) {
 
 static int check_ready(b200lm_handle h) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (h->nslot > 1 && h->nwin == 0)
+        return set_error(h, B200LM_EINVAL, "a fit set (nslot > 1) fits through windows: b200lm_set_windows has not "
+                                           "been called");
     if (!h->have_weights && h->nwin == 0) return set_error(h, B200LM_EINVAL, "b200lm_set_weights has not been called");
     if (!h->have_const) return set_error(h, B200LM_EINVAL, "b200lm_set_const has not been called");
     return B200LM_OK;
@@ -746,6 +777,7 @@ int b200lm_residual_jacobian(b200lm_handle h, int B, const double* d_p, long lon
     int rc = check_ready(h);
     if (rc) return rc;
     if (B < 0 || !d_p || !d_mean) return set_error(h, B200LM_EINVAL, "NULL required argument");
+    if (h->nslot > 1) return set_error(h, B200LM_EINVAL, "residual_jacobian is not built for fit sets");
     if (h->nwin > 0) return set_error(h, B200LM_EINVAL, "residual_jacobian is not built for window scans");
     if (B == 0) return B200LM_OK;
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");

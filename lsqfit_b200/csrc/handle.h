@@ -38,6 +38,9 @@ struct b200lm_handle_s {
     size_t smem_budget = 0;
     const b200lm::FunctorEntry* fe = nullptr;
     int ny = 0, np = 0, nx = 0, noprior = 0, N = 0, nchiv = 0;
+    // prior slots of np entries after the ny data rows (b200lm_create_set); a plan with nslot > 1 fits through windows,
+    // one slot per window
+    int nslot = 1;
     // device-resident problem description
     double* d_x = nullptr;
     b200lm::RowTables rows;     // the plan's whitening (b200lm_set_weights)

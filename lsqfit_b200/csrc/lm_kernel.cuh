@@ -296,6 +296,21 @@ __device__ __forceinline__ void consume_rows(WarpCtx<F>& c, int nrows, int slot0
 // returns cost.  Optionally writes the residual vector and J to global memory.
 // MODE 0: normal equations (A = J^T J, g = J^T r).  MODE 1: QR factor of J.diag(dsc) in c.A.
 // ---------------------------------------------------------------------------
+// the row tables of one window (P.win[w]), in the names eval_rows reads
+struct WinRows {
+    int nd_fn, nd_pr, nblk, pr_base;
+    const int* dfn_idx;
+    const double* dfn_w;
+    const int* dpr_idx;
+    const double* dpr_w;
+    const BlockDesc* blk;
+};
+
+// the entry of y(+)prior that holds prior entry 0 (parameter j sits at prior_base + j): the plan's one prior follows
+// its ny data rows; a window's is its own slot (every data row of a fit set precedes every slot)
+__device__ __forceinline__ int prior_base(const FitParams& P) { return P.ny; }
+__device__ __forceinline__ int prior_base(const WinRows& T) { return T.pr_base; }
+
 // T: the row tables (nd_fn, dfn_idx, dfn_w, nd_pr, dpr_idx, dpr_w, nblk, blk) -- the FitParams themselves, or those of
 // one window (WinRows)
 template <class F, int MODE, bool WSMEM, class RS>
@@ -313,7 +328,7 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
     // 1x1 prior rows: J row = w e_j, analytic contribution
     for (int i = lane; i < T.nd_pr; i += 32) {
         const int idx = T.dpr_idx[i];
-        const int j = idx - P.ny;
+        const int j = idx - prior_base(T);
         const double w = T.dpr_w[i];
         const double r = w * (pv[j] - c.mean[idx]);
         if (MODE == 0) {
@@ -377,7 +392,7 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
                         const double f = F::value_grad(P.x + (size_t)idx * P.nx, idx, pv, 1.0, row_);
                         dlt = f - c.mean[idx];
                     } else {
-                        const int j0 = idx - P.ny;
+                        const int j0 = idx - prior_base(T);
 #pragma unroll
                         for (int j = 0; j < NP; ++j) row_[j] = (j == j0) ? 1.0 : 0.0;
                         dlt = pv[j0] - c.mean[idx];
@@ -474,16 +489,6 @@ __device__ __forceinline__ double eval_full(WarpCtx<F>& c, const double* pv, dou
                           : eval_full_impl<F, MODE, false>(c, pv, fout, Jout);
 }
 
-// the row tables of one window (P.win[w]), in the names eval_rows reads
-struct WinRows {
-    int nd_fn, nd_pr, nblk;
-    const int* dfn_idx;
-    const double* dfn_w;
-    const int* dpr_idx;
-    const double* dpr_w;
-    const BlockDesc* blk;
-};
-
 // window evaluation: the weights stay in global memory (a scan's windows together are too large to stage, and the
 // fits of one window are contiguous in the batch, so the warps in flight share a few windows' weights in L2)
 template <class F, int MODE>
@@ -498,7 +503,7 @@ __device__ __noinline__ double eval_win_impl(const WarpCtx<F>& c_in, int w, cons
     const FitParams& P = c.P;
     const WinDesc wd = P.win[w];
     WinRows T;
-    T.nd_fn = wd.nd_fn; T.nd_pr = wd.nd_pr; T.nblk = wd.nblk;
+    T.nd_fn = wd.nd_fn; T.nd_pr = wd.nd_pr; T.nblk = wd.nblk; T.pr_base = wd.pr_base;
     T.dfn_idx = P.dfn_idx + wd.dfn_off; T.dfn_w = P.dfn_w + wd.dfn_off;
     T.dpr_idx = P.dpr_idx + wd.dpr_off; T.dpr_w = P.dpr_w + wd.dpr_off;
     T.blk = P.blk + wd.blk_off;

@@ -19,9 +19,12 @@ struct BlockDesc {
 
 // One window of a window scan (b200lm_set_windows): its part of the concatenated row tables of FitParams.
 // BlockDesc::idx_off and wt_off address the concatenated blk_idx / blk_wt, chiv_off the window's own residual vector.
+// pr_base: the first entry of the window's prior slot in y(+)prior (prior entry idx is parameter idx - pr_base): ny
+// for a window scan, ny + k np for problem k of a fit set (b200lm_create_set).
 struct WinDesc {
     int nd_fn, nd_pr, nblk, nchiv;
     int dfn_off, dpr_off, blk_off;
+    int pr_base;
 };
 
 // normal_diag_kernel (lm_rows.cuh): rows of the per-CTA partial buffer that b200lm_normal_diag allocates per SM

@@ -32,6 +32,7 @@ static cudaError_t scratch(b200lm_handle h, size_t need) {
 extern "C" int b200lm_propagate(b200lm_handle h, int B, const double* d_x, const double* d_cov,
                                 const double* d_C, double* d_D, double* d_covp, void* stream) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (h->nslot > 1) return set_error(h, B200LM_EINVAL, "propagate is not built for fit sets");
     if (!h->have_weights || !h->have_const) return set_error(h, B200LM_EINVAL, "plan is not complete");
     if (h->nwin > 0) return set_error(h, B200LM_EINVAL, "propagate is not built for window scans");
     if (B < 0 || !d_x || !d_cov || !d_D) return set_error(h, B200LM_EINVAL, "NULL required argument");
@@ -222,6 +223,8 @@ __global__ void __launch_bounds__(256) window_covp_finish_kernel(const __grid_co
 extern "C" int b200lm_window_propagate(b200lm_handle h, const double* d_cov, const double* d_J, const double* d_C,
                                        const double* d_dC, double* d_D, double* d_covp, void* stream) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    // the joint fit.p of the problems of a fit set (a covariance across problems) is not built
+    if (h->nslot > 1) return set_error(h, B200LM_EINVAL, "window_propagate is not built for fit sets");
     if (h->nwin == 0) return set_error(h, B200LM_EINVAL, "no windows set (b200lm_set_windows)");
     if (!d_cov || !d_J || !d_D) return set_error(h, B200LM_EINVAL, "NULL required argument");
     if (d_covp && !d_C) return set_error(h, B200LM_EINVAL, "d_C is required for cov(p)");

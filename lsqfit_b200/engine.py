@@ -49,21 +49,27 @@ class BatchResult(object):
 
 
 class Plan(object):
-    def __init__(self, functor, np_, ny, x, i_invwgts, noprior=False, device=0, team=None):
+    def __init__(self, functor, np_, ny, x, i_invwgts, noprior=False, device=0, team=None, nslot=1):
+        """nslot > 1: a fit set (b200lm_create_set) -- y (+) prior is ny data rows, then nslot prior slots of np
+        entries; ``i_invwgts`` must be None, and the plan fits once ``set_windows`` has given one window per problem."""
         if isinstance(functor, str):
             functor = Functor(functor)
         self.functor = functor
-        self.np, self.ny, self.noprior = int(np_), int(ny), bool(noprior)
-        self.N = self.ny if self.noprior else self.ny + self.np
+        self.np, self.ny, self.noprior, self.nslot = int(np_), int(ny), bool(noprior), int(nslot)
+        self.N = self.ny if self.noprior else self.ny + self.nslot * self.np
         self.device = int(device)
         self._h = _cabi.handle_t()
         if not torch.cuda.is_available():
             raise RuntimeError("lsqfit_b200: no CUDA device visible; this engine has no CPU fallback")
-        _cabi.check(_cabi.lib.b200lm_create(functor.family, self.ny, self.np, functor.nx,
-                                            1 if noprior else 0, self.device, C.byref(self._h)))
+        if self.nslot > 1 and i_invwgts is not None:
+            raise ValueError("a plan with nslot > 1 has no whitening of its own: pass i_invwgts=None, then set_windows")
+        _cabi.check(_cabi.lib.b200lm_create_set(functor.family, self.ny, self.np, functor.nx, self.nslot,
+                                                1 if noprior else 0, self.device, C.byref(self._h)))
         xr = functor.xrows(x, self.ny)
         _cabi.check(_cabi.lib.b200lm_set_const(self._h, xr.ctypes.data, xr.size), self._h)
-        self.set_weights(i_invwgts)
+        self.nchiv, self.nwin = 0, 0
+        if i_invwgts is not None:
+            self.set_weights(i_invwgts)
         self.tdev = torch.device("cuda", self.device)
         if team is not None:
             self.set_team(team)

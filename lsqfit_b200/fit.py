@@ -24,23 +24,17 @@ import time
 import numpy as np
 import torch
 
-from .engine import STOPPING_CRITERION, BatchResult
+from .engine import STOPPING_CRITERION, BatchResult, normalize_tol
 from .fitter import ChivSpec, DeviceChiv, b200_lm
 from .functors import Functor
 from .whiten import PDF
+from .windows import cov2 as _cov2, yp_cov as _yp_cov
 
 
 def gammaQ(a, x):
     """Q(a, x): the reference uses scipy.special.gammaincc too (src/lsqfit/_scipy.py:16-18)."""
     from scipy.special import gammaincc
     return gammaincc(a, x)
-
-
-def _cov2(c, n):
-    c = np.asarray(c, dtype=float)
-    if c.ndim == 0:
-        c = np.full(n, float(c))
-    return np.diag(c ** 2) if c.ndim == 1 else c
 
 
 def resolve_svdcut_eps(svdcut, eps):
@@ -126,16 +120,7 @@ class nonlinear_fit(object):
         # ---- whitening (device) : __init__.py:539-561 ------------------------------
         if _yp_pdf is None:
             if yp_cov is None:
-                yerr = np.asarray(yerr, dtype=float)
-                pdiag = noprior or np.count_nonzero(pcov - np.diag(np.diag(pcov))) == 0
-                if yerr.ndim <= 1 and pdiag:
-                    sd = np.full(ny, float(yerr)) if yerr.ndim == 0 else yerr
-                    yp_cov = sd if noprior else np.concatenate([sd, np.sqrt(np.diag(pcov))])
-                else:
-                    yp_cov = np.zeros((N, N))
-                    yp_cov[:ny, :ny] = _cov2(yerr, ny)
-                    if not noprior:
-                        yp_cov[ny:, ny:] = pcov
+                yp_cov = _yp_cov(yerr, pcov, ny)
             pdf = PDF(mean, yp_cov, svdcut=svdcut, eps=eps, device=self.device, noise=self.noise[0],
                       noise_seed=noise_seed)
             mean = pdf.mean                       # with the svd noise, if any (y.flat = yp_pdf.distribution, __init__.py:1896-1900)
@@ -392,15 +377,78 @@ class BatchFits(object):
 
 
 class _Window(object):
-    """What FitView and BatchFits read from the fit a result belongs to, for one window of a scan."""
+    """What FitView and BatchFits read from the fit a result belongs to, for one window of a scan or one problem of a
+    fit set."""
 
-    def __init__(self, parent, pdf, nchiv, np_):
-        self.prior, self.tol = parent.prior, parent.tol
+    def __init__(self, prior, tol, pdf, nchiv, np_):
+        self.prior, self.tol = prior, tol
         self.yp_pdf, self.svdn = pdf, pdf.nmod
         self.dof = int(nchiv) - int(np_)
 
 
-class WindowScan(object):
+def _whiten_each(parts, svdcut, eps, device):
+    """PDFs of many problems ``parts`` [(mean, covariance matrix or vector of standard deviations), ...], with the
+    correlated blocks of all of them whitened in ONE call (b200lm_whiten: one CTA per block, and a block's result
+    depends on that block alone -- each PDF is bit for bit that of a PDF of its problem by itself)."""
+    from .whiten import cov_blocks, whiten_blocks
+    covs = [np.asarray(c, dtype=float) for _, c in parts]
+    blocks = [cov_blocks(c)[1] if c.ndim == 2 else [] for c in covs]
+    ns = [b.size for bl in blocks for b in bl]
+    if ns:
+        flat = np.concatenate([c[np.ix_(b, b)].reshape(-1) for c, bl in zip(covs, blocks) for b in bl])
+        W, Cc, nout, nmod, ld = whiten_blocks(np.array(ns), flat, svdcut, eps, device)
+    pdfs = []
+    o = k = 0
+    for (mean, _), c, bl in zip(parts, covs, blocks):
+        nb, nel = len(bl), sum(b.size ** 2 for b in bl)
+        part = (W[o:o + nel], Cc[o:o + nel], nout[k:k + nb], nmod[k:k + nb], ld[k:k + nb]) if nb else None
+        pdfs.append(PDF(mean, c, svdcut=svdcut, eps=eps, device=device, _whitened=part))
+        o, k = o + nel, k + nb
+    return pdfs
+
+
+class _WindowFits(object):
+    """What a window scan and a fit set share: a plan whose windows are separate fits, each with its own rows,
+    whitening and start (b200lm_set_windows), the unpacking of its central batch into arrays over fits, and the
+    views of single fits.  Subclasses set ``np``, ``device``, ``args`` (the arguments of ``Plan.fit_batch``), ``p0``
+    and the mean vector ``_mean`` of the central fits, then call ``_setup``."""
+
+    def _setup(self, plan, sels, pdfs, prior_of, tol):
+        """plan: a plan without windows; sels[w] / pdfs[w]: window w's entries of the plan's y (+) prior vector and its
+        whitening; prior_of(w): the prior of window w's fit (None: no prior).  Fits the central batch."""
+        from .windows import window_weights
+        self.pdfs, self.sels = pdfs, sels
+        desc = window_weights(sels, [p.i_invwgts for p in pdfs])
+        self.nchiv = desc["nchiv"]
+        self.plan = plan
+        plan.set_windows(desc)
+        self.nwin = len(pdfs)
+        self.windows = [_Window(prior_of(w), tol, p, n, self.np) for w, (p, n) in enumerate(zip(pdfs, self.nchiv))]
+        self.dof = np.array([w.dof for w in self.windows])
+        self.svdn = np.array([w.svdn for w in self.windows])
+        out = self._fit(self._mean, self.p0, self.nwin)
+        a = out.numpy()
+        self.out, self._arrays = out, a
+        self.pmean, self.cov, self.chi2, self.nit = a["x"], a["cov"], a["chi2"], a["nit"]
+        self.psdev = np.sqrt(np.diagonal(self.cov, axis1=1, axis2=2))
+        self.Q = gammaQ(self.dof / 2., self.chi2 / 2.)
+        self.logGBF = (None if self.windows[0].prior is None else
+                       np.array([_logGBF(a["logdet"][w], p.logdet, a["chi2"][w], d)
+                                 for w, (p, d) in enumerate(zip(pdfs, self.dof))]))
+        self.stopping_criterion = np.array([STOPPING_CRITERION[int(s)] for s in a["status"]])
+        self.error = np.array([None if s > 0 else "b200_lm: no convergence" for s in a["status"]], dtype=object)
+
+    def _fit(self, means, p0, B, want_fJ=False):
+        return self.plan.fit_batch(means, p0, B=B, want_fJ=want_fJ, **self.args)
+
+    def __len__(self):
+        return self.nwin
+
+    def __getitem__(self, w):
+        return FitView(self.windows[w], self._arrays, w)
+
+
+class WindowScan(_WindowFits):
     """The central fits of a fit-window scan (``nonlinear_fit.window_fits``).
 
     Arrays over windows: ``pmean psdev`` [nwin, np], ``cov`` [nwin, np, np], ``chi2 dof Q logGBF svdn nit
@@ -416,8 +464,7 @@ class WindowScan(object):
 
     def __init__(self, parent, masks, p0=None, **kargs):
         from .engine import Plan
-        from .whiten import cov_blocks, whiten_blocks
-        from .windows import check_masks, window_cov, window_weights
+        from .windows import check_masks, window_cov
         # kernel= is ignored: window batches always run one warp per fit
         self.args, _, loss, gsl = parent._batch_args(kargs)
         refuse = lambda what: ValueError("b200_lm: %s not built for window scans" % what)
@@ -433,47 +480,15 @@ class WindowScan(object):
         self.parent, self.device = parent, parent.device
         self.np, self.ny = spec.np, spec.ny
         self.masks = check_masks(masks, self.ny)
-        self.nwin = self.masks.shape[0]
         pdf = parent.yp_pdf
         cov = pdf.cov_in if pdf.cov_in is not None else pdf.sdev_in
         wins = [window_cov(cov, self.ny, m) for m in self.masks]
-        # the correlated blocks of every window, whitened in ONE call (b200lm_whiten: one CTA per block, and a block's
-        # result depends on that block alone -- each window's whitening is bit for bit that of a PDF of its own)
-        blocks = [cov_blocks(c)[1] if c.ndim == 2 else [] for _, c in wins]
-        ns = [b.size for bl in blocks for b in bl]
-        if ns:
-            flat = np.concatenate([c[np.ix_(b, b)].reshape(-1) for (_, c), bl in zip(wins, blocks) for b in bl])
-            W, Cc, nout, nmod, ld = whiten_blocks(np.array(ns), flat, pdf.svdcut, pdf.eps, self.device)
-        self.pdfs = []
-        o = k = 0
-        for (sel, c), bl in zip(wins, blocks):
-            nb, nel = len(bl), sum(b.size ** 2 for b in bl)
-            part = (W[o:o + nel], Cc[o:o + nel], nout[k:k + nb], nmod[k:k + nb], ld[k:k + nb]) if nb else None
-            self.pdfs.append(PDF(pdf.mean[sel], c, svdcut=pdf.svdcut, eps=pdf.eps, device=self.device,
-                                 _whitened=part))
-            o, k = o + nel, k + nb
-        self.sels = [sel for sel, _ in wins]
-        desc = window_weights(self.sels, [p.i_invwgts for p in self.pdfs])
-        self.nchiv = desc["nchiv"]
-        self.plan = Plan(spec.functor, spec.np, spec.ny, spec.x, spec.i_invwgts, noprior=spec.noprior,
-                         device=self.device)
-        self.plan.set_windows(desc)
-        self.windows = [_Window(parent, p, n, self.np) for p, n in zip(self.pdfs, self.nchiv)]
-        self.dof = np.array([w.dof for w in self.windows])
-        self.svdn = np.array([w.svdn for w in self.windows])
+        pdfs = _whiten_each([(pdf.mean[sel], c) for sel, c in wins], pdf.svdcut, pdf.eps, self.device)
+        plan = Plan(spec.functor, spec.np, spec.ny, spec.x, spec.i_invwgts, noprior=spec.noprior, device=self.device)
         p0 = parent.pmean if p0 is None else np.asarray(p0, dtype=float)
-        self.p0 = np.array(np.broadcast_to(p0, (self.nwin, self.np)))
-        out = self._fit(spec.mean, self.p0, self.nwin)
-        a = out.numpy()
-        self.out, self._arrays = out, a
-        self.pmean, self.cov, self.chi2, self.nit = a["x"], a["cov"], a["chi2"], a["nit"]
-        self.psdev = np.sqrt(np.diagonal(self.cov, axis1=1, axis2=2))
-        self.Q = gammaQ(self.dof / 2., self.chi2 / 2.)
-        self.logGBF = (None if parent.prior is None else
-                       np.array([_logGBF(a["logdet"][w], p.logdet, a["chi2"][w], d)
-                                 for w, (p, d) in enumerate(zip(self.pdfs, self.dof))]))
-        self.stopping_criterion = np.array([STOPPING_CRITERION[int(s)] for s in a["status"]])
-        self.error = np.array([None if s > 0 else "b200_lm: no convergence" for s in a["status"]], dtype=object)
+        self.p0 = np.array(np.broadcast_to(p0, (len(wins), self.np)))
+        self._mean = spec.mean
+        self._setup(plan, [sel for sel, _ in wins], pdfs, lambda w: parent.prior, parent.tol)
         self._p = None
 
     def _getp(self):
@@ -502,15 +517,6 @@ class WindowScan(object):
         c = self._getp()[1].reshape(self.nwin * self.np, -1)
         return np.sqrt(np.diagonal(c)).reshape(self.nwin, self.np)
 
-    def _fit(self, means, p0, B, want_fJ=False):
-        return self.plan.fit_batch(means, p0, B=B, want_fJ=want_fJ, **self.args)
-
-    def __len__(self):
-        return self.nwin
-
-    def __getitem__(self, w):
-        return FitView(self.windows[w], self._arrays, w)
-
     def bootstrapped_fits(self, n=None, seed=None, means=None):
         """n bootstrap copies of every window in ONE launch (nwin * n fits).  The copies are the parent's
         ``bootstrap_means(n, seed)`` (or ``means`` [n, N]); every window of copy j reads its rows from the same row j,
@@ -521,11 +527,11 @@ class WindowScan(object):
         return WindowBootstrap(self, self._fit(means, self.pmean, self.nwin * n), n)
 
 
-class WindowBootstrap(object):
-    """The bootstrap copies of a window scan: fit b is copy b % n of window b // n."""
+class _Copies(object):
+    """The copies of every fit of a ``_WindowFits`` in one batch: fit b is copy b % n of fit b // n."""
 
-    def __init__(self, scan, out, n):
-        self.scan, self.out, self.n = scan, out, n
+    def __init__(self, fits, out, n):
+        self.fits, self.out, self.n = fits, out, n
 
     def __len__(self):
         return self.out.x.shape[0]
@@ -533,13 +539,156 @@ class WindowBootstrap(object):
     def arrays(self):
         return self.out.numpy()
 
-    def window(self, w):
-        """BatchFits of window w's copies (arrays(), iteration, pmean_stats())."""
+    def _part(self, w):
         s = slice(w * self.n, (w + 1) * self.n)
         o = self.out
         part = BatchResult(*[None if t is None else t[s] for t in (o.x, o.chi2, o.cov, o.logdet, o.nit, o.status,
                                                                     o.f, o.J)])
-        return BatchFits(self.scan.windows[w], part)
+        return BatchFits(self.fits.windows[w], part)
+
+
+class WindowBootstrap(_Copies):
+    """The bootstrap copies of a window scan: fit b is copy b % n of window b // n."""
+
+    @property
+    def scan(self):
+        return self.fits
+
+    def window(self, w):
+        """BatchFits of window w's copies (arrays(), iteration, pmean_stats())."""
+        return self._part(w)
+
+
+# functors whose parameters are indexed by the data row (xerr_logistic reads p[4 + row]): stacking renumbers rows
+_ROW_INDEXED = ("xerr_logistic",)
+_SET_ARGS = ("tol", "maxit", "scaler", "polish", "policy", "kernel", "device", "bounds", "loss", "noise", "yp_cov")
+
+
+class FitSet(_WindowFits):
+    """K independent fits of one model in one launch (``lsqfit_b200.fit_set``).
+
+    Problem k is ``nonlinear_fit(data=data[k], prior=prior[k], fcn=fcn, p0=p0[k], svdcut=svdcut, eps=eps,
+    **fitterargs)``: its own x grid, data, covariance and prior, whitened on its own.  Arrays over problems:
+    ``pmean psdev`` [K, np], ``cov`` [K, np, np], ``chi2 dof Q logGBF svdn nit stopping_criterion error`` [K];
+    ``fs[k]`` has the attribute names of ``nonlinear_fit``; ``pdfs[k]`` is problem k's whitening.  The plan holds every
+    problem's data rows, then one prior slot of np entries per problem (b200lm_create_set), and fits problem k as
+    window k with its slot as prior."""
+
+    def __init__(self, data, prior=None, fcn=None, p0=None, svdcut=False, eps=False, tol=1e-8, maxit=1000,
+                 **fitterargs):
+        from .engine import POLICY, Plan
+        from .windows import set_description
+        refuse = lambda what: ValueError("b200_lm: %s not built for fit sets" % what)
+        unknown = sorted(set(fitterargs) - set(_SET_ARGS))
+        if unknown:
+            raise ValueError("fit_set: unknown fitter arguments: " + ", ".join(unknown))
+        if fitterargs.get("bounds") is not None:
+            raise refuse("bounds are")
+        if fitterargs.get("loss", "linear") != "linear":
+            raise refuse("a robust loss is")
+        if POLICY.get(fitterargs.get("policy", "trf")) != 0:
+            raise refuse("policy=%r is" % (fitterargs.get("policy"),))
+        if fitterargs.get("noise"):
+            raise refuse("noise is")
+        if fitterargs.get("yp_cov") is not None:
+            raise refuse("yp_cov (data-prior correlations) is")
+        if isinstance(fcn, str):
+            fcn = Functor(fcn)
+        if not isinstance(fcn, Functor):
+            raise ValueError("fcn must be a lsqfit_b200.Functor (device model registry)")
+        if fcn.name in _ROW_INDEXED:
+            raise refuse("a functor whose parameters are indexed by the data row (%s) is" % fcn.name)
+        svdcut, eps = resolve_svdcut_eps(svdcut, eps)
+        d = set_description(data, prior, fcn)
+        self.fcn, self.device = fcn, int(fitterargs.get("device", 0))
+        self.K, self.ny, self.N, self.noprior = len(d["sels"]), d["ny"], d["N"], d["noprior"]
+        self.description = d
+        # p0 per problem: [np] shared, [K, np], or (with a prior) nonlinear_fit's default from each prior
+        if p0 is None:
+            if self.noprior:
+                raise ValueError("need p0 if there is no prior")
+            p0 = np.array([np.where(m != 0.0, m, m + 0.1 * np.sqrt(np.diag(c)))
+                           for m, c in zip(d["pmeans"], d["pcovs"])])
+        p0 = np.array(p0, dtype=float)
+        npar = p0.shape[-1] if self.noprior else d["np"]
+        if p0.ndim not in (1, 2) or p0.shape[-1] != npar or (p0.ndim == 2 and p0.shape[0] != self.K):
+            raise refuse("p0 of shape %s for %d problems of np = %d is" % (p0.shape, self.K, npar))
+        self.np = npar
+        self._spec = ChivSpec(fcn, d["x"], None, self.noprior, self.ny, npar)
+        self.p0 = np.array(np.broadcast_to(p0, (self.K, npar)))
+        self.svdcut, self.eps, self.tol, self.maxit = svdcut, eps, normalize_tol(tol), maxit
+        self.args = dict(tol=self.tol, maxit=maxit, scaler=fitterargs.get("scaler", "more"),
+                         polish=fitterargs.get("polish", 0))
+        self.prior = None if self.noprior else list(zip(d["pmeans"], d["pcovs"]))
+        pdfs = _whiten_each(list(zip(d["means"], d["covs"])), svdcut, eps, self.device)
+        plan = Plan(fcn, npar, self.ny, d["x"], None, noprior=self.noprior, device=self.device, nslot=self.K)
+        self._mean = d["mean"]
+        self.p0 = self._spec.to_device(self.p0)
+        self._setup(plan, d["sels"], pdfs, lambda k: None if self.noprior else self.prior[k], self.tol)
+        self.pmean, self.cov = self._spec.from_device(self.pmean, self.cov)[:2]
+        self._L = [None] * self.K
+        self.seeds = None
+
+    def bootstrap_means(self, n, seed=None, seeds=None):
+        """[n, N] device tensor: copy j of every problem's y (+) prior means in one row; problem k's columns (its data
+        rows and its prior slot) are copy j of its own ``bootstrap_means(n, seeds[k])`` stream, bit for bit.  ``seeds``
+        [K] defaults to ``np.random.SeedSequence(seed).generate_state(K, np.uint64)`` (``seed`` None: a fresh one);
+        ``self.seeds`` keeps the seeds used.  Memory: n N doubles (256 problems of 80 entries, 1000 copies: 164 MB)."""
+        from .bootstrap import bootstrap_means_into
+        if n is None:
+            raise ValueError("n=None is not supported: a batch is one launch; pass the number of copies")
+        if seeds is None:
+            seed = fresh_seed() if seed is None else int(seed)
+            seeds = np.random.SeedSequence(seed).generate_state(self.K, np.uint64)
+        seeds = [int(s) for s in np.asarray(seeds, dtype=np.uint64).reshape(-1)]
+        if len(seeds) != self.K:
+            raise ValueError("seeds: one per problem (%d), got %d" % (self.K, len(seeds)))
+        self.seeds = seeds
+        n = int(n)
+        out = torch.empty((n, self.N), dtype=torch.float64, device=torch.device("cuda", self.device))
+        d = self.description
+        for k, (pdf, sel) in enumerate(zip(self.pdfs, self.sels)):
+            if self._L[k] is None:
+                self._L[k] = pdf.sqrt_cov()
+            L, nyk = self._L[k], int(d["nys"][k])
+            # the data rows and the slot are two column ranges of the stacked vector: the copies of each, from the
+            # same normals (the same seed and M), are the rows of the problem's own L z
+            bootstrap_means_into(out, int(sel[0]), pdf.mean[:nyk], L[:nyk], n, seeds[k], device=self.device)
+            if nyk < sel.size:
+                bootstrap_means_into(out, int(sel[nyk]), pdf.mean[nyk:], L[nyk:], n, seeds[k], device=self.device)
+        return out
+
+    def bootstrapped_fits(self, n=None, seed=None, seeds=None, means=None):
+        """n bootstrap copies of every problem in ONE launch (K * n fits): fit b is copy b % n of problem b // n, started
+        from that problem's central ``pmean``.  Problem k's copies are its own bootstrap stream (``bootstrap_means``;
+        lsqfit's semantics for separate fits), or rows of ``means`` [n, N] in the stacked layout."""
+        if means is None:
+            means = self.bootstrap_means(n, seed, seeds)
+        n = int(means.shape[0])
+        return SetBootstrap(self, self._fit(means, self._spec.to_device(self.pmean), self.K * n), n)
+
+
+class SetBootstrap(_Copies):
+    """The bootstrap copies of a fit set: fit b is copy b % n of problem b // n."""
+
+    def problem(self, k):
+        """BatchFits of problem k's copies (arrays(), iteration, pmean_stats())."""
+        return self._part(k)
+
+
+def fit_set(data, prior=None, fcn=None, p0=None, svdcut=False, eps=False, tol=1e-8, maxit=1000, **fitterargs):
+    """Fit K independent problems of one model in ONE launch, and their bootstrap copies in one more.
+
+    ``data``: a list of K data sets in the forms ``nonlinear_fit`` accepts ((x, y, ycov | ysdev) or (y, ycov | ysdev));
+    ``ny`` and the x grid may differ between problems.  ``prior``: a list of K priors (pmean, pcov | psdev), one prior
+    shared by all, or None (then ``p0`` is required).  ``p0``: None, [np] or [K, np].  Problem k is exactly
+    ``nonlinear_fit(data=data[k], prior=prior[k], fcn=fcn, p0=p0[k], svdcut=svdcut, eps=eps, **fitterargs)``; the
+    problems are independent (the stacked covariance is block diagonal).  Fitter arguments: ``tol``, ``maxit``,
+    ``scaler``, ``polish``, ``device``; ``kernel=`` is accepted and ignored (sets run one warp per fit).  ``bounds``, a
+    robust ``loss``, ``policy='gsl'``, ``noise``, ``yp_cov``, priors for some problems only, an empty list, priors of
+    different sizes and functors that index parameters by data row are refused ("not built for fit sets").
+    Returns a ``FitSet``."""
+    return FitSet(data, prior, fcn, p0, svdcut, eps, tol, maxit, **fitterargs)
 
 
 class WAvg(object):

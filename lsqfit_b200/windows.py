@@ -1,4 +1,4 @@
-"""Fit-window scans: the problem description of many data windows of one fit (pure numpy, no device).
+"""Fit-window scans and fit sets: the problem description of many fits in one plan (pure numpy, no device).
 
 A window is a boolean mask over the parent fit's ``ny`` data rows.  Window ``w`` is the fit of the rows
 ``m = masks[w]`` with the parent's prior: its y (+) prior vector is ``sel = rows(m) ++ prior``, and its covariance
@@ -6,8 +6,38 @@ is the parent's input covariance restricted to ``sel``.  Whitening that sub-matr
 ``i_invwgts`` (indices into the window's own y (+) prior vector); ``window_weights`` renumbers them to indices
 of the parent's FULL y (+) prior vector and concatenates the windows in the layout of ``b200lm_set_windows``.
 The device then reads every window's rows from the same full-length mean vector of a bootstrap copy.
+
+A fit set (``set_description``) stacks K unrelated problems of one model the same way: the stacked y (+) prior
+vector is every problem's data rows, problem after problem, then one prior slot of np entries per problem
+(``b200lm_create_set``).  Problem k is the window ``sel_k = rows_k ++ slot_k`` of that vector.
 """
 import numpy as np
+
+
+def cov2(c, n):
+    """A covariance matrix from a covariance matrix, a vector of n standard deviations or one shared one."""
+    c = np.asarray(c, dtype=float)
+    if c.ndim == 0:
+        c = np.full(n, float(c))
+    return np.diag(c ** 2) if c.ndim == 1 else c
+
+
+def yp_cov(yerr, pcov, ny):
+    """The covariance of y (+) prior that ``nonlinear_fit`` whitens, from the data's ``yerr`` (covariance matrix, vector
+    of standard deviations or one shared one) and the prior covariance ``pcov`` (matrix; None: no prior): the vector of
+    standard deviations when both are diagonal, else the block-diagonal matrix."""
+    yerr = np.asarray(yerr, dtype=float)
+    noprior = pcov is None
+    pdiag = noprior or np.count_nonzero(pcov - np.diag(np.diag(pcov))) == 0
+    if yerr.ndim <= 1 and pdiag:
+        sd = np.full(ny, float(yerr)) if yerr.ndim == 0 else yerr
+        return sd if noprior else np.concatenate([sd, np.sqrt(np.diag(pcov))])
+    N = ny if noprior else ny + pcov.shape[0]
+    c = np.zeros((N, N))
+    c[:ny, :ny] = cov2(yerr, ny)
+    if not noprior:
+        c[ny:, ny:] = pcov
+    return c
 
 
 def check_masks(masks, ny):
@@ -81,3 +111,77 @@ def window_corrections(pdfs):
         return None
     d = np.ascontiguousarray(np.concatenate(parts), dtype=np.float64)
     return d if d.any() else None
+
+
+def _is_pair(prior):
+    """True for one prior (pmean, pcov | psdev), False for a sequence of them."""
+    if not isinstance(prior, tuple) or len(prior) != 2:
+        return False
+    try:
+        return np.ndim(np.asarray(prior[0], dtype=float)) == 1
+    except (TypeError, ValueError):
+        return False
+
+
+def set_description(data, prior, fcn):
+    """The stacked problem of a fit set (``lsqfit_b200.fit_set``).
+
+    data: a list of K data sets, each in a form ``nonlinear_fit`` accepts, (x, ymean, yerr) or (ymean, yerr); prior: a
+    list of K priors (pmean, pcov | psdev), one prior shared by every problem, or None (no prior); fcn: the Functor.
+    Returns a dict with ``x`` [ny, nx] (every problem's x rows, stacked as fcn.xrows reads them), ``mean`` [N] (the
+    stacked y (+) prior means), ``ny`` (all data rows), ``N``, ``np``, ``noprior``, and per problem: ``nys``,
+    ``row_off`` (first data row), ``sels`` (its y (+) prior entries in the stacked vector, in its own order: data rows,
+    then its slot ``ny + k np ...``), ``means`` and ``covs`` (its own y (+) prior means and the covariance
+    ``nonlinear_fit`` would whiten), ``pmeans`` and ``pcovs`` (None without a prior).  ValueError for an empty list,
+    a mix of problems with and without a prior, and priors of different sizes."""
+    refuse = lambda what: ValueError("%s not built for fit sets" % what)
+    if not isinstance(data, (list, tuple)) or len(data) == 0:
+        raise refuse("an empty list of problems is")
+    K = len(data)
+    if prior is None or _is_pair(prior):
+        priors = [prior] * K
+    else:
+        priors = list(prior)
+        if len(priors) != K:
+            raise ValueError("%d priors for %d problems: priors of that number are not built for fit sets"
+                             % (len(priors), K))
+    noprior = priors[0] is None
+    if any((p is None) != noprior for p in priors):
+        raise refuse("a mix of problems with and without a prior is")
+    xs, ys, yerrs = [], [], []
+    for k, d in enumerate(data):
+        if not isinstance(d, tuple) or len(d) not in (2, 3):
+            raise ValueError("problem %d: data tuple wrong length" % k)
+        x, ymean, yerr = d if len(d) == 3 else (False,) + tuple(d)
+        ymean = np.array(ymean, dtype=float).reshape(-1)
+        xs.append(fcn.xrows(x, ymean.size))
+        ys.append(ymean)
+        yerrs.append(yerr)
+    nys = np.array([y.size for y in ys], dtype=np.int64)
+    ny = int(nys.sum())
+    row_off = np.concatenate([[0], np.cumsum(nys)[:-1]]).astype(np.int64)
+    pmeans = pcovs = None
+    if noprior:
+        npar = -1
+    else:
+        pmeans = [np.array(p[0], dtype=float).reshape(-1) for p in priors]
+        npar = pmeans[0].size
+        if any(m.size != npar for m in pmeans):
+            raise refuse("priors of different sizes (np %s) are" % sorted(set(m.size for m in pmeans)))
+        pcovs = [cov2(p[1], npar) for p in priors]
+    N = ny if noprior else ny + K * npar
+    sels, means, covs = [], [], []
+    for k in range(K):
+        rows = np.arange(row_off[k], row_off[k] + nys[k])
+        if noprior:
+            sels.append(rows.astype(np.intp))
+            means.append(ys[k])
+        else:
+            sels.append(np.concatenate([rows, ny + k * npar + np.arange(npar)]).astype(np.intp))
+            means.append(np.concatenate([ys[k], pmeans[k]]))
+        covs.append(yp_cov(yerrs[k], None if noprior else pcovs[k], int(nys[k])))
+    mean = np.zeros(N)
+    for sel, m in zip(sels, means):
+        mean[sel] = m
+    return dict(x=np.ascontiguousarray(np.concatenate(xs)), mean=mean, ny=ny, N=N, np=npar, noprior=noprior,
+                nys=nys, row_off=row_off, sels=sels, means=means, covs=covs, pmeans=pmeans, pcovs=pcovs)
