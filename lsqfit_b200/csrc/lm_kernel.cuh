@@ -115,6 +115,12 @@ struct WarpCtx {
     double *Abuf[2], *gbuf[2];      // c.A / c.g point at the buffer the next evaluation writes
     int lane;
     __device__ WarpCtx(const FitParams& P_) : P(P_) {}
+    // select buffer k (0 or 1) without indexing Abuf / gbuf at run time: a dynamic index would keep the whole
+    // context in local memory
+    __device__ __forceinline__ void use_buf(int k) {
+        A = k ? Abuf[1] : Abuf[0];
+        g = k ? gbuf[1] : gbuf[0];
+    }
 };
 
 // D(8x8) += A(8x4) . B(4x8) on the FP64 tensor path.  Fragment ownership (PTX m8n8k4):
@@ -233,13 +239,12 @@ __device__ __forceinline__ void emit_rows(const double* S, int nrows, int slot0,
 // S is destroyed.  Used for the final covariance: (J^T J)^-1 = dsc Rt^-1 Rt^-T dsc has a
 // relative error ~kappa(J)*eps instead of kappa^2*eps for the normal equations.
 template <class F>
-__device__ __forceinline__ void qr_update(WarpCtx<F>& c, double* S, int nrows) {
+__device__ __forceinline__ void qr_update(double* A, const double* dsc, double* S, int nrows, int lane) {
     typedef FitLayout<F> Lay;
     constexpr int NP = Lay::NP, LDR = Lay::LDR, LDA = Lay::LDA;
-    const int lane = c.lane;
     for (int i = lane; i < nrows; i += 32) {
 #pragma unroll
-        for (int j = 0; j < NP; ++j) S[i * LDR + j] *= c.dsc[j];
+        for (int j = 0; j < NP; ++j) S[i * LDR + j] *= dsc[j];
     }
     __syncwarp();
     for (int j = 0; j < NP; ++j) {
@@ -247,7 +252,7 @@ __device__ __forceinline__ void qr_update(WarpCtx<F>& c, double* S, int nrows) {
         for (int i = lane; i < nrows; i += 32) { const double v = S[i * LDR + j]; ss = fma(v, v, ss); }
         ss = warp_sum(ss);
         if (ss == 0.0) continue;                             // uniform across the warp
-        const double rjj = c.A[j * LDA + j];
+        const double rjj = A[j * LDA + j];
         const double nrm = sqrt(fma(rjj, rjj, ss));
         const double alpha = rjj > 0.0 ? -nrm : nrm;
         const double v0 = rjj - alpha;
@@ -261,7 +266,7 @@ __device__ __forceinline__ void qr_update(WarpCtx<F>& c, double* S, int nrows) {
             for (int q = 0; q < NP; ++q) if (q > j) t[q] = fma(sj, S[i * LDR + q], t[q]);
         }
 #pragma unroll
-        for (int q = 0; q < NP; ++q) if (q > j) t[q] = (fma(v0, c.A[j * LDA + q], warp_sum(t[q]))) * beta;
+        for (int q = 0; q < NP; ++q) if (q > j) t[q] = (fma(v0, A[j * LDA + q], warp_sum(t[q]))) * beta;
         __syncwarp();
         for (int i = lane; i < nrows; i += 32) {
             const double sj = S[i * LDR + j];
@@ -270,8 +275,8 @@ __device__ __forceinline__ void qr_update(WarpCtx<F>& c, double* S, int nrows) {
         }
         if (lane == 0) {
 #pragma unroll
-            for (int q = 0; q < NP; ++q) if (q > j) c.A[j * LDA + q] = fma(-t[q], v0, c.A[j * LDA + q]);
-            c.A[j * LDA + j] = alpha;
+            for (int q = 0; q < NP; ++q) if (q > j) A[j * LDA + q] = fma(-t[q], v0, A[j * LDA + q]);
+            A[j * LDA + j] = alpha;
         }
         __syncwarp();
     }
@@ -286,7 +291,7 @@ __device__ __forceinline__ void consume_rows(WarpCtx<F>& c, int nrows, int slot0
         mma_accumulate<F>(c, c.R, (nrows + 3) & ~3, na);
     } else {
         __syncwarp();
-        qr_update<F>(c, c.R, nrows);
+        qr_update<F>(c.A, c.dsc, c.R, nrows, c.lane);
     }
     __syncwarp();
 }
@@ -1283,7 +1288,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
         __syncwarp();
 
         int cur = 0;                              // buffer holding J^T J, J^T r of the current point
-        c.A = c.Abuf[0]; c.g = c.gbuf[0];
+        c.use_buf(0);
         const long long t_fit0 = B200LM_CLOCK();
         double cost = 0.0;
         bool have_A = false;
@@ -1375,11 +1380,11 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
                         // quadratic_preduction * |f|^2 / 2 = -(1/2 dx^T A dx + g^T dx)
                         const double predicted = warp_sum(act ? -step * (0.5 * As + gi) : 0.0);
                         __syncwarp();
-                        c.A = c.Abuf[cur ^ 1]; c.g = c.gbuf[cur ^ 1];
+                        c.use_buf(cur ^ 1);
                         const long long t_e0 = B200LM_CLOCK();
                         cost_new = ev.run(c, c.pn, nullptr, nullptr, 0);
                         pk.eval += B200LM_CLOCK() - t_e0;
-                        c.A = c.Abuf[cur]; c.g = c.gbuf[cur];
+                        c.use_buf(cur);
                         ++nfev; ++njev;
                         // trust_calc_rho: |f_trial| >= |f| (or NaN) rejects; rho = (1 - u^2) / pred
                         if (cost_new < cost && predicted > 0.0) rho = (cost - cost_new) / predicted;
@@ -1387,7 +1392,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
                     if (rho > 0.0) {
                         if (act) c.p[lane] = c.pn[lane];
                         cur ^= 1;
-                        c.A = c.Abuf[cur]; c.g = c.gbuf[cur];
+                        c.use_buf(cur);
                         cost = cost_new;
                         __syncwarp();
                         if (P.scaler != 0) {
@@ -1509,11 +1514,11 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
                 // point, into the other buffer.  ~87 % of the trials are accepted, and then no
                 // second pass over the rows is needed; a rejected trial leaves the current
                 // buffers untouched.
-                c.A = c.Abuf[cur ^ 1]; c.g = c.gbuf[cur ^ 1];
+                c.use_buf(cur ^ 1);
                 const long long t_e0 = B200LM_CLOCK();
                 cost_new = ev.run(c, c.pn, nullptr, nullptr, 0);
                 pk.eval += B200LM_CLOCK() - t_e0;
-                c.A = c.Abuf[cur]; c.g = c.gbuf[cur];
+                c.use_buf(cur);
                 ++nfev; ++njev;
                 if (!isfinite(cost_new)) { Delta = 0.25 * sqrt(sh2); continue; }
                 actual_reduction = cost - cost_new;
@@ -1545,7 +1550,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
                 // accept: the trial buffers become the current ones
                 if (act) c.p[lane] = c.pn[lane];
                 cur ^= 1;
-                c.A = c.Abuf[cur]; c.g = c.gbuf[cur];
+                c.use_buf(cur);
                 cost = cost_new;
                 __syncwarp();
                 if (act && P.scaler == 1) sinv = fmax(sinv, sqrt(c.A[lane * LDA + lane]));

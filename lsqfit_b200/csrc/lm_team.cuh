@@ -26,9 +26,6 @@
 #ifndef B200LM_P2_PIPE
 #define B200LM_P2_PIPE 1
 #endif
-#ifndef B200LM_EVAL_BYREF
-#define B200LM_EVAL_BYREF 0
-#endif
 
 namespace b200lm {
 
@@ -134,13 +131,13 @@ __device__ __forceinline__ void team_pointers(TeamCtx<F, TW>& tc, const FitParam
     c.mean = tc.mean_s;
 }
 
+__device__ __forceinline__ double* shared_ptr(unsigned s) { return reinterpret_cast<double*>(__cvta_shared_to_generic(s)); }
+__device__ __forceinline__ unsigned shared_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
+
+// the operands arrive as shared-memory addresses: a context passed by reference would have to sit in local memory
 template <class F>
-__device__ __noinline__ void qr_update_rows(const WarpCtx<F>& c_in, double* S, int nrows) {
-    WarpCtx<F> c = c_in;
-    __builtin_assume(__isShared(S));
-    __builtin_assume(__isShared(c.A));
-    __builtin_assume(__isShared(c.dsc));
-    qr_update<F>(c, S, nrows);
+__device__ __noinline__ void qr_update_rows(unsigned A_s, unsigned dsc_s, unsigned S_s, int nrows, int lane) {
+    qr_update<F>(shared_ptr(A_s), shared_ptr(dsc_s), shared_ptr(S_s), nrows, lane);
 }
 
 // partial normal equations of one warp in DMMA C-fragment layout
@@ -235,52 +232,26 @@ __device__ __forceinline__ double team_flush(WarpCtx<F>& c, TeamAcc<F, TW>& na) 
 // A = J^T J, g = J^T r in c.A / c.g and the cost as return value.  mode 1: the leader instead folds
 // all rows into the Householder factor of J.diag(dsc) (final covariance of ill-conditioned fits).
 template <class F, int TW, bool STAGED>
-#if B200LM_EVAL_BYREF
-__device__ __noinline__ double team_eval_impl(const TeamCtx<F, TW>& tc_in, int flags, double* fout, double* Jout) {
-#else
 __device__ __noinline__ double team_eval_impl(const FitParams& P, unsigned base_s, unsigned stage_s, int ids, int flags,
                                               double* fout, double* Jout) {
     // the context arrives as two shared-memory OFFSETS: every pointer is rebuilt from them (constants and
     // kernel parameters only), so nothing is copied through local memory and the compiler knows the
     // address space of everything it derives (LDS/STS without __builtin_assume)
-    double* base = reinterpret_cast<double*>(__cvta_shared_to_generic(base_s));
-    const double* stage = reinterpret_cast<const double*>(__cvta_shared_to_generic(stage_s));
-#endif
+    double* base = shared_ptr(base_s);
+    const double* stage = shared_ptr(stage_s);
     typedef FitLayout<F> Lay;
     typedef TeamLayout<F, TW> TL;
     constexpr int NP = Lay::NP, NT = Lay::NT, LDR = Lay::LDR, LDA = Lay::LDA, NCOL = Lay::NCOL;
     constexpr int CH = TL::CH, MT = TL::MT, RW = TL::RW, LDT = TL::LDT, TROWS = TL::TROWS, LPR = TL::LPR;
     // ids = lane | tw << 8 | bar << 16 ;  flags = mode | pv_sel << 1 | cur << 2
-#if B200LM_EVAL_BYREF
-    TeamCtx<F, TW> tc = tc_in;
-    WarpCtx<F>& c = tc.c;
-    const FitParams& P = c.P;
-#else
     TeamCtx<F, TW> tc(P);
     WarpCtx<F>& c = tc.c;
     team_pointers<F, TW>(tc, P, base, stage);
     c.lane = ids & 31; tc.tw = (ids >> 8) & 7; tc.bar = ids >> 16;
-#endif
-    const int mode = flags & 1, cur_ = (flags >> 2) & 1;
-    c.A = c.Abuf[cur_]; c.g = c.gbuf[cur_];
+    const int mode = flags & 1;
+    c.use_buf((flags >> 2) & 1);
     const double* pv = (flags & 2) ? c.pn : c.p;
     const int lane = c.lane, tw = tc.tw, bar = tc.bar;
-#if B200LM_EVAL_BYREF
-    __builtin_assume(__isShared(c.R));
-    __builtin_assume(__isShared(c.A));
-    __builtin_assume(__isShared(c.g));
-    __builtin_assume(__isShared(c.dsc));
-    __builtin_assume(__isShared(pv));
-    __builtin_assume(__isShared(c.mean));
-    if constexpr (STAGED) {
-        __builtin_assume(__isShared(tc.xs));
-        __builtin_assume(__isShared(tc.fw));
-        __builtin_assume(__isShared(tc.pw));
-        __builtin_assume(__isShared(tc.bidx));
-        __builtin_assume(__isShared(tc.fidx));
-        __builtin_assume(__isShared(tc.pidx));
-    }
-#endif
     double* Jb = c.R;                       // row-major view  [CH][LDR]  of finished rows [J | r]
     double* T = c.R;                        // transposed view [TROWS][LDT] of a chunk of [G | delta]
     double* Jown = Jb + tw * RW * LDR;      // the rows this warp owns
@@ -357,7 +328,7 @@ __device__ __noinline__ double team_eval_impl(const FitParams& P, unsigned base_
                 const int nall = min(CH, P.nd_fn - c0);
                 if (fout || Jout) emit_rows<F>(Jb, nall, c0, lane, fout, Jout);
                 __syncwarp();
-                qr_update_rows<F>(c, Jb, nall);
+                qr_update_rows<F>(shared_addr(c.A), shared_addr(c.dsc), shared_addr(Jb), nall, lane);
             }
             dirty = true;
         }
@@ -369,9 +340,6 @@ __device__ __noinline__ double team_eval_impl(const FitParams& P, unsigned base_
     for (int b = 0; b < P.nblk; ++b) {
         const BlockDesc bd = P.blk[b];
         const double* W = c.wt + bd.wt2_off;
-#if B200LM_EVAL_BYREF
-        if constexpr (STAGED) __builtin_assume(__isShared(W));
-#endif
         const int ldw = bd.ldw2;
         for (int g0 = 0; g0 < bd.n_out; g0 += CH) {
             double pc[MT][NT][2];
@@ -521,7 +489,7 @@ __device__ __noinline__ double team_eval_impl(const FitParams& P, unsigned base_
                     const int nall = min(CH, bd.n_out - g0);
                     if (fout || Jout) emit_rows<F>(Jb, nall, bd.chiv_off + g0, lane, fout, Jout);
                     __syncwarp();
-                    qr_update_rows<F>(c, Jb, nall);
+                    qr_update_rows<F>(shared_addr(c.A), shared_addr(c.dsc), shared_addr(Jb), nall, lane);
                 }
             }
             dirty = true;
@@ -608,48 +576,45 @@ __device__ __noinline__ double team_eval_impl(const FitParams& P, unsigned base_
 }
 
 template <class F, int TW>
-__device__ __forceinline__ double team_eval(const TeamCtx<F, TW>& tc, const double* pv, int mode,
+__device__ __forceinline__ double team_eval(const WarpCtx<F>& c, int tw, int bar, const double* pv, int mode,
                                             double* fout, double* Jout) {
-    const WarpCtx<F>& c = tc.c;
-    const int ids = c.lane | (tc.tw << 8) | (tc.bar << 16);
+    const int ids = c.lane | (tw << 8) | (bar << 16);
     const int flags = (mode & 1) | ((pv == c.pn) ? 2 : 0) | ((c.A == c.Abuf[1]) ? 4 : 0);
-#if B200LM_EVAL_BYREF
-    (void)ids;
-    return c.P.staged ? team_eval_impl<F, TW, true>(tc, flags, fout, Jout)
-                      : team_eval_impl<F, TW, false>(tc, flags, fout, Jout);
-#else
-    const unsigned base_s = (unsigned)__cvta_generic_to_shared(c.R);
-    const unsigned stage_s = c.P.staged ? (unsigned)__cvta_generic_to_shared(c.wt) : 0u;
+    const unsigned base_s = shared_addr(c.R);
+    const unsigned stage_s = c.P.staged ? shared_addr(c.wt) : 0u;
     return c.P.staged ? team_eval_impl<F, TW, true>(c.P, base_s, stage_s, ids, flags, fout, Jout)
                       : team_eval_impl<F, TW, false>(c.P, base_s, stage_s, ids, flags, fout, Jout);
-#endif
 }
 
-// leader side of fit_one's evaluator: post the command, then take part in the evaluation
+// leader side of fit_one's evaluator: post the command, then take part in the evaluation.  It holds the
+// team's command block, means and barrier by value: a pointer to the team context would keep that
+// context, and every pointer of the leader's WarpCtx, in local memory.
 template <class F, int TW>
 struct TeamEval {
-    TeamCtx<F, TW>* tc;
+    int* cmd;
+    double* mean_s;
+    int bar;
     int b;
     // stage the means of fit b in the team's shared memory (read by every warp of the team)
     __device__ __forceinline__ const double* begin(WarpCtx<F>& c, const FitParams& P, int b_) {
         b = b_;
         const double* src = P.mean + (size_t)b_ * P.mean_stride;
-        for (int i = c.lane; i < P.N; i += 32) tc->mean_s[i] = src[i];
+        for (int i = c.lane; i < P.N; i += 32) mean_s[i] = src[i];
         __syncwarp();
-        return tc->mean_s;
+        return mean_s;
     }
     __device__ __forceinline__ double run(WarpCtx<F>& c, const double* pv, double* fout, double* Jout, int mode) {
         if (c.lane == 0) {
-            tc->cmd[0] = 1;
-            tc->cmd[1] = b;
-            tc->cmd[2] = (pv == c.pn) ? 1 : 0;
-            tc->cmd[3] = mode;
-            tc->cmd[4] = (fout ? 1 : 0) | (Jout ? 2 : 0);
-            tc->cmd[5] = (c.A == c.Abuf[1]) ? 1 : 0;
+            cmd[0] = 1;
+            cmd[1] = b;
+            cmd[2] = (pv == c.pn) ? 1 : 0;
+            cmd[3] = mode;
+            cmd[4] = (fout ? 1 : 0) | (Jout ? 2 : 0);
+            cmd[5] = (c.A == c.Abuf[1]) ? 1 : 0;
         }
         __syncwarp();
-        team_sync<TW>(tc->bar);
-        return team_eval<F, TW>(*tc, pv, mode, fout, Jout);
+        team_sync<TW>(bar);
+        return team_eval<F, TW>(c, 0, bar, pv, mode, fout, Jout);
     }
 };
 
@@ -692,7 +657,9 @@ fit_team_kernel(const __grid_constant__ FitParams P) {
         PhaseClock pk;
         pk.clear();
         TeamEval<F, TW> ev;
-        ev.tc = &tc;
+        ev.cmd = tc.cmd;
+        ev.mean_s = tc.mean_s;
+        ev.bar = tc.bar;
         for (;;) {
             int b = 0;
             if (lane == 0) {
@@ -721,10 +688,10 @@ fit_team_kernel(const __grid_constant__ FitParams P) {
             const int op = tc.cmd[0], b = tc.cmd[1], sel = tc.cmd[2], mode = tc.cmd[3], flags = tc.cmd[4];
             const int cur = tc.cmd[5];
             if (op == 0) break;
-            c.A = c.Abuf[cur]; c.g = c.gbuf[cur];
+            c.use_buf(cur);
             double* fout = (flags & 1) ? P.f_out + (size_t)b * P.nchiv : nullptr;
             double* Jout = (flags & 2) ? P.J_out + (size_t)b * P.nchiv * NP : nullptr;
-            team_eval<F, TW>(tc, sel ? c.pn : c.p, mode, fout, Jout);
+            team_eval<F, TW>(c, tw, tc.bar, sel ? c.pn : c.p, mode, fout, Jout);
         }
     }
 }
