@@ -207,6 +207,20 @@ int b200lm_set_policy(b200lm_handle h, int policy);
  * b200lm_fit_batch_host refuses a host p0 outside the box ("`x0` is infeasible.", as scipy does).  Every returned x
  * lies in the box. */
 int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub);
+/* parameter distributions of the following fit_batch and residual_jacobian calls on this handle: lsqfit's prior keys
+ * log(k), sqrt(k) and BufferDict.uniform(f, lo, hi) names.  h_code, h_lo, h_hi: HOST arrays of np entries in device
+ * parameter order; code 0 = plain key (the model sees p), 1 = log(k) (the model sees exp(p)), 2 = sqrt(k) (p^2),
+ * 3 = uniform (lo + (hi - lo) (1 + erf(p / sqrt 2)) / 2; h_lo / h_hi are read for code 3 only and may be NULL when no
+ * entry has it).  The fit runs in p: p0, x, cov, J, f, log det and the prior rows are in fit space, and only the data
+ * rows see q = T(p), with Jacobian columns df/dq_j T'(p_j).  NULL h_code clears the setting, and so does an all-zero
+ * code vector (the batches then run today's kernels, bit for bit).  With distributions set, fit_batch runs the
+ * one-warp kernel fit_kernel<F, 5> (the scipy trf decisions, polish and the QR covariance pass included): the default
+ * kernel choice drops to one warp per fit and an explicit b200lm_set_team(2 | 4 | 32) is B200LM_EINVAL at fit time.
+ * B200LM_EINVAL, with a message, for an unknown code; for code 3 with a non-finite lo or hi or lo >= hi; on a handle
+ * with windows or nslot > 1, with bounds, or with the GSL policy.  b200lm_set_windows, b200lm_set_bounds (finite
+ * bounds) and b200lm_set_policy(1) are refused in the same way while distributions are set.  Transforms on the team and
+ * wave kernels, windows, fit sets, bounds and the GSL policy are not built. */
+int b200lm_set_param_dist(b200lm_handle h, const int* h_code, const double* h_lo, const double* h_hi);
 /* number of kernel launches issued through this handle so far */
 long long b200lm_launch_count(b200lm_handle h);
 

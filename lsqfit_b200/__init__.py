@@ -18,6 +18,7 @@ from .fit import nonlinear_fit, gammaQ, BatchFits, FitView, wavg, WAvg, fit_set,
 from .dense import DenseFit
 from .bootstrap import bootstrap_means, normals
 from .multifit import MultiFitter, FunctorModel, SharedExpModel, ChainedFit
+from . import pdist                                   # noqa: F401  (parameter distributions: log(k), sqrt(k), uniform)
 
 __version__ = "0.1.0"
 

@@ -57,6 +57,36 @@ def _prior_size(prior):
     return int(np.size(getattr(prior, "flat", prior)[:]))
 
 
+def _prior_dist(prior):
+    """(code, lo, hi) in the order of the flat prior buffer from the distribution keys of a dictionary prior (``log(E)``,
+    ``sqrt(a)``, a ``BufferDict.uniform`` name), or None.  Each key's function is classified from a probe: a dictionary
+    of the prior's own type holding one value under ``f(k)``, read under ``k`` -- names are not trusted.  A prior whose
+    type does not resolve ``k`` (a plain dict) or a function the device does not have raises ValueError."""
+    from . import pdist as P
+    d = prior[0] if isinstance(prior, tuple) else prior
+    if not hasattr(d, "keys"):
+        return None
+    keys = list(d.keys())
+    if not any(P.parse_key(k)[0] is not None for k in keys):
+        return None
+    n = _prior_size(prior)
+    code, lo, hi = np.zeros(n, dtype=np.int32), np.zeros(n), np.ones(n)
+    cls, off = type(d), 0
+    for k in keys:
+        m = int(np.size(d[k]))
+        sl = d.slice(k) if hasattr(d, "slice") else slice(off, off + m)
+        off += m
+        fname, base = P.parse_key(k)
+        if fname is None:
+            continue
+        try:
+            c, a, b = P.classify(lambda v, k=k, base=base: cls({k: v})[base])
+        except ValueError as e:
+            raise ValueError("prior key %r: %s" % (k, e))
+        code[sl], lo[sl], hi[sl] = c, a, b
+    return (code, lo, hi) if code.any() else None
+
+
 def install(lsqfit):
     if getattr(lsqfit, "_b200lm_installed", False):
         return lsqfit
@@ -74,6 +104,13 @@ def install(lsqfit):
         if noprior:
             npar = None                         # taken from p0 by the fitter
         spec = ChivSpec(functor, x, yp_pdf, noprior, ny, npar if npar is not None else -1, pperm=pperm)
+        if not noprior:
+            # distribution keys: the device fits them with codes; one it cannot fit is refused by the device fitters
+            # only (the CPU fitters evaluate fcn on the prior's own dictionary and are not concerned)
+            try:
+                spec.pdist = _prior_dist(prior)
+            except ValueError as e:
+                spec.pdist_error = str(e)
         return _ChivProxy(cv, spec), cvw
 
     class b200_lm_plugin(b200_lm):

@@ -47,6 +47,7 @@ void fill_params(b200lm_handle_s* h, FitParams& P) {
     P.counter = h->d_counter;
     P.stats = h->d_stats;
     P.policy = h->policy;
+    if (h->ntrans > 0) { P.ntrans = h->ntrans; P.pd_code = h->d_pd_code; P.pd_lo = h->d_pd_lo; P.pd_hi = h->d_pd_hi; }
 }
 }  // namespace b200lm
 
@@ -198,7 +199,7 @@ static bool wave_ok(b200lm_handle_s* h) {
 // and <F, 3>).  Otherwise B200LM_TEAM = 0/1, 2, 4, 32 overrides default_team, and a team that the functor or the
 // shapes do not allow falls back to one warp.
 static int kernel_team(b200lm_handle_s* h) {
-    if (h->nwin > 0 || h->policy == 1 || h->bounded) return 1;
+    if (h->nwin > 0 || h->policy == 1 || h->bounded || h->ntrans > 0) return 1;
     int team = default_team(h);
     if (const char* env = getenv("B200LM_TEAM")) team = atoi(env);
     if (team == 32) return wave_ok(h) ? 32 : 1;
@@ -444,6 +445,7 @@ void b200lm_destroy(b200lm_handle h) {
     cudaFree(h->d_counter); cudaFree(h->d_stats); cudaFree(h->d_stage); cudaFree(h->d_scratch);
     cudaFree(h->d_order_key); cudaFree(h->d_order); cudaFree(h->d_wave_A);
     cudaFree(h->d_lb); cudaFree(h->d_ub);
+    cudaFree(h->d_pd_code); cudaFree(h->d_pd_lo); cudaFree(h->d_pd_hi);
     if (h->h_pinned) cudaFreeHost(h->h_pinned);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
@@ -486,6 +488,7 @@ int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* d
                        const double* blk_w) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
     if (nwin < 1 || !ndiag || !nblk) return set_error(h, B200LM_EINVAL, "bad window description");
+    if (h->ntrans > 0) return set_error(h, B200LM_EINVAL, "parameter distributions are not built for window scans");
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     // a window lists every prior entry and its own data rows exactly once; in a fit set, every entry of one slot
     // (checked below) and its own data rows
@@ -588,6 +591,9 @@ int b200lm_fit_batch(b200lm_handle h, int B,
         return set_error(h, B200LM_EINVAL, "bounds need the scipy trf policy (GSL's lm has no bound constraints)");
     rc = window_refusal(h, B);
     if (rc) return rc;
+    if (h->ntrans > 0 && h->team_request > 1)
+        return set_error(h, B200LM_EINVAL, "parameter distributions run one warp per fit: team / wave kernels (set_team "
+                                           "2, 4, 32) are not built for them");
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     cudaStream_t s = (cudaStream_t)stream;
     FitParams P;
@@ -704,6 +710,8 @@ int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub) {
             finite = finite || h_lb[j] > -INFINITY || h_ub[j] < INFINITY;
         }
     }
+    if (finite && h->ntrans > 0)
+        return set_error(h, B200LM_EINVAL, "bounds are not built for fits with parameter distributions");
     if (!finite) {                               // no bounds, or all infinite: scipy's unbounded trf
         h->bounded = false;
         h->h_lb.clear(); h->h_ub.clear();
@@ -720,7 +728,46 @@ int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub) {
 int b200lm_set_policy(b200lm_handle h, int policy) {
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
     if (policy != 0 && policy != 1) return set_error(h, B200LM_EINVAL, "policy must be 0 (scipy trf) or 1 (gsl lm)");
+    if (policy == 1 && h->ntrans > 0)
+        return set_error(h, B200LM_EINVAL, "the GSL policy is not built for fits with parameter distributions");
     h->policy = policy;
+    return B200LM_OK;
+}
+
+int b200lm_set_param_dist(b200lm_handle h, const int* h_code, const double* h_lo, const double* h_hi) {
+    if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (!h_code) { h->ntrans = 0; return B200LM_OK; }
+    int n = 0;
+    for (int j = 0; j < h->np; ++j) {
+        const int c = h_code[j];
+        const std::string where = "parameter " + std::to_string(j) + ": ";
+        if (c < 0 || c > 3)
+            return set_error(h, B200LM_EINVAL, where + "unknown distribution code " + std::to_string(c) +
+                                               " (0 plain, 1 log, 2 sqrt, 3 uniform)");
+        if (c == 3) {
+            if (!h_lo || !h_hi) return set_error(h, B200LM_EINVAL, where + "a uniform distribution needs lo and hi");
+            if (!std::isfinite(h_lo[j]) || !std::isfinite(h_hi[j]))
+                return set_error(h, B200LM_EINVAL, where + "the bounds of a uniform distribution must be finite");
+            if (!(h_lo[j] < h_hi[j]))
+                return set_error(h, B200LM_EINVAL, where + "a uniform distribution needs lo < hi");
+        }
+        n += c != 0;
+    }
+    if (h->nwin > 0 || h->nslot > 1)
+        return set_error(h, B200LM_EINVAL, "parameter distributions are not built for window scans or fit sets");
+    if (h->bounded) return set_error(h, B200LM_EINVAL, "bounds are not built for fits with parameter distributions");
+    if (h->policy == 1)
+        return set_error(h, B200LM_EINVAL, "the GSL policy is not built for fits with parameter distributions");
+    if (n == 0) { h->ntrans = 0; return B200LM_OK; }        // all plain: today's kernels
+    std::vector<double> lo(h->np, 0.0), hi(h->np, 1.0);
+    for (int j = 0; j < h->np; ++j)
+        if (h_code[j] == 3) { lo[j] = h_lo[j]; hi[j] = h_hi[j]; }
+    CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
+    h->ntrans = 0;                  // upload() frees the old buffers first: a failure below leaves the handle without codes
+    CUDA_TRY(h, upload(&h->d_pd_code, h_code, (size_t)h->np), "upload distribution codes");
+    CUDA_TRY(h, upload(&h->d_pd_lo, lo.data(), lo.size()), "upload distribution codes");
+    CUDA_TRY(h, upload(&h->d_pd_hi, hi.data(), hi.size()), "upload distribution codes");
+    h->ntrans = n;
     return B200LM_OK;
 }
 

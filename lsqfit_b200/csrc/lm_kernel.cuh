@@ -318,12 +318,17 @@ __device__ __forceinline__ int prior_base(const WinRows& T) { return T.pr_base; 
 
 // T: the row tables (nd_fn, dfn_idx, dfn_w, nd_pr, dpr_idx, dpr_w, nblk, blk) -- the FitParams themselves, or those of
 // one window (WinRows)
-template <class F, int MODE, bool WSMEM, class RS>
-__device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const double* pv, double* fout, double* Jout) {
+// TRANS (parameter distributions, fit_kernel<F, 5>): the data rows see the model at qv = T(pv), and their Jacobian
+// columns are scaled by tp = T'(pv); the prior rows stay in pv
+template <class F, int MODE, bool WSMEM, class RS, bool TRANS = false>
+__device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const double* pv, double* fout, double* Jout,
+                                            const double* qv = nullptr, const double* tp = nullptr) {
     typedef FitLayout<F> Lay;
     constexpr int NP = Lay::NP, NT = Lay::NT, LDR = Lay::LDR, LDA = Lay::LDA, NCOL = Lay::NCOL;
     const FitParams& P = c.P;
     const int lane = c.lane;
+    const double* mv = pv;                  // the parameters the model sees
+    if constexpr (TRANS) mv = qv;
     for (int e = lane; e < NP * LDA; e += 32) c.A[e] = 0.0;
     if (MODE == 0 && lane < NP) c.g[lane] = 0.0;
     __syncwarp();
@@ -356,7 +361,11 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
         if (lane < nrows) {
             const int row = T.dfn_idx[c0 + lane];
             const double w = T.dfn_w[c0 + lane];
-            const double f = F::value_grad(P.x + (size_t)row * P.nx, row, pv, w, row_);
+            const double f = F::value_grad(P.x + (size_t)row * P.nx, row, mv, w, row_);
+            if constexpr (TRANS) {
+#pragma unroll
+                for (int j = 0; j < NP; ++j) row_[j] *= tp[j];
+            }
             row_[NP] = w * (f - c.mean[row]);
 #pragma unroll
             for (int j = NP + 1; j < NCOL; ++j) row_[j] = 0.0;
@@ -394,7 +403,11 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
                     const int idx = P.blk_idx[bd.idx_off + k0 + lane];
                     double dlt;
                     if (idx < P.ny) {
-                        const double f = F::value_grad(P.x + (size_t)idx * P.nx, idx, pv, 1.0, row_);
+                        const double f = F::value_grad(P.x + (size_t)idx * P.nx, idx, mv, 1.0, row_);
+                        if constexpr (TRANS) {
+#pragma unroll
+                            for (int j = 0; j < NP; ++j) row_[j] *= tp[j];
+                        }
                         dlt = f - c.mean[idx];
                     } else {
                         const int j0 = idx - prior_base(T);
@@ -520,6 +533,47 @@ __device__ __noinline__ double eval_win_impl(const WarpCtx<F>& c_in, int w, cons
             for (int q = 0; q < F::NP; ++q) Jout[(size_t)i * F::NP + q] = 0.0;
     }
     return cost;
+}
+
+// q = T(p) and dq/dp of one parameter with distribution code `code` (FitParams::pd_code; the uniform form is
+// written with erfc, which keeps q - lo accurate in the lower tail; host mirror: lsqfit_b200/pdist.py)
+__device__ __forceinline__ void param_transform(int code, double lo, double hi, double p, double& q, double& dq) {
+    if (code == 1) {
+        q = exp(p); dq = q;
+    } else if (code == 2) {
+        q = p * p; dq = 2.0 * p;
+    } else if (code == 3) {
+        const double w = hi - lo;
+        q = fma(w, 0.5 * erfc(-0.7071067811865476 * p), lo);
+        dq = w * 0.3989422804014327 * exp(-0.5 * p * p);                 // (hi - lo) exp(-p^2/2) / sqrt(2 pi)
+    } else {
+        q = p; dq = 1.0;
+    }
+}
+
+// evaluation with parameter distributions: lane j < NP puts q_j = T(p_j) and T'(p_j) into the warp's qt buffer
+// (q [NP] | T' [NP], behind the per-warp layout of FitLayout), then the rows as in eval_full with TRANS set
+template <class F, int MODE, bool WSMEM>
+__device__ __noinline__ double eval_trans_impl(const WarpCtx<F>& c_in, double* qt, const double* pv, double* fout,
+                                               double* Jout) {
+    WarpCtx<F> c = c_in;
+    __builtin_assume(__isShared(c.R));
+    __builtin_assume(__isShared(c.dvec));
+    __builtin_assume(__isShared(c.A));
+    __builtin_assume(__isShared(c.g));
+    __builtin_assume(__isShared(c.dsc));
+    __builtin_assume(__isShared(pv));
+    __builtin_assume(__isShared(qt));
+    constexpr int NP = F::NP;
+    const FitParams& P = c.P;
+    if (c.lane < NP) {
+        double q, dq;
+        param_transform(P.pd_code[c.lane], P.pd_lo[c.lane], P.pd_hi[c.lane], pv[c.lane], q, dq);
+        qt[c.lane] = q;
+        qt[NP + c.lane] = dq;
+    }
+    __syncwarp();
+    return eval_rows<F, MODE, WSMEM, FitParams, true>(c, P, pv, fout, Jout, qt, qt + NP);
 }
 
 // ---------------------------------------------------------------------------
@@ -1190,7 +1244,8 @@ __device__ double select_step(WarpCtx<F>& c, double x, double gh, double& s_h, d
 // ---------------------------------------------------------------------------
 // the fit kernel
 // ---------------------------------------------------------------------------
-template <class F>
+// EXTRA: doubles per warp behind the layout of FitLayout (the q | T' buffer of TransEval)
+template <class F, int EXTRA = 0>
 __device__ __forceinline__ void setup_ctx(WarpCtx<F>& c, double* smem, const FitParams& P) {
     typedef FitLayout<F> Lay;
     const int warp = threadIdx.x >> 5;
@@ -1202,7 +1257,7 @@ __device__ __forceinline__ void setup_ctx(WarpCtx<F>& c, double* smem, const Fit
     } else {
         c.wt = P.blk_wt;
     }
-    double* base = smem + wt_region + (size_t)warp * Lay::per_warp_doubles(P.rb);
+    double* base = smem + wt_region + (size_t)warp * (Lay::per_warp_doubles(P.rb) + EXTRA);
     c.R = base;
     c.dvec = c.R + (size_t)P.rb * Lay::LDR;
     c.Abuf[0] = c.dvec + P.rb;
@@ -1247,8 +1302,28 @@ struct WinEval {
     }
 };
 
-template <class F, int MODE> struct EvalOf { typedef WarpEval<F> type; };
-template <class F> struct EvalOf<F, 4> { typedef WinEval<F> type; };
+// Evaluator of the kernels with parameter distributions (fit_kernel<F, 5>, resjac_trans_kernel): as WarpEval, with the
+// model evaluated at q = T(p) (eval_trans_impl)
+template <class F>
+struct TransEval {
+    static constexpr int EXTRA = 2 * F::NP;         // doubles per warp: q | T'
+    double* qt;
+    __device__ __forceinline__ const double* begin(WarpCtx<F>& c, const FitParams& P, int b) {
+        qt = c.R + FitLayout<F>::per_warp_doubles(P.rb);
+        return P.mean + (size_t)b * P.mean_stride;
+    }
+    __device__ __forceinline__ double run(WarpCtx<F>& c, const double* pv, double* fout, double* Jout, int mode) {
+        if (c.P.wt_in_smem)
+            return mode == 0 ? eval_trans_impl<F, 0, true>(c, qt, pv, fout, Jout)
+                             : eval_trans_impl<F, 1, true>(c, qt, pv, fout, Jout);
+        return mode == 0 ? eval_trans_impl<F, 0, false>(c, qt, pv, fout, Jout)
+                         : eval_trans_impl<F, 1, false>(c, qt, pv, fout, Jout);
+    }
+};
+
+template <class F, int MODE> struct EvalOf { typedef WarpEval<F> type; static constexpr int EXTRA = 0; };
+template <class F> struct EvalOf<F, 4> { typedef WinEval<F> type; static constexpr int EXTRA = 0; };
+template <class F> struct EvalOf<F, 5> { typedef TransEval<F> type; static constexpr int EXTRA = TransEval<F>::EXTRA; };
 
 // One complete fit (number b of the batch) driven by the warp that owns `c`: trust-region loop, optional
 // polish, covariance, results.  EV::run evaluates residual + Jacobian + normal equations at a point -- by
@@ -1265,7 +1340,9 @@ struct PhaseClock {
 // would only cost registers and instruction cache):  0 = scipy TRF decisions (the default kernels),  1 = GSL trust/lm
 // decisions (b200lm_set_policy),  2 = no loop at all: finalisation of fits the wave kernel has already converged,
 // 3 = scipy TRF with bound constraints (trf_bounds: Coleman-Li scaling, select_step; b200lm_set_bounds),
-// 4 = scipy TRF on fit windows (the loop of MODE 0; EV = WinEval: rows, weights and means per window, b200lm_set_windows).
+// 4 = scipy TRF on fit windows (the loop of MODE 0; EV = WinEval: rows, weights and means per window, b200lm_set_windows),
+// 5 = scipy TRF with parameter distributions (the loop of MODE 0; EV = TransEval: the model at q = T(p),
+// b200lm_set_param_dist).
 template <class F, class EV, int MODE = 0>
 __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& P, int b,
                                         unsigned long long& tot_nfev, unsigned long long& tot_njev,
@@ -1428,7 +1505,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
 
         // MODE 3 (bounds) is the same loop with scipy's trf_bounds changes: the gtol test on |g v|_inf, the scaling
         // d = sqrt(v) / scale_inv, the Coleman-Li diagonal in the sub-problem, select_step, strictly feasible trials
-        while ((MODE == 0 || MODE == 3 || MODE == 4) && status == -2) {
+        while ((MODE == 0 || MODE == 3 || MODE == 4 || MODE == 5) && status == -2) {
             const double gi = act ? c.g[lane] : 0.0;
             double v = 1.0, dv = 0.0;                              // Coleman-Li scaling (MODE 3)
             const double xi = act ? c.p[lane] : 0.0;
@@ -1670,7 +1747,7 @@ __global__ void __launch_bounds__(FitLayout<F>::MAX_WARPS * 32, 1) fit_kernel(co
     static_assert(Lay::NP <= 32, "one lane per parameter");
     extern __shared__ double smem[];
     WarpCtx<F> c(P);
-    setup_ctx<F>(c, smem, P);
+    setup_ctx<F, EvalOf<F, MODE>::EXTRA>(c, smem, P);
     const int lane = c.lane;
     unsigned long long tot_nfev = 0, tot_njev = 0, tot_nfac = 0;
     typename EvalOf<F, MODE>::type ev;
@@ -1722,6 +1799,29 @@ __global__ void __launch_bounds__(FitLayout<F>::MAX_WARPS * 32, 1) resjac_kernel
     }
 }
 
+// the same with parameter distributions (P.ntrans > 0): f and J in fit space, J = dchiv/dp
+template <class F>
+__global__ void __launch_bounds__(FitLayout<F>::MAX_WARPS * 32, 1) resjac_trans_kernel(const __grid_constant__ FitParams P) {
+    constexpr int NP = F::NP;
+    extern __shared__ double smem[];
+    WarpCtx<F> c(P);
+    setup_ctx<F, TransEval<F>::EXTRA>(c, smem, P);
+    const int lane = c.lane;
+    TransEval<F> ev;
+    const int warp_global = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int nwarps = gridDim.x * (blockDim.x >> 5);
+    for (int b = warp_global; b < P.B; b += nwarps) {
+        c.mean = ev.begin(c, P, b);
+        const double* p0 = P.p0 + (size_t)b * P.p0_stride;
+        if (lane < NP) c.p[lane] = p0[lane];
+        __syncwarp();
+        const double cost = ev.run(c, c.p, P.f_out ? P.f_out + (size_t)b * P.nchiv : nullptr,
+                                   P.J_out ? P.J_out + (size_t)b * P.nchiv * NP : nullptr, 0);
+        if (lane == 0 && P.chi2) P.chi2[b] = 2.0 * cost;
+        __syncwarp();
+    }
+}
+
 // ---------------------------------------------------------------------------
 // host-side launchers
 // ---------------------------------------------------------------------------
@@ -1730,11 +1830,12 @@ struct LaunchInfo {
     size_t smem;
 };
 
+// extra: doubles per warp behind the FitLayout (EvalOf<F, MODE>::EXTRA of the kernel launched)
 template <class F>
-inline cudaError_t plan_launch(FitParams& P, int sm_count, size_t smem_budget, LaunchInfo& li) {
+inline cudaError_t plan_launch(FitParams& P, int sm_count, size_t smem_budget, LaunchInfo& li, int extra = 0) {
     typedef FitLayout<F> Lay;
     const size_t wt_bytes = ((size_t)(P.wt_total + 1) & ~(size_t)1) * sizeof(double);
-    const size_t per_warp = (size_t)Lay::per_warp_doubles(P.rb) * sizeof(double);
+    const size_t per_warp = (size_t)(Lay::per_warp_doubles(P.rb) + extra) * sizeof(double);
     P.wt_in_smem = (P.nwin == 0 && P.wt_total > 0 && wt_bytes + 4 * per_warp <= smem_budget) ? 1 : 0;
     const size_t avail = smem_budget - (P.wt_in_smem ? wt_bytes : 0);
     int warps = (int)(avail / per_warp);
@@ -1766,8 +1867,12 @@ cudaError_t launch_fit_mode(const FitParams& P, const LaunchInfo& li, cudaStream
 template <class F>
 cudaError_t launch_fit(FitParams P, int sm_count, size_t smem_budget, cudaStream_t stream) {
     LaunchInfo li;
-    cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li);
+    // parameter distributions: b200lm_set_param_dist refuses windows, bounds and the GSL policy, and the wave kernel
+    // (the only user of finalize_only) does not run with them
+    const bool trans = P.ntrans > 0;
+    cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li, trans ? EvalOf<F, 5>::EXTRA : 0);
     if (e != cudaSuccess) return e;
+    if (trans) return launch_fit_mode<F, 5>(P, li, stream);
     if (P.nwin > 0) return launch_fit_mode<F, 4>(P, li, stream);
     if (P.finalize_only) return launch_fit_mode<F, 2>(P, li, stream);
     if (P.bounded) return launch_fit_mode<F, 3>(P, li, stream);
@@ -1778,6 +1883,14 @@ cudaError_t launch_fit(FitParams P, int sm_count, size_t smem_budget, cudaStream
 template <class F>
 cudaError_t launch_resjac(FitParams P, int sm_count, size_t smem_budget, cudaStream_t stream) {
     LaunchInfo li;
+    if (P.ntrans > 0) {
+        cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li, TransEval<F>::EXTRA);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(resjac_trans_kernel<F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)li.smem);
+        if (e != cudaSuccess) return e;
+        resjac_trans_kernel<F><<<li.grid, li.block, li.smem, stream>>>(P);
+        return cudaGetLastError();
+    }
     cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li);
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(resjac_kernel<F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)li.smem);

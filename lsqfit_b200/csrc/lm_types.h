@@ -93,6 +93,13 @@ struct FitParams {
                                 // tables above (dfn_*, dpr_*, blk, blk_idx, blk_wt) hold every window, one after the other
     int win_copies;
     const WinDesc* win;         // [nwin]
+    // ---- parameter distributions (last, for the same reason; b200lm_set_param_dist) ----
+    int ntrans;                 // > 0: the model sees q = T(p) (fit_kernel<F, 5>, resjac_trans_kernel); the fit, the prior
+                                // rows and every output stay in p
+    const int* pd_code;         // [np] 0: q = p, 1 log(k): q = exp(p), 2 sqrt(k): q = p^2,
+                                //      3 uniform: q = lo + (hi - lo) (1 + erf(p / sqrt 2)) / 2
+    const double* pd_lo;        // [np] lo and hi of code 3
+    const double* pd_hi;
 };
 
 }  // namespace b200lm

@@ -359,6 +359,12 @@ class DenseFit(object):
         self.d_y = torch.as_tensor(np.ascontiguousarray(data_mean)).to(dev)
         self.d_pm = torch.as_tensor(pm).to(dev)
         self.d_wp = torch.as_tensor(np.zeros(self.np) if self.noprior_rows else 1.0 / psd).to(dev)
+        # parameter distributions (lsqfit_b200/pdist.py): the model rows see q = T(p), their columns are scaled by T'(p)
+        self._pd = None
+        if spec is not None and spec.pdist is not None:
+            if bounds is not None:
+                raise ValueError("b200_dense: bounds are not built for fits with parameter distributions")
+            self._pd = tuple(torch.as_tensor(a).to(dev) for a in spec.device_pdist)
         self.prior_mean, self.prior_sdev = pm, psd
         self.logdet_pdf = data_logdet + prior_logdet
         self.nchiv = nd + npr
@@ -406,7 +412,26 @@ class DenseFit(object):
             pass
 
     # ---- residuals and Jacobian (a-2) -------------------------------------------------------
+    def _transform(self, p):
+        """(q = T(p), T'(p)) on the device; (p, None) without parameter distributions"""
+        if self._pd is None:
+            return p, None
+        code, lo, hi = self._pd
+        e = torch.exp(torch.where(code == 1, p, torch.zeros_like(p)))
+        u = lo + (hi - lo) * (0.5 * torch.special.erfc(-0.7071067811865476 * p))
+        du = (hi - lo) * 0.3989422804014327 * torch.exp(-0.5 * p * p)
+        q = torch.where(code == 1, e, torch.where(code == 2, p * p, torch.where(code == 3, u, p)))
+        dq = torch.where(code == 1, e, torch.where(code == 2, 2.0 * p, torch.where(code == 3, du, torch.ones_like(p))))
+        return q.contiguous(), dq
+
     def _model(self, p, with_G):
+        p, dq = self._transform(p)
+        self._keep_q = p                                        # (the launch reads it asynchronously)
+        self._model_at(p, with_G)
+        if with_G and dq is not None:
+            self.G.mul_(dq[None, :])
+
+    def _model_at(self, p, with_G):
         la = self.la
         if self._h is not None:
             _cabi.check(_cabi.lib.b200lm_model_rows(
@@ -475,7 +500,9 @@ class DenseFit(object):
         fp = self._prior_residual(p)
         self.nfev_jac += 1
         if self.fused and not materialize:
-            _cabi.check(_cabi.lib.b200lm_normal_diag(self._h, p.data_ptr(), self.d_y.data_ptr(), self.wdiag.data_ptr(),
+            q, dq = self._transform(p)
+            self._keep_q = q
+            _cabi.check(_cabi.lib.b200lm_normal_diag(self._h, q.data_ptr(), self.d_y.data_ptr(), self.wdiag.data_ptr(),
                                                      self.nacc.data_ptr(), la.stream()), self._h)
             la.launches += 2
             n = self.np
@@ -484,6 +511,9 @@ class DenseFit(object):
             self.A[self._triu[0], self._triu[1]] = self.nacc[:nt]
             self.A.copy_(self.A + self.A.T - torch.diag(self.A.diagonal()))
             g = self.nacc[nt:nt + n].clone()
+            if dq is not None:                                  # J = J_q diag(T'): J^T J and J^T r in fit space
+                self.A.mul_(dq[:, None] * dq[None, :])
+                g.mul_(dq)
             self.cost_data = self.nacc[nt + n].clone()
             return None, fp, self._add_prior(fp, g)
         self._model(p, True)
@@ -887,6 +917,8 @@ class b200_dense(object):
         if spec is None:
             raise ValueError("the b200_dense fitter needs a device functor: use lsqfit_b200.Functor(...) as fcn "
                              "and install the hook with lsqfit_b200.register() (no CPU fallback exists)")
+        if spec.pdist_error is not None:
+            raise ValueError("b200_dense: " + spec.pdist_error)
         self.tol, self.maxit, self.n = normalize_tol(tol), maxit, n
         self.x0 = np.array(x0, dtype=float)
         if spec.np < 0:

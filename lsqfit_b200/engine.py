@@ -49,9 +49,11 @@ class BatchResult(object):
 
 
 class Plan(object):
-    def __init__(self, functor, np_, ny, x, i_invwgts, noprior=False, device=0, team=None, nslot=1):
+    def __init__(self, functor, np_, ny, x, i_invwgts, noprior=False, device=0, team=None, nslot=1, pdist=None):
         """nslot > 1: a fit set (b200lm_create_set) -- y (+) prior is ny data rows, then nslot prior slots of np
-        entries; ``i_invwgts`` must be None, and the plan fits once ``set_windows`` has given one window per problem."""
+        entries; ``i_invwgts`` must be None, and the plan fits once ``set_windows`` has given one window per problem.
+        pdist: None or (code, lo, hi) in device parameter order (lsqfit_b200/pdist.py, b200lm_set_param_dist): every
+        fit and residual / Jacobian of the plan then sees the model at q = T(p)."""
         if isinstance(functor, str):
             functor = Functor(functor)
         self.functor = functor
@@ -73,6 +75,24 @@ class Plan(object):
         self.tdev = torch.device("cuda", self.device)
         if team is not None:
             self.set_team(team)
+        self.pdist = None
+        if pdist is not None:
+            self.set_param_dist(*pdist)
+
+    def set_param_dist(self, code=None, lo=None, hi=None):
+        """Parameter distributions (b200lm_set_param_dist): code [np] (0 plain, 1 log, 2 sqrt, 3 uniform), lo / hi [np]
+        (read for code 3), device parameter order; no arguments clear them."""
+        if code is None:
+            _cabi.check(_cabi.lib.b200lm_set_param_dist(self._h, None, None, None), self._h)
+            self.pdist = None
+            return
+        code = np.ascontiguousarray(code, dtype=np.int32)
+        lo = np.ascontiguousarray(np.zeros(self.np) if lo is None else lo, dtype=np.float64)
+        hi = np.ascontiguousarray(np.ones(self.np) if hi is None else hi, dtype=np.float64)
+        if code.shape != (self.np,) or lo.shape != (self.np,) or hi.shape != (self.np,):
+            raise ValueError("set_param_dist: code, lo and hi need np = %d entries" % self.np)
+        _cabi.check(_cabi.lib.b200lm_set_param_dist(self._h, code.ctypes.data, lo.ctypes.data, hi.ctypes.data), self._h)
+        self.pdist = (code, lo, hi) if code.any() else None
 
     # ---- whitening ---------------------------------------------------------------
     def set_weights(self, i_invwgts):

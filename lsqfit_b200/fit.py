@@ -15,6 +15,10 @@ Array forms of the reference's GVar inputs:
           or (ymean, ycov | ysdev) for ``fcn(p)`` models without x
   prior = (pmean, pcov | psdev) or None
   yp_cov= optional joint covariance of y (+) prior when data and prior are correlated
+  pdist = optional parameter distributions, the array form of lsqfit's ``log(k)`` / ``sqrt(k)`` /
+          ``BufferDict.uniform`` prior keys: one entry per parameter, None, 'log', 'sqrt' or ('uniform', lo, hi).
+          The fit runs in the fit parameters p (prior, p0, pmean, cov, fit.p, logGBF), and ``fcn`` sees
+          q = T(p) (lsqfit_b200/pdist.py)
 
 Reference lines followed: src/lsqfit/__init__.py:455-733 (constructor), :897-922 (_getp),
 :1391-1469, 1471-1543 (simulated fits), :1548-1642 (bootstrap), :1947-1948 (default p0).
@@ -71,7 +75,7 @@ class nonlinear_fit(object):
 
     def __init__(self, data=None, fcn=None, prior=None, p0=None, svdcut=False, eps=False,
                  tol=1e-8, maxit=1000, fitter="b200_lm", yp_cov=None, _yp_pdf=None,
-                 noise=False, noise_seed=None, **fitterargs):
+                 noise=False, noise_seed=None, pdist=None, **fitterargs):
         clock = time.perf_counter()
         svdcut, eps = resolve_svdcut_eps(svdcut, eps)
         # noise = (svd noise, prior noise), a bool meaning both (src/lsqfit/__init__.py:493-499, 516)
@@ -115,6 +119,8 @@ class nonlinear_fit(object):
                 Lp = np.linalg.cholesky(pcov) if np.count_nonzero(pcov - np.diag(np.diag(pcov))) else np.diag(np.sqrt(np.diag(pcov)))
                 pmean = pmean + Lp @ normals(npar, int(noise_seed) ^ 0x9E3779B97F4A7C15,
                                              device=int(fitterargs.get("device", 0))).cpu().numpy()
+        from .pdist import codes as _pdist_codes
+        self.pdist = _pdist_codes(pdist, npar)
         N = ny if noprior else ny + npar
         mean = ymean if noprior else np.concatenate([ymean, pmean])
         # ---- whitening (device) : __init__.py:539-561 ------------------------------
@@ -143,7 +149,7 @@ class nonlinear_fit(object):
         if self.p0.size != npar:
             raise ValueError("p0 and prior shapes incompatible")
         # ---- chiv : __init__.py:571-575 ---------------------------------------------
-        spec = ChivSpec(fcn, x, pdf, noprior, ny, npar)
+        spec = ChivSpec(fcn, x, pdf, noprior, ny, npar, pdist=self.pdist)
         self._chiv = DeviceChiv(spec, self.device)
         nf = pdf.nchiv
         self.dof = nf - self.p0.size
@@ -222,8 +228,16 @@ class nonlinear_fit(object):
                    maxit=self.maxit if args.get("maxit") is None else args["maxit"],
                    scaler=args.get("scaler", "more"), polish=args.get("polish", 0), policy=args.get("policy", "trf"),
                    bounds=bounds)
-        kernel = args.get("kernel")
-        return fit, 32 if kernel == "wave" else kernel, args.get("loss", "linear"), POLICY.get(fit["policy"]) == 1
+        kernel = 32 if args.get("kernel") == "wave" else args.get("kernel")
+        if self.pdist is not None:
+            if kernel is not None and int(kernel) > 1:
+                raise ValueError("b200_lm: kernel=%r is not built for fits with parameter distributions (they run one "
+                                 "warp per fit)" % (args.get("kernel"),))
+            if bounds is not None:
+                raise ValueError("b200_lm: bounds are not built for fits with parameter distributions")
+            if POLICY.get(fit["policy"]) == 1:
+                raise ValueError("b200_lm: policy='gsl' is not built for fits with parameter distributions")
+        return fit, kernel, args.get("loss", "linear"), POLICY.get(fit["policy"]) == 1
 
     def _batch(self, means, p0, tol=None, maxit=None, want_cov=True, **kargs):
         plan = self._spec.plan(self.device)
@@ -282,14 +296,18 @@ class nonlinear_fit(object):
 
     def simulated_means(self, n, pexact=None, add_priornoise=False, seed=None):
         """__init__.py:1471-1543: data means fcn(pexact) + noise, prior means fixed unless
-        add_priornoise."""
+        add_priornoise.  pexact is in fit space: with parameter distributions the data means are fcn(T(pexact))."""
         pexact = self.pmean if pexact is None else np.asarray(pexact, dtype=float)
         plan = self._spec.plan(self.device)
         # f(pexact) from the device functor: residuals with zero means and unit weights are
         # not available, so evaluate the registered host mirror (numpy) -- it is the same
         # call the reference makes on the host (__init__.py:1522).
         ny = self._spec.ny
-        fexact = np.asarray(self.fcn(self.fcn.xrows(self.x, ny), pexact), dtype=float)
+        qexact = pexact
+        if self.pdist is not None:
+            from .pdist import transform
+            qexact = transform(*self.pdist, pexact)[0]
+        fexact = np.asarray(self.fcn(self.fcn.xrows(self.x, ny), qexact), dtype=float)
         means = self.bootstrap_means(n, seed)
         base = torch.as_tensor(self.yp_pdf.mean).to(means.device)
         noise = means - base[None, :]
@@ -476,6 +494,8 @@ class WindowScan(_WindowFits):
             raise refuse("policy='gsl' is")
         if any(parent.noise):
             raise refuse("fits made with noise are")
+        if parent.pdist is not None:
+            raise refuse("parameter distributions (pdist) are")
         spec = parent._spec
         self.parent, self.device = parent, parent.device
         self.np, self.ny = spec.np, spec.ny
@@ -579,6 +599,9 @@ class FitSet(_WindowFits):
         from .engine import POLICY, Plan
         from .windows import set_description
         refuse = lambda what: ValueError("b200_lm: %s not built for fit sets" % what)
+        if fitterargs.get("pdist") is not None:
+            raise refuse("parameter distributions (pdist) are")
+        fitterargs.pop("pdist", None)
         unknown = sorted(set(fitterargs) - set(_SET_ARGS))
         if unknown:
             raise ValueError("fit_set: unknown fitter arguments: " + ", ".join(unknown))

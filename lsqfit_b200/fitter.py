@@ -25,7 +25,8 @@ class PlanCache(object):
     The reference's iterators construct one ``nonlinear_fit`` per bootstrap copy (src/lsqfit/__init__.py:1612-1624)
     and each of them rebuilds chiv -- but model, x and whitening are the same for every copy, only the means move.
     A plan (device handle, uploaded x and weights, workspaces, stream) is therefore keyed by a digest of
-    (functor, np, ny, x, i_invwgts, noprior, device): a copy then costs one launch, not a ``b200lm_create``."""
+    (functor, np, ny, x, i_invwgts, noprior, device) and the parameter distributions (b200lm_set_param_dist; a plan
+    is never shared between fits with different ones): a copy then costs one launch, not a ``b200lm_create``."""
 
     def __init__(self, capacity=16):
         import collections
@@ -34,7 +35,7 @@ class PlanCache(object):
         self.hits = self.misses = 0
 
     @staticmethod
-    def key(functor, np_, ny, x, i_invwgts, noprior, device):
+    def key(functor, np_, ny, x, i_invwgts, noprior, device, pdist=None):
         import hashlib
         h = hashlib.blake2b(digest_size=16)
         h.update(("%s|%d|%d|%d|%d|%d" % (functor.name, functor.family, int(np_), int(ny), int(bool(noprior)), int(device))).encode())
@@ -42,17 +43,21 @@ class PlanCache(object):
         for idx, w in i_invwgts:
             h.update(np.ascontiguousarray(idx, dtype=np.int64).tobytes())
             h.update(np.ascontiguousarray(w, dtype=np.float64).tobytes())
+        if pdist is not None:
+            h.update(b"pdist")
+            for a, dt in zip(pdist, (np.int32, np.float64, np.float64)):
+                h.update(np.ascontiguousarray(a, dtype=dt).tobytes())
         return h.hexdigest()
 
-    def get(self, functor, np_, ny, x, i_invwgts, noprior, device):
-        k = self.key(functor, np_, ny, x, i_invwgts, noprior, device)
+    def get(self, functor, np_, ny, x, i_invwgts, noprior, device, pdist=None):
+        k = self.key(functor, np_, ny, x, i_invwgts, noprior, device, pdist)
         plan = self.plans.get(k)
         if plan is not None:
             self.hits += 1
             self.plans.move_to_end(k)
             return plan
         self.misses += 1
-        plan = Plan(functor, np_, ny, x, i_invwgts, noprior=noprior, device=device)
+        plan = Plan(functor, np_, ny, x, i_invwgts, noprior=noprior, device=device, pdist=pdist)
         self.plans[k] = plan
         while len(self.plans) > self.capacity:
             _, old = self.plans.popitem(last=False)
@@ -72,13 +77,24 @@ PLAN_CACHE = PlanCache()
 class ChivSpec(object):
     """Everything the device needs to evaluate chiv: functor, x, whitening, means."""
 
-    def __init__(self, functor, x, pdf, noprior, ny, np_, pperm=None):
+    def __init__(self, functor, x, pdf, noprior, ny, np_, pperm=None, pdist=None):
         self.functor, self.x, self.pdf, self.noprior = functor, x, pdf, bool(noprior)
         self.ny, self.np = int(ny), int(np_)
         # pperm[k] = position in the CALLER's flat parameter buffer of device parameter k (composite functors fix
         # their own parameter order; lsqfit's buffer follows the prior dictionary); None = identical
         self.pperm = None if pperm is None else np.asarray(pperm, dtype=np.int64)
+        # parameter distributions (code, lo, hi) in the CALLER's order (lsqfit_b200/pdist.py); None = all plain;
+        # pdist_error: why the prior's distribution keys cannot be fitted on the device (the device fitters refuse)
+        self.pdist = pdist
+        self.pdist_error = None
         self._plans = {}
+
+    @property
+    def device_pdist(self):
+        """the parameter distributions in DEVICE order (None: all plain)"""
+        if self.pdist is None:
+            return None
+        return tuple(np.ascontiguousarray(a if self.pperm is None else a[self.pperm]) for a in self.pdist)
 
     def _inv(self):
         inv = np.empty_like(self.pperm)
@@ -119,7 +135,7 @@ class ChivSpec(object):
     def plan(self, device=0):
         if device not in self._plans:
             self._plans[device] = PLAN_CACHE.get(self.functor, self.np, self.ny, self.x, self.i_invwgts,
-                                                 self.noprior, device)
+                                                 self.noprior, device, self.device_pdist)
         return self._plans[device]
 
 
@@ -189,6 +205,8 @@ class b200_lm(object):
             raise ValueError(
                 "the b200_lm fitter needs a device functor: use lsqfit_b200.Functor(...) as fcn "
                 "and install the hook with lsqfit_b200.register() (no CPU fallback exists)")
+        if spec.pdist_error is not None:
+            raise ValueError("b200_lm: " + spec.pdist_error)
         self.tol = normalize_tol(tol)
         self.maxit = maxit
         self.n = n
@@ -203,6 +221,11 @@ class b200_lm(object):
         if spec.np < 0:
             spec.np = self.x0.size
         robust = loss != "linear"
+        if spec.pdist is not None and bounds is not None:
+            raise ValueError("b200_lm: bounds are not built for fits with parameter distributions (pdist / log(k), "
+                             "sqrt(k) prior keys)")
+        if spec.pdist is not None and gsl:
+            raise ValueError("b200_lm: policy='gsl' is not built for fits with parameter distributions")
         if bounds is not None or robust or not any(fam == spec.functor.family and m == spec.np
                                                    for fam, m, _, _ in functor_table()):
             # no batched kernel for this parameter count, bound constraints (scipy's ``bounds``) or a robust loss

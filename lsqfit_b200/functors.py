@@ -188,6 +188,12 @@ class Functor(object):
         self._host = _HOST[name]
 
     def __call__(self, x, p):
+        if hasattr(p, "keys"):
+            # a dictionary of parameters (lsqfit's BufferDict): flattened in its key order under the MODEL-space keys,
+            # so a key log(E) contributes p['E'] = exp(p['log(E)']) -- what the device functor sees through the
+            # distribution codes
+            from .pdist import parse_key
+            p = np.concatenate([np.atleast_1d(p[parse_key(k)[1]]) for k in p.keys()])
         return self._host(x, p)
 
     def xrows(self, x, ny):

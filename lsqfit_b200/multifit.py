@@ -61,11 +61,21 @@ def composite(multifcn, po, yo):
     if M not in (2, 3) or len(set(m.E for m in models)) != 1 or len(set(m.a for m in models)) != M:
         return None
     ps, ys = _slices(po), _slices(yo)
+    from .pdist import parse_key
+
+    def key(k):
+        """the prior key that holds model key k: k itself or a distribution key f(k) (its code: _lsqfit_hook)"""
+        if k in ps:
+            return k
+        return next((kk for kk in ps if parse_key(kk)[0] is not None and parse_key(kk)[1] == k), k)
+
     def idx(s):
         return np.arange(s.start, s.stop) if isinstance(s, slice) else np.atleast_1d(np.asarray(s))
-    E = idx(ps[models[0].E])
+    if any(key(k) not in ps for k in [models[0].E] + [m.a for m in models]):
+        return None
+    E = idx(ps[key(models[0].E)])
     K = E.size
-    amps = [idx(ps[m.a]) for m in models]
+    amps = [idx(ps[key(m.a)]) for m in models]
     if any(a.size != K for a in amps) or sum(a.size for a in amps) + K != sum(idx(s).size for s in ps.values()):
         return None                                          # parameters the models do not use: no device mapping
     by_tag = dict((m.datatag, (i, m)) for i, m in enumerate(models))
