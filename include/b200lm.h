@@ -221,6 +221,20 @@ int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub);
  * bounds) and b200lm_set_policy(1) are refused in the same way while distributions are set.  Transforms on the team and
  * wave kernels, windows, fit sets, bounds and the GSL policy are not built. */
 int b200lm_set_param_dist(b200lm_handle h, const int* h_code, const double* h_lo, const double* h_hi);
+/* robust loss of the following b200lm_fit_batch / b200lm_fit_batch_host calls on this handle: scipy's least_squares
+ * loss= / f_scale= (lsqfit.scipy_least_squares(loss=..., f_scale=...)).  code 0 = linear (clears the setting: today's
+ * kernels, bit for bit), 1 = huber, 2 = soft_l1, 3 = cauchy, 4 = arctan; one loss and one f_scale C for every fit of a
+ * batch.  Each fit follows scipy's trf_no_bounds with a loss function, in the one-warp kernel fit_kernel<F, 6>: the cost
+ * is 1/2 C^2 sum rho((f_i / C)^2) over every chiv row (data, prior and whitened block rows), and every row enters the
+ * trust-region loop rescaled as in scipy's scale_for_robust_loss_function.  Outputs: x, nit (nfev) and status as
+ * without a loss; cov from the rescaled normal matrix at the solution (scipy's fit.jac); chi2, f, J and log det from
+ * the TRUE residuals and Jacobian at the solution.  Polish is skipped; team and wave requests are overridden
+ * (b200lm_last_team reports 1).  B200LM_EINVAL, with a message, for an unknown code; for f_scale not finite or not > 0;
+ * on a handle with windows or nslot > 1, with finite bounds, with parameter distributions or with the GSL policy.
+ * b200lm_set_windows, b200lm_set_bounds (finite bounds), b200lm_set_param_dist (any nonzero code) and
+ * b200lm_set_policy(1) are refused in the same way while a loss is set.  b200lm_residual_jacobian and
+ * b200lm_propagate do not see the loss: they keep returning the true chiv and J. */
+int b200lm_set_loss(b200lm_handle h, int code, double f_scale);
 /* number of kernel launches issued through this handle so far */
 long long b200lm_launch_count(b200lm_handle h);
 

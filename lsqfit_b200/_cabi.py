@@ -75,6 +75,7 @@ SIGNATURES = {
     "b200lm_set_policy": (C.c_int, [handle_t, C.c_int]),
     "b200lm_set_bounds": (C.c_int, [handle_t, C.c_void_p, C.c_void_p]),
     "b200lm_set_param_dist": (C.c_int, [handle_t, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b200lm_set_loss": (C.c_int, [handle_t, C.c_int, C.c_double]),
     "b200lm_launch_count": (C.c_longlong, [handle_t]),
     "b200lm_residual_jacobian": (C.c_int, [handle_t, C.c_int, C.c_void_p, C.c_longlong, C.c_void_p,
                                            C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

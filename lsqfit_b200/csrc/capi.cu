@@ -48,6 +48,7 @@ void fill_params(b200lm_handle_s* h, FitParams& P) {
     P.stats = h->d_stats;
     P.policy = h->policy;
     if (h->ntrans > 0) { P.ntrans = h->ntrans; P.pd_code = h->d_pd_code; P.pd_lo = h->d_pd_lo; P.pd_hi = h->d_pd_hi; }
+    if (h->loss > 0) { P.loss = h->loss; P.f_scale = h->f_scale; }
 }
 }  // namespace b200lm
 
@@ -195,11 +196,11 @@ static bool wave_ok(b200lm_handle_s* h) {
 }
 
 // The warps per fit of a batch: 1 (fit_kernel), 2 or 4 (fit_team_kernel) or 32 (the wave kernel).  Windows run in
-// the one-warp kernel (fit_kernel<F, 4>), and so do the GSL decisions and the bounded scipy decisions (fit_kernel<F, 1>
-// and <F, 3>).  Otherwise B200LM_TEAM = 0/1, 2, 4, 32 overrides default_team, and a team that the functor or the
+// the one-warp kernel (fit_kernel<F, 4>), and so do the GSL decisions, the bounded scipy decisions, parameter
+// distributions and a robust loss (fit_kernel<F, 1>, <F, 3>, <F, 5>, <F, 6>).  Otherwise B200LM_TEAM = 0/1, 2, 4, 32 overrides default_team, and a team that the functor or the
 // shapes do not allow falls back to one warp.
 static int kernel_team(b200lm_handle_s* h) {
-    if (h->nwin > 0 || h->policy == 1 || h->bounded || h->ntrans > 0) return 1;
+    if (h->nwin > 0 || h->policy == 1 || h->bounded || h->ntrans > 0 || h->loss > 0) return 1;
     int team = default_team(h);
     if (const char* env = getenv("B200LM_TEAM")) team = atoi(env);
     if (team == 32) return wave_ok(h) ? 32 : 1;
@@ -489,6 +490,7 @@ int b200lm_set_windows(b200lm_handle h, int nwin, const int* ndiag, const int* d
     if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
     if (nwin < 1 || !ndiag || !nblk) return set_error(h, B200LM_EINVAL, "bad window description");
     if (h->ntrans > 0) return set_error(h, B200LM_EINVAL, "parameter distributions are not built for window scans");
+    if (h->loss > 0) return set_error(h, B200LM_EINVAL, "a robust loss is not built for window scans");
     CUDA_TRY(h, cudaSetDevice(h->device), "cudaSetDevice");
     // a window lists every prior entry and its own data rows exactly once; in a fit set, every entry of one slot
     // (checked below) and its own data rows
@@ -712,6 +714,7 @@ int b200lm_set_bounds(b200lm_handle h, const double* h_lb, const double* h_ub) {
     }
     if (finite && h->ntrans > 0)
         return set_error(h, B200LM_EINVAL, "bounds are not built for fits with parameter distributions");
+    if (finite && h->loss > 0) return set_error(h, B200LM_EINVAL, "bounds are not built for fits with a robust loss");
     if (!finite) {                               // no bounds, or all infinite: scipy's unbounded trf
         h->bounded = false;
         h->h_lb.clear(); h->h_ub.clear();
@@ -730,6 +733,8 @@ int b200lm_set_policy(b200lm_handle h, int policy) {
     if (policy != 0 && policy != 1) return set_error(h, B200LM_EINVAL, "policy must be 0 (scipy trf) or 1 (gsl lm)");
     if (policy == 1 && h->ntrans > 0)
         return set_error(h, B200LM_EINVAL, "the GSL policy is not built for fits with parameter distributions");
+    if (policy == 1 && h->loss > 0)
+        return set_error(h, B200LM_EINVAL, "the GSL policy is not built for fits with a robust loss");
     h->policy = policy;
     return B200LM_OK;
 }
@@ -759,6 +764,8 @@ int b200lm_set_param_dist(b200lm_handle h, const int* h_code, const double* h_lo
     if (h->policy == 1)
         return set_error(h, B200LM_EINVAL, "the GSL policy is not built for fits with parameter distributions");
     if (n == 0) { h->ntrans = 0; return B200LM_OK; }        // all plain: today's kernels
+    if (h->loss > 0)
+        return set_error(h, B200LM_EINVAL, "parameter distributions are not built for fits with a robust loss");
     std::vector<double> lo(h->np, 0.0), hi(h->np, 1.0);
     for (int j = 0; j < h->np; ++j)
         if (h_code[j] == 3) { lo[j] = h_lo[j]; hi[j] = h_hi[j]; }
@@ -768,6 +775,25 @@ int b200lm_set_param_dist(b200lm_handle h, const int* h_code, const double* h_lo
     CUDA_TRY(h, upload(&h->d_pd_lo, lo.data(), lo.size()), "upload distribution codes");
     CUDA_TRY(h, upload(&h->d_pd_hi, hi.data(), hi.size()), "upload distribution codes");
     h->ntrans = n;
+    return B200LM_OK;
+}
+
+int b200lm_set_loss(b200lm_handle h, int code, double f_scale) {
+    if (!h) return set_error(h, B200LM_EINVAL, "NULL handle");
+    if (code < 0 || code > 4)
+        return set_error(h, B200LM_EINVAL, "unknown loss code " + std::to_string(code) +
+                                           " (0 linear, 1 huber, 2 soft_l1, 3 cauchy, 4 arctan)");
+    if (code == 0) { h->loss = 0; h->f_scale = 1.0; return B200LM_OK; }
+    if (!std::isfinite(f_scale) || !(f_scale > 0.0))
+        return set_error(h, B200LM_EINVAL, "f_scale must be finite and > 0");
+    if (h->nwin > 0 || h->nslot > 1)
+        return set_error(h, B200LM_EINVAL, "a robust loss is not built for window scans or fit sets");
+    if (h->bounded) return set_error(h, B200LM_EINVAL, "bounds are not built for fits with a robust loss");
+    if (h->ntrans > 0)
+        return set_error(h, B200LM_EINVAL, "parameter distributions are not built for fits with a robust loss");
+    if (h->policy == 1) return set_error(h, B200LM_EINVAL, "the GSL policy is not built for fits with a robust loss");
+    h->loss = code;
+    h->f_scale = f_scale;
     return B200LM_OK;
 }
 

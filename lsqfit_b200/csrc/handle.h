@@ -69,6 +69,9 @@ struct b200lm_handle_s {
     // parameter distributions (b200lm_set_param_dist): ntrans = entries with a nonzero code; 0 = none set
     int ntrans = 0;
     int* d_pd_code = nullptr; double* d_pd_lo = nullptr; double* d_pd_hi = nullptr;
+    // robust loss (b200lm_set_loss): scipy's loss code (0 = none) and f_scale
+    int loss = 0;
+    double f_scale = 1.0;
     // queue order (longest-expected fits first): key = chi2 at the start point, one evaluation per fit
     int order_request = -1;     // -1: default policy (by problem shape and batch size); 0: off; 1: on  (b200lm_set_order)
     int last_order = 0;         // 1 if the last fit_batch launch used an ordered queue

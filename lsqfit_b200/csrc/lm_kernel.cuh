@@ -282,11 +282,67 @@ __device__ __forceinline__ void qr_update(double* A, const double* dsc, double* 
     }
 }
 
-// rows of the buffer are finished [J | r]: emit / fold them into the normal equations or the QR factor
-template <class F, int MODE>
+// scipy's robust losses (least_squares loss= / f_scale=, P.loss codes as lsqfit_b200.dense.LOSSES), one residual r at a
+// time: z = (r / C)^2 (divide, then square, as construct_loss_function does), rho, rho', rho'' of the loss, and the row
+// scale of scale_for_robust_loss_function, s = sqrt(max(rho' + 2 rho'' r^2 / C^2, EPS)): the row [J | r] becomes
+// [s J | r rho' / s].  Returns C^2 rho(z), the row's share of twice the robust cost.  `loss` is warp-uniform.
+__device__ __forceinline__ double robust_row(int loss, double C, double r, double& s, double& rs) {
+    const double u = r / C;
+    const double z = u * u;
+    double rho0, rho1, rho2;
+    switch (loss) {
+    case 1:                                                  // huber
+        if (z <= 1.0) {
+            rho0 = z; rho1 = 1.0; rho2 = 0.0;
+        } else {
+            const double sz = sqrt(z);
+            rho0 = 2.0 * sz - 1.0; rho1 = 1.0 / sz; rho2 = -0.5 * rho1 / z;
+        }
+        break;
+    case 2: {                                                // soft_l1
+        const double t = 1.0 + z, st = sqrt(t);
+        rho0 = 2.0 * (st - 1.0); rho1 = 1.0 / st; rho2 = -0.5 * rho1 / t;
+        break;
+    }
+    case 3: {                                                // cauchy
+        rho0 = log1p(z); rho1 = 1.0 / (1.0 + z); rho2 = -rho1 * rho1;
+        break;
+    }
+    case 4: {                                                // arctan
+        rho0 = atan(z); rho1 = 1.0 / fma(z, z, 1.0); rho2 = -2.0 * z * rho1 * rho1;
+        break;
+    }
+    default:
+        rho0 = z; rho1 = 1.0; rho2 = 0.0;
+    }
+    const double C2 = C * C;
+    double js = rho1 + 2.0 * (rho2 / C2) * (r * r);
+    // scipy clips J_scale < EPS to EPS; for cauchy and arctan that is every row with z > 1 (rho' + 2 z rho'' < 0)
+    if (js < 2.220446049250313e-16) js = 2.220446049250313e-16;
+    s = sqrt(js);
+    rs = r * (rho1 / s);
+    return C2 * rho0;
+}
+
+// rows of the buffer are finished [J | r]: emit / fold them into the normal equations or the QR factor.
+// ROBUST (fit_kernel<F, 6>): after the (true) rows are emitted, each is rescaled by the loss (robust_row) and its
+// C^2 rho is added to `rcost`; without it, rcost is untouched.
+template <class F, int MODE, bool ROBUST = false>
 __device__ __forceinline__ void consume_rows(WarpCtx<F>& c, int nrows, int slot0, double* fout, double* Jout,
-                                             NormalAcc<F>& na) {
+                                             NormalAcc<F>& na, double& rcost) {
     if (fout || Jout) emit_rows<F>(c.R, nrows, slot0, c.lane, fout, Jout);
+    if constexpr (ROBUST) {
+        constexpr int NP = FitLayout<F>::NP;
+        if (c.lane < nrows) {
+            double* row = c.R + c.lane * FitLayout<F>::LDR;
+            double s, rs;
+            rcost += robust_row(c.P.loss, c.P.f_scale, row[NP], s, rs);
+#pragma unroll
+            for (int j = 0; j < NP; ++j) row[j] *= s;
+            row[NP] = rs;
+        }
+        __syncwarp();
+    }
     if (MODE == 0) {
         mma_accumulate<F>(c, c.R, (nrows + 3) & ~3, na);
     } else {
@@ -320,7 +376,9 @@ __device__ __forceinline__ int prior_base(const WinRows& T) { return T.pr_base; 
 // one window (WinRows)
 // TRANS (parameter distributions, fit_kernel<F, 5>): the data rows see the model at qv = T(pv), and their Jacobian
 // columns are scaled by tp = T'(pv); the prior rows stay in pv
-template <class F, int MODE, bool WSMEM, class RS, bool TRANS = false>
+// ROBUST (robust loss, fit_kernel<F, 6>): every row is rescaled by the loss before it enters A / g or the QR factor,
+// and the returned cost is 1/2 sum C^2 rho; emitted rows (fout, Jout) are the true ones
+template <class F, int MODE, bool WSMEM, class RS, bool TRANS = false, bool ROBUST = false>
 __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const double* pv, double* fout, double* Jout,
                                             const double* qv = nullptr, const double* tp = nullptr) {
     typedef FitLayout<F> Lay;
@@ -341,13 +399,19 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
         const int j = idx - prior_base(T);
         const double w = T.dpr_w[i];
         const double r = w * (pv[j] - c.mean[idx]);
-        if (MODE == 0) {
-            c.A[j * LDA + j] += w * w;
-            c.g[j] += w * r;
-        } else {
-            c.A[j * LDA + j] = w * c.dsc[j];                 // a diagonal matrix is triangular
+        double ws = w, rs = r;                               // the row as it enters A / g (ROBUST: rescaled)
+        if constexpr (ROBUST) {
+            double s;
+            acc += robust_row(P.loss, P.f_scale, r, s, rs);
+            ws = s * w;
         }
-        acc = fma(r, r, acc);
+        if (MODE == 0) {
+            c.A[j * LDA + j] += ws * ws;
+            c.g[j] += ws * rs;
+        } else {
+            c.A[j * LDA + j] = ws * c.dsc[j];                // a diagonal matrix is triangular
+        }
+        if constexpr (!ROBUST) acc = fma(r, r, acc);
         if (fout) fout[T.nd_fn + i] = r;
         if (Jout) {
             for (int q = 0; q < NP; ++q) Jout[(size_t)(T.nd_fn + i) * NP + q] = (q == j) ? w : 0.0;
@@ -374,7 +438,7 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
             for (int j = 0; j < NCOL; ++j) row_[j] = 0.0;
         }
         __syncwarp();
-        consume_rows<F, MODE>(c, nrows, c0, fout, Jout, na);
+        consume_rows<F, MODE, ROBUST>(c, nrows, c0, fout, Jout, na, acc);
     }
     // correlated blocks: J_blk = W.[G | delta] on the FP64 tensor path.  The C fragments of a
     // 64-row output group stay in registers while the input rows stream through the row buffer
@@ -473,7 +537,7 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
                         if (m4 < mt_here && (lane & 3) == 0) c.R[(8 * m4 + (lane >> 2)) * LDR + NP] = pr[m4][0];
                 }
                 __syncwarp();
-                consume_rows<F, MODE>(c, nrows, bd.chiv_off + g0 + 32 * half, fout, Jout, na);
+                consume_rows<F, MODE, ROBUST>(c, nrows, bd.chiv_off + g0 + 32 * half, fout, Jout, na, acc);
 #pragma unroll
                 for (int m4 = 0; m4 < 4; ++m4) {
 #pragma unroll
@@ -483,7 +547,10 @@ __device__ __forceinline__ double eval_rows(WarpCtx<F>& c, const RS& T, const do
             }
         }
     }
-    if (MODE == 0) acc += flush_normal<F>(c, na);
+    if (MODE == 0) {
+        const double rr = flush_normal<F>(c, na);
+        if constexpr (!ROBUST) acc += rr;                   // ROBUST: r^T r of the rescaled rows is not the cost
+    }
     return 0.5 * warp_sum(acc);
 }
 
@@ -574,6 +641,19 @@ __device__ __noinline__ double eval_trans_impl(const WarpCtx<F>& c_in, double* q
     }
     __syncwarp();
     return eval_rows<F, MODE, WSMEM, FitParams, true>(c, P, pv, fout, Jout, qt, qt + NP);
+}
+
+// evaluation with a robust loss (fit_kernel<F, 6>): the rows of eval_full, rescaled by the loss; returns the robust cost
+template <class F, int MODE, bool WSMEM>
+__device__ __noinline__ double eval_robust_impl(const WarpCtx<F>& c_in, const double* pv, double* fout, double* Jout) {
+    WarpCtx<F> c = c_in;
+    __builtin_assume(__isShared(c.R));
+    __builtin_assume(__isShared(c.dvec));
+    __builtin_assume(__isShared(c.A));
+    __builtin_assume(__isShared(c.g));
+    __builtin_assume(__isShared(c.dsc));
+    __builtin_assume(__isShared(pv));
+    return eval_rows<F, MODE, WSMEM, FitParams, false, true>(c, c.P, pv, fout, Jout);
 }
 
 // ---------------------------------------------------------------------------
@@ -1276,6 +1356,34 @@ __device__ __forceinline__ void setup_ctx(WarpCtx<F>& c, double* smem, const Fit
     __syncthreads();
 }
 
+// Robust loss (fit_kernel<F, 6>): the covariance of the rescaled normal matrix in c.A at the solution, by the rule of
+// fit_one's results block -- columns scaled by their norms; the Cholesky factor when well conditioned, else the QR
+// pass over the rescaled rows (EV::run mode 1); NaN at a non-finite point.  fit_one then evaluates the true rows.
+template <class F, class EV>
+__device__ __forceinline__ void robust_covariance(WarpCtx<F>& c, bool finite, double* cov_out, int& nfac, int& njev,
+                                                  EV& ev) {
+    constexpr int NP = FitLayout<F>::NP, LDA = FitLayout<F>::LDA;
+    const int lane = c.lane;
+    const bool act = lane < NP;
+    if (act) {
+        const double s = sqrt(c.A[lane * LDA + lane]);
+        c.dsc[lane] = s > 0.0 ? 1.0 / s : 1.0;
+    }
+    __syncwarp();
+    ++nfac;
+    double pdummy, fres[3];
+    const bool okc = factor_solve<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, 0.0, 0.0, true, &pdummy, fres);
+    if (okc && fres[2] > 1e-6) {
+        covariance_from_chol<F>(c, cov_out);
+    } else if (finite) {
+        ev.run(c, c.p, nullptr, nullptr, 1);
+        ++njev;
+        covariance_from_qr<F>(c, cov_out);
+    } else if (cov_out && act) {
+        for (int j = 0; j < NP; ++j) cov_out[lane * NP + j] = nan("");
+    }
+}
+
 // Evaluator of the one-warp-per-fit kernel: the warp evaluates all rows itself.
 template <class F>
 struct WarpEval {
@@ -1321,7 +1429,22 @@ struct TransEval {
     }
 };
 
+// Evaluator of the robust-loss kernel (fit_kernel<F, 6>): as WarpEval, with every row rescaled by the loss and the
+// robust cost returned (eval_robust_impl).  The true rows at the solution come from eval_full (fit_one, MODE 6).
+template <class F>
+struct RobustEval {
+    __device__ __forceinline__ const double* begin(WarpCtx<F>&, const FitParams& P, int b) {
+        return P.mean + (size_t)b * P.mean_stride;
+    }
+    __device__ __forceinline__ double run(WarpCtx<F>& c, const double* pv, double* fout, double* Jout, int mode) {
+        if (c.P.wt_in_smem)
+            return mode == 0 ? eval_robust_impl<F, 0, true>(c, pv, fout, Jout) : eval_robust_impl<F, 1, true>(c, pv, fout, Jout);
+        return mode == 0 ? eval_robust_impl<F, 0, false>(c, pv, fout, Jout) : eval_robust_impl<F, 1, false>(c, pv, fout, Jout);
+    }
+};
+
 template <class F, int MODE> struct EvalOf { typedef WarpEval<F> type; static constexpr int EXTRA = 0; };
+template <class F> struct EvalOf<F, 6> { typedef RobustEval<F> type; static constexpr int EXTRA = 0; };
 template <class F> struct EvalOf<F, 4> { typedef WinEval<F> type; static constexpr int EXTRA = 0; };
 template <class F> struct EvalOf<F, 5> { typedef TransEval<F> type; static constexpr int EXTRA = TransEval<F>::EXTRA; };
 
@@ -1342,7 +1465,9 @@ struct PhaseClock {
 // 3 = scipy TRF with bound constraints (trf_bounds: Coleman-Li scaling, select_step; b200lm_set_bounds),
 // 4 = scipy TRF on fit windows (the loop of MODE 0; EV = WinEval: rows, weights and means per window, b200lm_set_windows),
 // 5 = scipy TRF with parameter distributions (the loop of MODE 0; EV = TransEval: the model at q = T(p),
-// b200lm_set_param_dist).
+// b200lm_set_param_dist),
+// 6 = scipy TRF with a robust loss (trf_no_bounds with loss_function: the loop of MODE 0 on the rows rescaled by the
+// loss and the robust cost, EV = RobustEval; no polish; b200lm_set_loss).
 template <class F, class EV, int MODE = 0>
 __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& P, int b,
                                         unsigned long long& tot_nfev, unsigned long long& tot_njev,
@@ -1505,7 +1630,7 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
 
         // MODE 3 (bounds) is the same loop with scipy's trf_bounds changes: the gtol test on |g v|_inf, the scaling
         // d = sqrt(v) / scale_inv, the Coleman-Li diagonal in the sub-problem, select_step, strictly feasible trials
-        while ((MODE == 0 || MODE == 3 || MODE == 4 || MODE == 5) && status == -2) {
+        while ((MODE == 0 || MODE == 3 || MODE == 4 || MODE == 5 || MODE == 6) && status == -2) {
             const double gi = act ? c.g[lane] : 0.0;
             double v = 1.0, dv = 0.0;                              // Coleman-Li scaling (MODE 3)
             const double xi = act ? c.p[lane] : 0.0;
@@ -1652,8 +1777,8 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
         // from the stationary point (so does the reference's solver).  Undamped Gauss-Newton
         // steps, accepted on the decrease of the Newton decrement instead of the cost, take the
         // solution on to the gradient's rounding level.
-        // (not with bounds: undamped steps would leave the box)
-        if (MODE != 3 && status >= 1 && P.polish > 0) {
+        // (not with bounds: undamped steps would leave the box; not with a loss, as on the single-fit path)
+        if (MODE != 3 && MODE != 6 && status >= 1 && P.polish > 0) {
             // Newton decrement dec = g^T (J^T J)^-1 g = predicted decrease of chi2; sqrt(dec) is
             // the distance to the stationary point in standard deviations.
             const double d = 1.0 / sinv;
@@ -1694,11 +1819,19 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
         }
 
         // ---- results -----------------------------------------------------------
-        if (P.f_out || P.J_out) {
+        if constexpr (MODE == 6) {
+            // robust loss: cov from the rescaled normal matrix of the solution (scipy's fit.jac); then the true rows at
+            // the solution: f / J, chi2 and the J^T J whose log det the block below takes
+            robust_covariance<F>(c, isfinite(cost), P.cov ? P.cov + (size_t)b * NP * NP : nullptr, nfac, njev, ev);
+            cost = eval_full<F, 0>(c, c.p, P.f_out ? P.f_out + (size_t)b * P.nchiv : nullptr,
+                                   P.J_out ? P.J_out + (size_t)b * P.nchiv * NP : nullptr);
+            ++njev;
+        } else if (P.f_out || P.J_out) {
             cost = ev.run(c, c.p, P.f_out ? P.f_out + (size_t)b * P.nchiv : nullptr,
                           P.J_out ? P.J_out + (size_t)b * P.nchiv * NP : nullptr, 0);
         }
-        // covariance at the solution, scaled by the current column norms for conditioning
+        // covariance at the solution, scaled by the current column norms for conditioning (MODE 6: the log det of the
+        // true J^T J only, its QR pass on the true rows)
         double dfin = 1.0;
         if (act) {
             const double s = sqrt(c.A[lane * LDA + lane]);
@@ -1710,14 +1843,15 @@ __device__ __forceinline__ void fit_one(WarpCtx<F>& c, EV& ev, const FitParams& 
         double pdummy, fres[3];
         const bool okc = factor_solve<NP, LDA>(c.A, c.dsc, c.L, c.idg, c.colb, lane, 0.0, 0.0, true, &pdummy, fres);
         const double pivr = fres[2];
-        double* cov_out = P.cov ? P.cov + (size_t)b * NP * NP : nullptr;
+        double* cov_out = (MODE != 6 && P.cov) ? P.cov + (size_t)b * NP * NP : nullptr;
         double ld = nan("");
         if (okc && pivr > 1e-6) {
             // well conditioned: kappa^2 * eps < ~2e-10, the normal-equation factor is accurate enough
             ld = covariance_from_chol<F>(c, cov_out);
         } else if (isfinite(cost)) {
             // ill conditioned: one more pass over the rows, Householder QR of J.diag(dsc)
-            ev.run(c, c.p, nullptr, nullptr, 1);
+            if constexpr (MODE == 6) eval_full<F, 1>(c, c.p, nullptr, nullptr);
+            else ev.run(c, c.p, nullptr, nullptr, 1);
             ++njev;
             ld = covariance_from_qr<F>(c, cov_out);
         } else if (cov_out && act) {
@@ -1873,6 +2007,9 @@ cudaError_t launch_fit(FitParams P, int sm_count, size_t smem_budget, cudaStream
     cudaError_t e = plan_launch<F>(P, sm_count, smem_budget, li, trans ? EvalOf<F, 5>::EXTRA : 0);
     if (e != cudaSuccess) return e;
     if (trans) return launch_fit_mode<F, 5>(P, li, stream);
+    // a robust loss: b200lm_set_loss refuses windows, bounds, distributions and the GSL policy, and the batch runs
+    // one warp per fit (no wave kernel, so no finalize_only)
+    if (P.loss > 0) return launch_fit_mode<F, 6>(P, li, stream);
     if (P.nwin > 0) return launch_fit_mode<F, 4>(P, li, stream);
     if (P.finalize_only) return launch_fit_mode<F, 2>(P, li, stream);
     if (P.bounded) return launch_fit_mode<F, 3>(P, li, stream);

@@ -100,6 +100,9 @@ struct FitParams {
                                 //      3 uniform: q = lo + (hi - lo) (1 + erf(p / sqrt 2)) / 2
     const double* pd_lo;        // [np] lo and hi of code 3
     const double* pd_hi;
+    // ---- robust loss (last, for the same reason; b200lm_set_loss) ----
+    int loss;                   // scipy's loss: 0 linear (none), 1 huber, 2 soft_l1, 3 cauchy, 4 arctan (fit_kernel<F, 6>)
+    double f_scale;             // scipy's f_scale C: the cost is 1/2 C^2 sum rho((f / C)^2) over every chiv row
 };
 
 }  // namespace b200lm

@@ -180,24 +180,50 @@ class Plan(object):
             raise ValueError("Each lower bound must be strictly less than each upper bound.")     # scipy least_squares
         return lb, ub
 
-    def _launch_bounded(self, bounds, launch):
-        """Run ``launch()`` with the box set on the handle (b200lm_set_bounds); the plan is cached and shared (the
-        parent fit, other drivers), so the bounds are cleared again afterwards."""
-        if bounds is None:
+    @staticmethod
+    def _loss(loss, f_scale, bounds, policy):
+        """scipy's loss= / f_scale= -> (code of lsqfit_b200.dense.LOSSES, f_scale), or None for 'linear'."""
+        from .dense import LOSSES
+        if loss not in LOSSES:
+            raise ValueError("`loss` must be one of %s" % (LOSSES,))
+        if loss == "linear":
+            return None
+        f_scale = float(f_scale)
+        if not (np.isfinite(f_scale) and f_scale > 0):
+            raise ValueError("f_scale must be finite and > 0")
+        if bounds is not None:
+            raise ValueError("a robust loss together with bounds is not built for batched fits")
+        if POLICY[policy] == 1:
+            raise ValueError("a robust loss is not built for the GSL policy (policy='gsl')")
+        return LOSSES.index(loss), f_scale
+
+    def _launch_with(self, bounds, loss, launch):
+        """Run ``launch()`` with the box (b200lm_set_bounds) and the robust loss (b200lm_set_loss) set on the handle;
+        the plan is cached and shared (the parent fit, other drivers), so both are cleared again afterwards."""
+        if bounds is None and loss is None:
             return launch()
-        lb, ub = bounds
-        _cabi.check(_cabi.lib.b200lm_set_bounds(self._h, lb.ctypes.data, ub.ctypes.data), self._h)
         try:
+            if bounds is not None:
+                lb, ub = bounds
+                _cabi.check(_cabi.lib.b200lm_set_bounds(self._h, lb.ctypes.data, ub.ctypes.data), self._h)
+            if loss is not None:
+                _cabi.check(_cabi.lib.b200lm_set_loss(self._h, loss[0], loss[1]), self._h)
             return launch()
         finally:
-            _cabi.lib.b200lm_set_bounds(self._h, None, None)
+            if loss is not None:
+                _cabi.lib.b200lm_set_loss(self._h, 0, 1.0)
+            if bounds is not None:
+                _cabi.lib.b200lm_set_bounds(self._h, None, None)
 
-    def _prepare(self, mean, sm, p0, sp, tol, maxit, scaler, polish, policy, bounds, want_cov, want_fJ, B=None):
+    def _prepare(self, mean, sm, p0, sp, tol, maxit, scaler, polish, policy, bounds, want_cov, want_fJ, B=None,
+                 loss="linear", f_scale=1.0):
         """What both launch entries check and compute.  mean [rows, N] (sm = N) or [N] (sm = 0), p0 likewise; with
         windows a row of means per copy and a start per window.  -> (B, solver arguments of the C entry, bounds as
-        two host arrays or None, shape and dtype of every output asked for, None for the others)."""
+        two host arrays or None, the loss as (code, f_scale) or None, shape and dtype of every output asked for, None
+        for the others)."""
         xtol, gtol, ftol = normalize_tol(tol)
         sc = self._set_policy(policy, scaler)
+        loss = self._loss(loss, f_scale, bounds, policy)
         if B is None:
             B = ((mean.shape[0] if sm else 1) * self.nwin if self.nwin else
                  (mean.shape[0] if sm else (p0.shape[0] if sp else 1)))
@@ -214,25 +240,29 @@ class Plan(object):
         shapes = dict(x=((B, self.np), f8), chi2=(B, f8), cov=((B, self.np, self.np), f8) if want_cov else None,
                       logdet=(B, f8), nit=(B, i4), status=(B, i4), f=((B, self.nchiv), f8) if want_fJ else None,
                       J=((B, self.nchiv, self.np), f8) if want_fJ else None)
-        return B, (xtol, gtol, ftol, int(maxit), sc, int(polish)), bounds, shapes
+        return B, (xtol, gtol, ftol, int(maxit), sc, int(polish)), bounds, loss, shapes
 
     def fit_batch(self, mean, p0, tol=1e-8, maxit=1000, scaler="more", B=None,
-                  want_cov=True, want_fJ=False, out=None, polish=0, policy="trf", bounds=None):
+                  want_cov=True, want_fJ=False, out=None, polish=0, policy="trf", bounds=None,
+                  loss="linear", f_scale=1.0):
         """Fit B problems on the device; inputs may be numpy arrays or device tensors.
 
         mean: [B, N] or [N] (shared);  p0: [B, np] or [np] (shared).
         bounds: None or (lb, ub) in device parameter order, scipy's ``bounds`` (±inf: none); p0 must lie in the box.
+        loss, f_scale: scipy's robust loss ('linear' | 'huber' | 'soft_l1' | 'cauchy' | 'arctan') for every fit of the
+        batch (b200lm_set_loss: cov from the rescaled rows, chi2 / f / J / logdet from the true ones; no polish; one
+        warp per fit).  Not with bounds or policy='gsl'.
         Returns a BatchResult of device tensors (no host synchronisation)."""
         tm, sm = self._dev(mean, self.N)
         tp, sp = self._dev(p0, self.np)
-        B, solver, bounds, shapes = self._prepare(tm, sm, tp, sp, tol, maxit, scaler, polish, policy, bounds,
-                                                  want_cov, want_fJ, B)
+        B, solver, bounds, loss, shapes = self._prepare(tm, sm, tp, sp, tol, maxit, scaler, polish, policy, bounds,
+                                                        want_cov, want_fJ, B, loss, f_scale)
         if out is None:
             out = BatchResult(*[s and torch.empty(s[0], device=self.tdev,
                                                   dtype=torch.int32 if s[1] is np.int32 else torch.float64)
                                 for s in shapes.values()])
         ptr = lambda t: t.data_ptr() if t is not None else None
-        self._launch_bounded(bounds, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch(
+        self._launch_with(bounds, loss, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch(
             self._h, B, tm.data_ptr(), sm, tp.data_ptr(), sp, *solver,
             out.x.data_ptr(), out.chi2.data_ptr(), ptr(out.cov), out.logdet.data_ptr(),
             out.nit.data_ptr(), out.status.data_ptr(), ptr(out.f), ptr(out.J), self._stream()), self._h))
@@ -240,10 +270,10 @@ class Plan(object):
         return out
 
     def fit_batch_host(self, mean, p0, tol=1e-8, maxit=1000, scaler="more", want_cov=True,
-                       want_fJ=False, out=None, polish=0, policy="trf", bounds=None):
+                       want_fJ=False, out=None, polish=0, policy="trf", bounds=None, loss="linear", f_scale=1.0):
         """Same fit through the host-buffer C entry point: numpy in, numpy out.
         ``out`` may hold preallocated arrays (dict with keys x, chi2, cov, logdet, nit, status).
-        ``bounds`` as for fit_batch."""
+        ``bounds``, ``loss`` and ``f_scale`` as for fit_batch."""
         # the C entry point reads raw host pointers: dtype, contiguity and shapes are checked HERE
         # (np.ascontiguousarray is a no-op for conforming arrays)
         mean = np.ascontiguousarray(mean, dtype=np.float64)
@@ -255,8 +285,9 @@ class Plan(object):
         sm = 0 if mean.ndim == 1 else self.N
         sp = 0 if p0.ndim == 1 else self.np
         # every array of a given ``out`` is checked
-        B, solver, bounds, shapes = self._prepare(mean, sm, p0, sp, tol, maxit, scaler, polish, policy, bounds,
-                                                  want_cov or out is not None, want_fJ or out is not None)
+        B, solver, bounds, loss, shapes = self._prepare(mean, sm, p0, sp, tol, maxit, scaler, polish, policy, bounds,
+                                                        want_cov or out is not None, want_fJ or out is not None,
+                                                        loss=loss, f_scale=f_scale)
         if out is None:
             out = dict((k, s and np.empty(*s)) for k, s in shapes.items())
         else:
@@ -273,7 +304,7 @@ class Plan(object):
                     raise ValueError("out[%r] must be a writable C-contiguous %s array of shape %s"
                                      % (k, np.dtype(dt).name, shp))
         ptr = lambda a: a.ctypes.data if a is not None else None
-        self._launch_bounded(bounds, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch_host(
+        self._launch_with(bounds, loss, lambda: _cabi.check(_cabi.lib.b200lm_fit_batch_host(
             self._h, B, mean.ctypes.data, sm, p0.ctypes.data, sp, *solver,
             ptr(out["x"]), ptr(out["chi2"]), ptr(out.get("cov")), ptr(out["logdet"]),
             ptr(out["nit"]), ptr(out["status"]), ptr(out.get("f")), ptr(out.get("J"))), self._h))

@@ -215,9 +215,11 @@ class nonlinear_fit(object):
     def _batch_args(self, kargs):
         """This fit's fitter arguments with ``kargs`` over them, as the batch drivers read them -> (the arguments of
         ``Plan.fit_batch``, kernel, loss, gsl).  tol and maxit default to this fit's; scipy's bounds=(lower, upper)
-        in this fit's parameter order go to device order (as the single-fit path does).  kernel=: None (default, by
-        problem shape), 1 / 2 / 4 warps per fit, or 32 / 'wave' -- the wave kernel, the fastest on saturated batches
-        (10^5 ... 10^6 copies of a small model); see b200lm_set_team."""
+        in this fit's parameter order go to device order (as the single-fit path does); this fit's scipy loss= /
+        f_scale= go to every copy (_batch refuses another one).  With a loss, kernel= is accepted and has no effect
+        (robust batches run one warp per fit).  kernel=: None (default, by problem shape), 1 / 2 / 4 warps per fit,
+        or 32 / 'wave' -- the wave kernel, the fastest on saturated batches (10^5 ... 10^6 copies of a small model);
+        see b200lm_set_team."""
         from .engine import POLICY
         args = dict(self.fitterargs, **kargs)
         bounds = args.get("bounds")
@@ -227,7 +229,7 @@ class nonlinear_fit(object):
         fit = dict(tol=self.tol if args.get("tol") is None else args["tol"],
                    maxit=self.maxit if args.get("maxit") is None else args["maxit"],
                    scaler=args.get("scaler", "more"), polish=args.get("polish", 0), policy=args.get("policy", "trf"),
-                   bounds=bounds)
+                   bounds=bounds, loss=args.get("loss", "linear"), f_scale=args.get("f_scale", 1.0))
         kernel = 32 if args.get("kernel") == "wave" else args.get("kernel")
         if self.pdist is not None:
             if kernel is not None and int(kernel) > 1:
@@ -237,14 +239,24 @@ class nonlinear_fit(object):
                 raise ValueError("b200_lm: bounds are not built for fits with parameter distributions")
             if POLICY.get(fit["policy"]) == 1:
                 raise ValueError("b200_lm: policy='gsl' is not built for fits with parameter distributions")
-        return fit, kernel, args.get("loss", "linear"), POLICY.get(fit["policy"]) == 1
+        return fit, kernel, fit["loss"], POLICY.get(fit["policy"]) == 1
 
     def _batch(self, means, p0, tol=None, maxit=None, want_cov=True, **kargs):
         plan = self._spec.plan(self.device)
         args, kernel, loss, gsl = self._batch_args(dict(kargs, tol=tol, maxit=maxit))
+        # the copies estimate the spread of THIS fit's estimator: they are fitted with its own loss, never another one
+        own = self.fitterargs.get("loss", "linear"), float(self.fitterargs.get("f_scale", 1.0))
+        if (loss, float(args["f_scale"])) != own and (loss != "linear" or own[0] != "linear"):
+            raise ValueError("b200_lm: batch copies are fitted with the fit's own robust loss (loss=%r, f_scale=%g); "
+                             "loss=%r, f_scale=%g was given: make the fit itself with that loss"
+                             % (own[0], own[1], loss, float(args["f_scale"])))
         if loss != "linear":
-            raise ValueError("batched fits with a robust loss (loss=%r) are not built: fit the copies one at a time "
-                             "(fitter='b200_dense')" % (loss,))
+            if args["bounds"] is not None:
+                raise ValueError("b200_lm: a robust loss together with bounds is not built for batched fits")
+            if self.pdist is not None:
+                raise ValueError("b200_lm: a robust loss is not built for fits with parameter distributions (pdist)")
+            if gsl:
+                raise ValueError("b200_lm: a robust loss is not built for policy='gsl'")
         if gsl and args["bounds"] is not None:
             raise ValueError("b200_lm: policy='gsl' has no bound constraints")
         if kernel is not None:
